@@ -19,6 +19,7 @@ Beside the headline the same run measures, and puts on the same JSON line:
                      on the rows the cpu_baseline leg traced
 
   python bench.py [--gpus N] [--steps K] [--warmup W]          one JSON line on stdout (rank 0)
+  python bench.py ... --dump-outputs DIR                      + the last timed step's outputs as DIR/*.npy (sampled)
   python bench.py --impl reference ...                        the CPU restatement of the reference
                                                               path on the host cores (oracle port;
                                                               Julia is not installed here)
@@ -47,6 +48,9 @@ BYTES_PER_RAY = 17                  # ex, ey (16 B) + mask (1 B)
 LOOP_STEPS = 12                     # reference loop iterations per ray (11 surfaces + image plane)
 WORKLOAD = ("double-Gauss (10 glass surfaces, 12 loop steps), 16Mi-ray half-pupil grid "
             f"{NY}x{NX} per field x 5 fields per GPU, outputs ex, ey, mask + per-field spot stats")
+DUMP_RAYS = 1 << 18                 # --dump-outputs: grid points sampled per field (5 fields x 20 B x 2^18 = 26 MB)
+DUMP_SEED = 20251020
+DUMP_MAX_BYTES = 64 << 20
 
 
 def log(*a):
@@ -155,6 +159,26 @@ def cpu_baseline(ort, wl, target_s=12.0, threads=0, keep=False):
     t, rays, outs = run(rows, keep)
     return dict(rps=rays / t, cores=nthreads, rows=rows, seconds=t, outs=outs,
                 sample=f"first {rows} of {NY} y-rows x {NX} x {len(wl['fields'])} fields = {rays} rays in {t:.2f} s")
+
+
+def dump_outputs(R, out_dir, d_ex, d_ey, d_mask, merged):
+    """What the timed path returned in its last step, as .npy files: ex, ey (float64) and mask (float32) at the same
+    DUMP_RAYS grid points of every field, drawn once with a fixed seed (sample_index holds their flat y-major indices),
+    and every member of the per-field statistics records (stats_<member>, float64).  The full grid is 1.43 GB per step.
+    At N > 1 rank 0 writes its own block of y-rows and the records merged over all ranks."""
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(d_ex.shape[1], DUMP_RAYS, replace=False))
+    d_idx = R.torch.from_numpy(idx).to(R.dev)
+    arrays = {"sample_index": idx.astype(np.float64),
+              "ex": d_ex[:, d_idx].cpu().numpy(), "ey": d_ey[:, d_idx].cpu().numpy(),
+              "mask": d_mask[:, d_idx].cpu().numpy().astype(np.float32)}
+    for name in merged.dtype.names:
+        arrays["stats_" + name] = merged[name].astype(np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, total
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    log(f"--dump-outputs: {len(arrays)} arrays, {total} bytes in {out_dir}")
 
 
 def main():
@@ -423,7 +447,13 @@ def _main(real_stdout):
     ap.add_argument("--arith", default="fast", choices=["fast", "strict"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="headline only: skip strong / secondary / parity")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step as DIR/<name>.npy (a fixed, seeded sample of the grid)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -525,6 +555,8 @@ def _main(real_stdout):
         allm = [torch.zeros_like(d_stats) for _ in range(n)]
         dist.all_gather(allm, d_stats)
         ident = bool(all(torch.equal(allm[0], t) for t in allm))
+    if args.dump_outputs and rank == 0:
+        dump_outputs(R, args.dump_outputs, d_ex, d_ey, d_mask, merged)
 
     # ---- e2e: the C-ABI host-pointer call, pinned host buffers, H2D of the grid coordinates and
     #      D2H of spot diagram + mask + statistics inside the timed region.  Two output forms are
