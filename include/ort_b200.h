@@ -39,7 +39,8 @@ extern "C" {
 #pragma GCC visibility push(default)   /* the library is built with -fvisibility=hidden */
 #endif
 
-#define ORT_VERSION 200 /* 0.2.0: communicator inside the library, ort_opts.gather_stats, ort_grid_out.stats_local */
+#define ORT_VERSION 200 /* 0.2.0: communicator inside the library, ort_opts.gather_stats, ort_grid_out.stats_local;
+                           ort_trace3d_focus / ort_trace3d_focus_dev (through-focus sweep) added without a version change */
 
 /* status codes */
 #define ORT_OK            0
@@ -56,6 +57,7 @@ extern "C" {
 #define ORT_MAX_LENS  128   /* rows of a paraxial Lens matrix */
 #endif
 #define ORT_MAX_GPUS   16   /* contexts of one process in ort_comm_init_all / ort_trace3d_grid_multi */
+#define ORT_MAX_FOCI   64   /* image planes per ort_trace3d_focus call */
 
 /* per-ray flag bits */
 #define ORT_FLAG_MISS   1u  /* conic discriminant < 0: position NaN from here on (PupilSampling.jl:9, RayTracing.jl:83) */
@@ -200,6 +202,37 @@ int ort_trace3d_grid_dev(ort_ctx *ctx, const ort_field *fields /* host */, int n
                          const double *d_ys, int ny, const double *d_xs, int nx,
                          int stop, double a_stop, const ort_opts *opts,
                          const ort_grid_out *d_out /* device pointers inside */, void *stream);
+
+/* ---- EXTENSION (no reference method): through-focus sweep.  The same pupil-grid sweep as ort_trace3d_grid, evaluated on
+ *      n_foci image planes in one pass: every ray is traced once up to the image plane and then transferred to each
+ *      plane, so the results at foci[j] are those of full_trace(..., focus = foci[j]) (src/PupilSampling.jl:85,111-114).
+ *      foci[j] (host, finite) replaces t[rows-2] of the current layout as the image distance; the last row must be a
+ *      plane (R = +-Inf, K = 0); stop <= rows - 2.  The layout's own t[rows-2] still takes part in how ort_set_layout
+ *      classifies the prescription: a non-finite value resolves ORT_ARITH_FAST to STRICT, and it is one term of the length
+ *      scale L that admits spheres with |R| <= 64 L to the SIMPLE kernel.  Set it to a focus of the sweep (full_trace's
+ *      paraxial one): then FAST results are bit-identical to an ort_trace3d_grid sweep at every focus whose layout
+ *      classifies the same -- which only a sphere within a few percent of the 64 L bound can fail to do.
+ *      Outputs (any pointer may be NULL):
+ *        ex, ey                    [n_fields][n_foci][ny*nx]; with opts.compact segment (f, j) holds stats[f*n_foci + j].n_kept
+ *                                  entries in push! order
+ *        r, theta, mask, flags     [n_fields][ny*nx], one per field (the same at every focus); with opts.compact r and
+ *                                  theta are compacted per field like ex, ey
+ *        stats                     [n_fields][n_foci]: n_kept, r_max and the flag counts are the same for every focus
+ *        wx, wy, opd, stats_local  must be NULL
+ *      Drop rule: a ray is dropped at every focus of its field if the stop clips it, if it misses a surface, or if its
+ *      position is NaN at ANY focus.  For every ray that is finite at all foci this is full_trace's own rule at each
+ *      focus; the two differ only for a ray with k3 = 0 after the last glass surface.  Likewise the image plane's TIR flag
+ *      (a refracting image plane) is raised iff the reference raises it at every focus: x^2 + y^2 on the plane finite at
+ *      all of them (the same k3 = 0 / overflow exception).
+ *      Honours opts.arith, opts.compact and opts.ys_per_field, field modes 0 and 1.  ORT_EUNSUPPORTED for opts.ext != 0,
+ *      opts.gather_stats and polynomial terms on the context.  A stats-only call launches two kernels whatever n_foci;
+ *      compaction adds three. */
+int ort_trace3d_focus(ort_ctx *ctx, const ort_field *fields, int n_fields, const double *ys, int ny,
+                      const double *xs, int nx, int stop, double a_stop,
+                      const double *foci /* host, n_foci */, int n_foci, const ort_opts *opts, ort_grid_out *out);
+int ort_trace3d_focus_dev(ort_ctx *ctx, const ort_field *fields /* host */, int n_fields, const double *d_ys, int ny,
+                          const double *d_xs, int nx, int stop, double a_stop, const double *foci /* host */, int n_foci,
+                          const ort_opts *opts, const ort_grid_out *d_out /* device pointers inside */, void *stream);
 
 /* ---- 3-D skew trace of N arbitrary rays, all surfaces recorded: replaces
  *      raytrace(surfaces, y, x, U, V, Vector{RealRay}) src/PupilSampling.jl:34-65 for a batch.

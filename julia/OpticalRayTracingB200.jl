@@ -202,6 +202,65 @@ function full_trace(::B200, surfaces::Layout, system::SystemOrRayBasis, H::Float
     return RealRayError(εx, εy, nu, ρ, θ, H, RMS)
 end
 
+# --- through focus: full_trace at every focus of `foci` (EXTENSION, no reference method) -----------
+# The prelude is full_trace's (:85-114) verbatim; the pupil grid is traced ONCE and evaluated on every image plane in one
+# ccall (ort_trace3d_focus).  rms[j] == full_trace(surfaces, system, H, k_rays, foci[j]).RMS.  best_focus / best_rms: the
+# vertex of the least-squares parabola of rms^2 over the foci (exact: the kept set is the same at every focus).
+# Like the rest of this file it cannot be run in the repository that ships it (no Julia there); the Python host's
+# through_focus is the tested form of the same calls.
+function through_focus(::B200, surfaces::Layout, system::SystemOrRayBasis, H::Float64, foci::Vector{Float64};
+                       k_rays::Int = spot_rays, arith = ORT_ARITH_FAST)
+    require_conic(surfaces)
+    H = abs(H)
+    H ≤ 1.0 || throw(DomainError(H, "Domain: |H| ≤ 1.0"))
+    stop = system.stop
+    a_stop = abs(system.a[stop])
+    real_chief = trace_chief_ray(surfaces, system)
+    real_marginal = trace_marginal_ray(surfaces, system)
+    EP_t = real_chief.z[1]
+    Ū = real_chief.u[1]
+    U = H * Ū
+    u = tan(U)
+    y_EP = abs(real_marginal.y[1])
+    y1, y2 = (±(y_EP) - u * EP_t for (±) ∈ (+, -))
+    y1, y2 = trace_edge_rays(surfaces, y1, y2, U, stop, a_stop)
+    if typeof(system) <: System
+        field = OrtField(0, 0, u, tan(0.0), 0.0, 1.0, u * system.f, 0.0, 0.0, 0.0, 0.0)
+    else
+        z0 = system.marginal.z[1]
+        ȳ = system.chief.y[2] + system.chief.u[1] * z0
+        field = OrtField(1, 0, 0.0, 0.0, ȳ, z0, system.chief.y[end], 0.0, 0.0, 0.0, 0.0)
+    end
+    # the extended surfaces of :111-114; t[end-1] is replaced by each focus inside the library
+    R = [surfaces.R; Inf]; t = [surfaces.t; 0.0]; n = [surfaces.n; 1.0]; K = [surfaces.K; 0.0]
+    set_layout(R, t, n, K)
+    ys = collect(range(y1, y2, k_rays))              # :121
+    xs = collect(range(0.0, y_EP, div(k_rays, 2)))   # :122
+    M = length(foci)
+    stats = [OrtStats(0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0) for _ in 1:M]
+    opts = Ref(OrtOpts(arith, 0, 0, 0, 0.0, 1.0, 1.0, 0, 0))
+    GC.@preserve stats begin
+        out = Ref(OrtGridOut(C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, C_NULL, pointer(stats), C_NULL))
+        check(ccall((:ort_trace3d_focus, LIB), Cint,
+                    (Ptr{Cvoid}, Ref{OrtField}, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint, Float64,
+                     Ptr{Float64}, Cint, Ref{OrtOpts}, Ref{OrtGridOut}),
+                    ctx(), Ref(field), 1, ys, length(ys), xs, length(xs), stop, a_stop, foci, M, opts, out))
+    end
+    rms = [s.n_kept == 0 ? NaN : sqrt((2 * (s.m2_x + s.n_kept * s.mean_x^2) + 2 * s.m2_y) / (2 * s.n_kept)) for s in stats]
+    n_kept = stats[1].n_kept
+    best_focus, best_rms = NaN, NaN
+    if length(unique(foci)) ≥ 3 && all(isfinite, rms)
+        fm = sum(foci) / M
+        d = foci .- fm
+        A, B, C = [d .^ 2 d ones(M)] \ (rms .^ 2)
+        if A > 0
+            best_focus = fm - B / (2A)
+            best_rms = sqrt(max(C - B^2 / (4A), 0.0))
+        end
+    end
+    return (rms = rms, n_kept = n_kept, best_focus = best_focus, best_rms = best_rms)
+end
+
 # --- batched 2-D meridional real rays: src/RayTracing.jl:145-173 ------------------------------
 # Returns (y, U, ts), each rows × N, for N rays in one kernel launch.
 function raytrace(surfaces::Layout{T}, ys::Vector{Float64}, Us::Vector{Float64}, ::Type{RealRay}) where T

@@ -11,7 +11,7 @@ from ._lib import (EXT_OPD, EXT_VIGNETTE, FAST, STRICT, FLAG_CLIP, FLAG_DOMAIN, 
                    Context, OrtError, PinnedArray, STATS_BYTES, STATS_DTYPE)
 from .host import (LAMBDA, SA, TSA, Aberration, aberrations, seidel_merit, Wavefront, aim_rays, wavefront, Layout, Lens, RayBasis, RealRay, RealRayError, System,
                    VectorRealRay, flatten, full_trace, full_trace_candidates, full_trace_fields, make_lens, merge_stats,
-                   raytrace, reverse_transfer, rms_from_stats, set_default_backend, solve,
+                   raytrace, reverse_transfer, rms_from_stats, set_default_backend, solve, through_focus, ThroughFocus,
                    trace_chief_ray, trace_edge_rays, trace_marginal_ray, transfer, transfer_matrix,
                    vignetting, Vignetting, wavegrad)
 
@@ -19,5 +19,5 @@ __all__ = ["_lib", "distributed", "host", "prescriptions", "Context", "OrtError"
            "STRICT", "FLAG_MISS", "FLAG_TIR", "FLAG_DOMAIN", "FLAG_CLIP", "FLAG_VIGN", "EXT_OPD", "EXT_VIGNETTE", "STATS_BYTES", "LAMBDA", "SA", "TSA", "Aberration", "aberrations", "seidel_merit", "Wavefront", "aim_rays", "wavefront",
            "Layout", "Lens", "RayBasis", "RealRay", "RealRayError", "System", "VectorRealRay",
            "flatten", "full_trace", "full_trace_candidates", "full_trace_fields", "make_lens", "merge_stats", "raytrace",
-           "reverse_transfer", "rms_from_stats", "set_default_backend", "solve", "trace_chief_ray",
+           "reverse_transfer", "rms_from_stats", "set_default_backend", "solve", "through_focus", "ThroughFocus", "trace_chief_ray",
            "trace_edge_rays", "trace_marginal_ray", "transfer", "transfer_matrix", "vignetting", "Vignetting", "wavegrad"]

@@ -12,7 +12,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("ORT_B200_LIB", os.path.join(_HERE, "lib", "libort_b200.so"))
 
 ORT_OK, ORT_EINVAL, ORT_ECUDA, ORT_ENCCL, ORT_EUNSUPPORTED, ORT_ENOMEM = 0, -1, -2, -3, -4, -5
-MAX_ROWS, MAX_FIELDS, MAX_LENS, MAX_GPUS = 64, 32, 128, 16
+MAX_ROWS, MAX_FIELDS, MAX_LENS, MAX_GPUS, MAX_FOCI = 64, 32, 128, 16, 64
 COMM_ID_BYTES = 128
 FLAG_MISS, FLAG_TIR, FLAG_DOMAIN, FLAG_CLIP, FLAG_VIGN = 1, 2, 4, 8, 16
 EXT_OPD, EXT_VIGNETTE = 1, 2
@@ -25,7 +25,7 @@ SYMBOLS = [
     "ort_version", "ort_init", "ort_free", "ort_last_error", "ort_sync", "ort_device_info",
     "ort_host_alloc", "ort_host_free", "ort_device_numa", "ort_bind_host_thread", "ort_launch_count", "ort_profile_enable", "ort_profile_read",
     "ort_set_layout", "ort_set_apertures", "ort_set_polynomials",
-    "ort_trace3d_grid", "ort_trace3d_grid_dev", "ort_trace3d_rays", "ort_trace3d_rays_opl", "ort_trace3d_rays_dev", "ort_trace2d_batch", "ort_aim2d",
+    "ort_trace3d_grid", "ort_trace3d_grid_dev", "ort_trace3d_focus", "ort_trace3d_focus_dev", "ort_trace3d_rays", "ort_trace3d_rays_opl", "ort_trace3d_rays_dev", "ort_trace2d_batch", "ort_aim2d",
     "ort_paraxial_batch", "ort_paraxial_batch_dev", "ort_transfer_batch", "ort_transfer_batch_dev",
     "ort_trace3d_candidates", "ort_trace3d_candidates_dev", "ort_aim_candidates", "ort_aim_candidates_dev", "ort_aim_fields",
     "ort_trace3d_candidates_aimed", "ort_trace3d_candidates_aimed_dev", "ort_vignetting_candidates",
@@ -118,6 +118,8 @@ def load():
                  C.c_int, C.c_double, C.POINTER(Opts), C.POINTER(GridOut)]
     L.ort_trace3d_grid.argtypes = grid_args
     L.ort_trace3d_grid_dev.argtypes = grid_args + [C.c_void_p]
+    L.ort_trace3d_focus.argtypes = grid_args[:9] + [_dp, C.c_int] + grid_args[9:]
+    L.ort_trace3d_focus_dev.argtypes = grid_args[:9] + [_dp, C.c_int] + grid_args[9:] + [C.c_void_p]
     L.ort_trace3d_rays.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p]
     L.ort_trace3d_rays_opl.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p, _dp]
     L.ort_trace3d_rays_dev.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 6
@@ -494,6 +496,53 @@ class Context:
         self._ck(self.L.ort_trace3d_grid_dev(self.h, farr, nf, C.c_void_p(d_ys), int(ny), C.c_void_p(d_xs),
                                              int(nx), int(stop), float(a_stop), C.byref(op), C.byref(go),
                                              C.c_void_p(stream)))
+
+    # ---- through-focus sweep -------------------------------------------------------------
+    def trace3d_focus(self, fields, ys, xs, stop, a_stop, foci, arith=FAST, compact=False, want=("stats",)):
+        """The grid sweep at M image planes in one pass (ort_trace3d_focus): foci[j] replaces t[rows-2] of the current
+        layout.  Returns a dict: 'stats' (n_fields, M) STATS_DTYPE; 'ex', 'ey' (n_fields, M, ny*nx); 'r', 'theta', 'mask',
+        'flags' (n_fields, ny*nx), the same for every focus.  With compact=True ex / ey [f, j] hold stats[f, j].n_kept
+        entries in push! order (r, theta per field likewise)."""
+        farr, nf = make_fields(fields)
+        ys, xs = _d(ys), _d(xs)
+        per_field = ys.ndim == 2
+        if per_field and ys.shape[0] != nf:
+            raise ValueError("ys must be (ny,) or (n_fields, ny)")
+        foci = _d(np.atleast_1d(foci))
+        M = len(foci)
+        ny, nx = ys.shape[-1], len(xs)
+        NN = ny * nx
+        res = {}
+        for name in ("ex", "ey"):
+            if name in want:
+                res[name] = np.empty((nf, M, NN), dtype=np.float64)
+        for name in ("r", "theta"):
+            if name in want:
+                res[name] = np.empty((nf, NN), dtype=np.float64)
+        for name in ("mask", "flags"):
+            if name in want:
+                res[name] = np.zeros((nf, NN), dtype=np.uint8)
+        stats = np.zeros((nf, M), dtype=STATS_DTYPE)
+        go = GridOut(*[(res[k].ctypes.data if k in res else None)
+                       for k in ("ex", "ey", "r", "theta", "wx", "wy", "opd", "mask", "flags")], stats.ctypes.data, None)
+        op = Opts(int(arith), int(bool(compact)), int(per_field), 0, 0.0, 1.0, 1.0, 0, 0)
+        self._ck(self.L.ort_trace3d_focus(self.h, farr, nf, _vp(ys), ny, _vp(xs), nx, int(stop), float(a_stop), _p(foci), M,
+                                          C.byref(op), C.byref(go)))
+        res["stats"] = stats
+        return res
+
+    def trace3d_focus_dev(self, fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, ptrs, stream=0, arith=FAST, compact=False,
+                          ys_per_field=False):
+        """Device-pointer through-focus sweep (enqueue only).  ptrs: dict name -> device address; 'ex', 'ey' are
+        [n_fields][M][ny*nx], 'r', 'theta', 'mask', 'flags' [n_fields][ny*nx], 'stats' [n_fields][M]."""
+        farr, nf = make_fields(fields)
+        foci = _d(np.atleast_1d(foci))
+        go = GridOut(*[ptrs.get(k) for k in ("ex", "ey", "r", "theta", "wx", "wy", "opd", "mask", "flags", "stats",
+                                             "stats_local")])
+        op = Opts(int(arith), int(bool(compact)), int(bool(ys_per_field)), 0, 0.0, 1.0, 1.0, 0, 0)
+        self._ck(self.L.ort_trace3d_focus_dev(self.h, farr, nf, C.c_void_p(d_ys), int(ny), C.c_void_p(d_xs), int(nx),
+                                              int(stop), float(a_stop), _p(foci), len(foci), C.byref(op), C.byref(go),
+                                              C.c_void_p(stream)))
 
     # ---- arbitrary rays ------------------------------------------------------------------
     def trace3d_rays(self, y0, x0, u0, v0, arith=STRICT, opl=False):

@@ -28,6 +28,14 @@ struct GridArgs {
     ort_field fields[ORT_MAX_FIELDS];
 };
 
+struct FocusArgs {                          // through-focus sweep (k_focus)
+    GridArgs G;                             // grid, stop, per-field outputs r / theta / mask / flags, tile counts; G.ex, G.ey
+                                            // are [n_fields][n_foci][NN]; G.partials is [n_fields * n_foci][gridDim.x]
+    int n_foci;
+    double t_lo, t_hi;                      // smallest and largest focus
+    double foci[ORT_MAX_FOCI];
+};
+
 struct CompactArgs {
     unsigned NN;
     const uint8_t* mask;
@@ -174,6 +182,9 @@ cudaError_t launch_grid(const Presc& P, const GridArgs& A, int arith, dim3 grid,
 cudaError_t launch_grid_finalize(const RawPart* partials, int nparts, int n_fields, ort_stats* stats,
                                  cudaStream_t st);
 cudaError_t launch_compact(int* tile_counts, const CompactArgs& C, int n_fields, cudaStream_t st);
+int focus_blocks_per_sm(int arith, int variant);
+cudaError_t launch_focus(const Presc& P, const FocusArgs& F, int arith, dim3 grid, cudaStream_t st);
+cudaError_t launch_compact_focus(int* tile_counts, const CompactArgs& C, int n_fields, int n_foci, cudaStream_t st);
 cudaError_t launch_rays(const Presc& P, const RaysArgs& A, int arith, cudaStream_t st);
 cudaError_t launch_candidates(const CandArgs& A, int arith, cudaStream_t st, int sm_count);
 cudaError_t launch_trace2d(const Presc& P, const Trace2dArgs& A, cudaStream_t st);

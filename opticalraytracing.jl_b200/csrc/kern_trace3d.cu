@@ -9,6 +9,7 @@
 //                      SIMPLE instantiation for prescriptions of refracting spheres and planes (three-body surface loop).
 //   k_grid_finalize    K6: deterministic fold of the per-CTA partials into ort_stats per field.
 //   k_tile_scan / k_compact   ordered compaction in the reference's push! order (:134-137).
+//   k_focus / k_compact_focus through-focus sweep: each ray traced once, evaluated on up to ORT_MAX_FOCI image planes.
 //   k_rays<ARITH>      arbitrary rays, every surface recorded (raytrace(...,Vector{RealRay}) :34-65).
 //   k_candidates<ARITH> K5: one CTA per candidate prescription staged in shared memory.
 #include "kern.cuh"
@@ -574,6 +575,388 @@ __global__ void __launch_bounds__(ORT_TILE) k_compact(CompactArgs C)
 }
 
 // ------------------------------------------------------------------------------------------
+// through-focus sweep: every ray traced once up to the image plane, then M image planes (foci)
+// ------------------------------------------------------------------------------------------
+// The image plane is the last row of the extended layout ([Inf 0 1], t[end-1] = focus, src/PupilSampling.jl:111-114).
+// Nothing before it depends on the focus: the stop clip, the miss / TIR / domain flags, r and theta are fixed one
+// surface earlier, and the position on a plane is one transfer from the state after the last glass surface.  k_focus
+// keeps that state per ray in five or six doubles (FocusRay) and evaluates the transfer once per focus with the plane
+// lines of the body k_grid would run -- strict_step's for STRICT, fast_step's plain-plane body for FAST, restated
+// operation for operation -- so every per-ray output is bit-identical to a k_grid sweep of the layout with
+// t[end-1] = foci[j].
+//
+// FAST: fast_div(n, d) = n * r with r a function of d alone, so the reciprocal of Kz is taken once per ray and a focus
+// costs one DADD, one DMUL and two DFMA (x, y) plus the statistics.  The position is affine in the rounded (t - z), so
+// it is non-finite at some focus iff it is at the smallest or the largest one: those two decide the strict re-trace.
+//
+// Drop rule: a ray is dropped for every focus of its field if the stop clips it, or if its position is NaN at ANY focus
+// (only a ray with k3 = 0 after the last glass surface can be NaN at one focus and not at another).  mask, flags, r,
+// theta and the kept count are therefore per field; for every ray that is finite at all foci this is full_trace's own
+// per-focus rule.
+struct FocusRay {
+    // STRICT state: a0 = x, a1 = y, a2 = sprev, a3 = v, a4 = u.  FAST state: a0 = x, a1 = y, a2 = z, a3 = Kx, a4 = Ky,
+    // a5 = 1 / Kz as fast_div forms it.
+    double a0, a1, a2, a3, a4, a5;
+};
+
+// strict_step's first and last position lines at a plane (sag s = 0), with t = the focus: src/PupilSampling.jl:46-47, 52-53
+__device__ __forceinline__ void focus_pos_strict(const FocusRay& q, double t, double& xf, double& yf)
+{
+    const double ti = SS(t, q.a2);
+    double y = SA(q.a1, SM(q.a4, ti));
+    double x = SA(q.a0, SM(q.a3, ti));
+    y = SA(y, SM(0.0, q.a4));
+    x = SA(x, SM(0.0, q.a3));
+    xf = x; yf = y;
+}
+
+// fast_step's plain-plane body: s = fast_div(t - z, Kz); x = fma(s, Kx, x); y = fma(s, Ky, y)
+__device__ __forceinline__ void focus_pos_fast(const FocusRay& q, double t, double& xf, double& yf)
+{
+    const double s = (t - q.a2) * q.a5;
+    xf = fma(s, q.a3, q.a0);
+    yf = fma(s, q.a4, q.a1);
+}
+
+// the reciprocal fast_div multiplies its numerator by
+__device__ __forceinline__ double fast_div_rcp(double d)
+{
+    double r = mufu_rcp(d);
+    const double e = fma(-d, r, 1.0);
+    return fma(r, fma(e, e, e), r);
+}
+
+struct FocusS {                     // strict state after surface nsurf - 2
+    FocusRay q;
+    double xs, ys;                  // position at the stop surface
+    unsigned flags;                 // ORT_FLAG_* of surfaces 0 .. nsurf-2, plus FOCUS_TIR_LAST (see below)
+};
+
+// Internal bit of FocusS::flags: the image plane refracts with total internal reflection IF strict_step's plane normal is
+// m = (0, 0, -1).  strict_step uses that normal when the position on the plane has |x|, |y| < 1e150; otherwise it
+// normalises (sgn x / sqrt(Inf - (x^2 + y^2)), ..., -1), which is the same m while x^2 + y^2 is finite and NaN (no flag)
+// when it is not.  So the flag is raised iff this bit is set and x^2 + y^2 on the plane is finite -- decided by k_focus
+// once the positions at the foci are known.
+#define FOCUS_TIR_LAST 0x80u
+
+// STRICT trace through surfaces 0 .. nsurf-2 (k_grid's per-surface body), the stop position at stop - 1, and the image
+// plane's TIR decision (FOCUS_TIR_LAST)
+template <bool XF>
+__device__ __forceinline__ FocusS focus_strict_impl(const Presc& P, int stop, double y, double x, double u, double v, int* bad)
+{
+    RayS r;
+    strict_init<XF>(r, y, x, u, v);
+    FocusS o; o.xs = o.ys = CUDART_NAN;
+    const int ns = P.nsurf - 1;
+    for (int i = 0; i < ns; i++) {
+        strict_step<false, false, XF>(P.s[i], r);
+        if (i == stop - 1) { o.xs = r.x; o.ys = r.y; }
+    }
+    const SurfK& S = P.s[ns];
+    double dot = SA(0.0, SM(r.k1, 0.0)); dot = SA(dot, SM(r.k2, 0.0)); dot = SA(dot, SM(r.k3, -1.0));
+    const double gam = -dot;
+    const double Dr = SS(1.0, SM(S.etasq, SS(1.0, SM(gam, gam))));
+    if (Dr < 0.0) r.flags |= FOCUS_TIR_LAST;
+    o.q.a0 = r.x; o.q.a1 = r.y; o.q.a2 = r.sprev; o.q.a3 = r.v; o.q.a4 = r.u; o.q.a5 = 0.0;
+    o.flags = r.flags;
+    if (XF) *bad = r.bad;
+    return o;
+}
+
+__device__ __noinline__ FocusS focus_strict_cold(const Presc& P, int stop, double y, double x, double u, double v)
+{
+    return focus_strict_impl<false>(P, stop, y, x, u, v, nullptr);
+}
+
+// k_grid's grid shape (tile-strided CTAs, blockIdx.y = field) and surface bodies.  Statistics per (field, focus): the
+// shifted moments of k_grid (the shift of focus j is the field's centre ray at focus j); per tile and focus the warp
+// reduces by shuffle and lane 0 adds into its own row of s_acc, so every partial is a fixed-order sum.  Counts, r_max
+// and flags are the same for every focus of a field and go into every record.
+template <int ARITH, int RPT, bool MIRROR, int SIMPLE>
+__global__ void __launch_bounds__(ORT_TILE, 2)
+k_focus(const __grid_constant__ Presc P, const __grid_constant__ FocusArgs F)
+{
+    constexpr int NWARPS = ORT_TILE / 32;
+    __shared__ double s_acc[NWARPS][ORT_MAX_FOCI][4];
+    __shared__ double s_c[ORT_MAX_FOCI][2];
+    __shared__ RawPart s_part[NWARPS];
+    __shared__ RawPart s_p0;
+    __shared__ double2 s_xy[RPT][ORT_TILE];     // FAST: position at the stop, kept out of registers (r^2 recomputed from it)
+    // per-thread counters and r_max, each thread in its own slot: registers stay with the rays (no spills at RPT = 3)
+    __shared__ int s_cnt[4][ORT_TILE];          // kept, (miss, tir) and (domain, clip) packed 16 + 16 as in RawAcc, strict
+    __shared__ double s_rmax[ORT_TILE];
+    const GridArgs& A = F.G;
+    const int M = F.n_foci;
+    const int f = blockIdx.y;
+    const ort_field& fld = A.fields[f];
+    const unsigned NN = A.NN;
+    const unsigned nsub = (NN + ORT_TILE - 1) / ORT_TILE;
+    const unsigned ntiles = (nsub + RPT - 1) / RPT;
+    const size_t fbase = (size_t)f * NN;
+    const double* ysf = A.ys + (size_t)f * A.ys_stride;
+    const unsigned ysoff = (unsigned)f * (unsigned)A.ys_stride;
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+
+    for (int i = threadIdx.x; i < NWARPS * ORT_MAX_FOCI * 4; i += ORT_TILE) (&s_acc[0][0][0])[i] = 0.0;
+    if (threadIdx.x == 0) {                      // common shift of every focus: the field's centre ray there
+        const double y0 = __ldg(ysf + A.ny / 2), x0 = __ldg(A.xs);
+        double u, v; field_slopes(fld, y0, x0, u, v);
+        const FocusS c = focus_strict_cold(P, A.stop, y0, x0, u, v);
+        for (int m = 0; m < M; m++) {
+            double xf, yf; focus_pos_strict(c.q, F.foci[m], xf, yf);
+            const double ey = yf - fld.h_prime;
+            const bool bad = nonfinite_bit(xf) < 0 || nonfinite_bit(ey) < 0;
+            s_c[m][0] = bad ? 0.0 : xf;
+            s_c[m][1] = bad ? 0.0 : ey;
+        }
+    }
+    __syncthreads();
+
+    int* const cnt_n = &s_cnt[0][threadIdx.x];
+    int* const cnt_lo = &s_cnt[1][threadIdx.x];
+    int* const cnt_hi = &s_cnt[2][threadIdx.x];
+    int* const cnt_strict = &s_cnt[3][threadIdx.x];
+    *cnt_n = *cnt_lo = *cnt_hi = *cnt_strict = 0;
+    s_rmax[threadIdx.x] = -CUDART_INF;
+    const SurfK& SL = P.s[P.nsurf - 1];          // the image plane
+    const bool refr_last = (SL.kcode & SURF_REFR) != 0;
+    const bool collimated = (fld.mode == 0);
+    double K0[3] = {0.0, 0.0, 0.0};
+    if (ARITH == ORT_ARITH_FAST && collimated) {
+        const double inv = P.n0 * fast_rsqrt(fma(fld.v, fld.v, fma(fld.u, fld.u, 1.0)));
+        K0[0] = fld.v * inv; K0[1] = fld.u * inv; K0[2] = inv;
+    }
+    const unsigned nxu = (unsigned)A.nx;
+
+    for (unsigned tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+        double y0[RPT], x0[RPT], u[RPT], v[RPT];
+        unsigned idx[RPT];
+        bool valid[RPT];
+#pragma unroll
+        for (int j = 0; j < RPT; j++) {
+            const unsigned i0 = (tile * RPT + j) * ORT_TILE + threadIdx.x;
+            valid[j] = i0 < NN;
+            idx[j] = min(i0, NN - 1);            // padded lanes trace the last ray: the warp stays convergent
+            const unsigned iy = idx[j] / nxu, ix = idx[j] - iy * nxu;      // a division per ray instead of 2 RPT registers
+            y0[j] = __ldg(A.ys + (ysoff + iy)); x0[j] = __ldg(A.xs + ix);
+            u[j] = 0.0; v[j] = 0.0;
+        }
+        if (!collimated || ARITH != ORT_ARITH_FAST) {
+#pragma unroll
+            for (int j = 0; j < RPT; j++) field_slopes(fld, y0[j], x0[j], u[j], v[j]);
+        }
+        FocusRay q[RPT];
+        double xs[RPT], ys[RPT];                // stop position of STRICT and re-traced rays (FAST: s_xy)
+        unsigned flg[RPT];
+        bool sv[RPT];
+        if (ARITH == ORT_ARITH_FAST) {
+            RaysF<RPT> r;
+#pragma unroll
+            for (int j = 0; j < RPT; j++) {
+                if (collimated) {
+                    r.x[j] = x0[j]; r.y[j] = y0[j]; r.z[j] = 0.0;
+                    r.Kx[j] = K0[0]; r.Ky[j] = K0[1]; r.Kz[j] = K0[2];
+                    r.amb[j] = 0; r.opl[j] = 0.0; r.vig[j] = 0;
+                } else fast_init(r, j, P.n0, y0[j], x0[j], u[j], v[j]);
+            }
+            const int ns = P.nsurf - 1;
+            int i = 0;
+            for (; i < A.stop; i++) fast_step<RPT, false, MIRROR, SIMPLE, 0>(P.s[i], r);
+#pragma unroll
+            for (int j = 0; j < RPT; j++) s_xy[j][threadIdx.x] = make_double2(r.x[j], r.y[j]);
+            for (; i < ns; i++) fast_step<RPT, false, MIRROR, SIMPLE, 0>(P.s[i], r);
+#pragma unroll
+            for (int j = 0; j < RPT; j++) {
+                int amb = r.amb[j];
+                if (refr_last) {                 // fast_step's refracting-plane decision and k_grid's test of the final Kz
+                    const double Dp = fma(r.Kz[j], r.Kz[j], SL.dn2);
+                    amb |= hi32(Dp) - SL.tir_thr;
+                    amb |= nonfinite_bit(MIRROR ? sign_of_n2(fast_sqrt(Dp), SL.n2mask) : fast_sqrt(Dp));
+                }
+                q[j].a0 = r.x[j]; q[j].a1 = r.y[j]; q[j].a2 = r.z[j]; q[j].a3 = r.Kx[j]; q[j].a4 = r.Ky[j];
+                q[j].a5 = fast_div_rcp(r.Kz[j]);
+                double xa, ya, xb, yb;
+                focus_pos_fast(q[j], F.t_lo, xa, ya);
+                focus_pos_fast(q[j], F.t_hi, xb, yb);
+                amb |= nonfinite_bit(xa) | nonfinite_bit(ya) | nonfinite_bit(xb) | nonfinite_bit(yb);
+                const double2 st = s_xy[j][threadIdx.x];
+                const double r2 = fma(st.x, st.x, st.y * st.y);                  // grid_epilogue's r^2 and stop guard band
+                amb |= tiny_vs_bit(r2 - A.a_stop2, A.a_stop2);
+                sv[j] = amb < 0;
+                flg[j] = 0u;
+            }
+        } else {
+#pragma unroll
+            for (int j = 0; j < RPT; j++) {
+                int bad = 0;
+                FocusS o = focus_strict_impl<ORT_STRICT_XF>(P, A.stop, y0[j], x0[j], u[j], v[j], &bad);
+                if (ORT_STRICT_XF && bad) o = focus_strict_cold(P, A.stop, y0[j], x0[j], u[j], v[j]);
+                q[j] = o.q; xs[j] = o.xs; ys[j] = o.ys; flg[j] = o.flags; sv[j] = true;
+            }
+        }
+        int kept[RPT];
+        int nk = 0, nclip = 0;
+        double rm = -CUDART_INF;
+#pragma unroll
+        for (int j = 0; j < RPT; j++) {
+            double ri = 0.0, r2 = 0.0;
+            bool clip;
+            if (ARITH == ORT_ARITH_FAST && !sv[j]) {
+                const double2 st = s_xy[j][threadIdx.x];
+                xs[j] = st.x; ys[j] = st.y;
+                r2 = fma(st.x, st.x, st.y * st.y);
+                clip = r2 > A.a_stop2;
+                if (A.r) ri = (r2 > 0.0) ? fast_sqrt(r2) : r2;
+            } else {
+                if (ARITH == ORT_ARITH_FAST) {       // rare in FAST mode: the ray's inputs once more, strict trace
+                    const unsigned iy = idx[j] / nxu, ix = idx[j] - iy * nxu;
+                    const double yy = __ldg(ysf + iy), xx = __ldg(A.xs + ix);
+                    double uu, vv; field_slopes(fld, yy, xx, uu, vv);
+                    const FocusS o = focus_strict_cold(P, A.stop, yy, xx, uu, vv);
+                    q[j] = o.q; xs[j] = o.xs; ys[j] = o.ys; flg[j] = o.flags;
+                }
+                ri = jl_hypot(xs[j], ys[j]);
+                clip = ri > A.a_stop;
+                r2 = ri * ri;
+            }
+            bool nan_any = false;
+            if (sv[j]) {                             // NaN at any focus drops the ray for all of them
+                bool fin_all = true;                 // x^2 + y^2 on the plane finite at every focus (FOCUS_TIR_LAST)
+                for (int m = 0; m < M; m++) {
+                    double xf, yf; focus_pos_strict(q[j], F.foci[m], xf, yf);
+                    nan_any = nan_any || is_nan_bits(xf) || is_nan_bits(yf);
+                    fin_all = fin_all && isfinite(SA(SM(xf, xf), SM(yf, yf)));
+                }
+                if (flg[j] & FOCUS_TIR_LAST) flg[j] = (flg[j] & ~FOCUS_TIR_LAST) | (fin_all ? ORT_FLAG_TIR : 0u);
+                if (valid[j]) {
+                    *cnt_strict += 1;
+                    *cnt_lo += (flg[j] & ORT_FLAG_MISS ? 1 : 0) + (flg[j] & ORT_FLAG_TIR ? 0x10000 : 0);
+                    *cnt_hi += (flg[j] & ORT_FLAG_DOMAIN ? 1 : 0);
+                }
+            }
+            const bool drop = clip || nan_any;
+            kept[j] = valid[j] && !drop;
+            const double rv = (ARITH == ORT_ARITH_STRICT) ? ri : r2;
+            if (valid[j]) {
+                const size_t o = fbase + idx[j];
+                if (A.r) A.r[o] = ri;
+                if (A.theta) A.theta[o] = atan2(ys[j], xs[j]);
+                if (A.mask) A.mask[o] = (uint8_t)kept[j];
+                if (A.flags) A.flags[o] = (uint8_t)(flg[j] | (clip ? ORT_FLAG_CLIP : 0u));
+                nclip += clip ? 1 : 0;
+            }
+            if (kept[j]) { if (rv > rm) rm = rv; nk++; }      // kept rays: never NaN
+        }
+        *cnt_n += nk;
+        *cnt_hi += nclip << 16;
+        if (rm > s_rmax[threadIdx.x]) s_rmax[threadIdx.x] = rm;
+        int any_kept = 0;
+#pragma unroll
+        for (int j = 0; j < RPT; j++) any_kept |= kept[j];
+        const bool warp_kept = __any_sync(0xffffffffu, any_kept);       // uniform per warp: no reduction for an empty warp
+        const bool want_e = A.ex != nullptr;
+        if (warp_kept || want_e) {
+            for (int m = 0; m < M; m++) {
+                const double t = F.foci[m];
+                const double cxm = s_c[m][0], cym = s_c[m][1];
+                double sx = 0.0, sxx = 0.0, sy = 0.0, syy = 0.0;
+#pragma unroll
+                for (int j = 0; j < RPT; j++) {
+                    double xf, yf;
+                    if (ARITH == ORT_ARITH_FAST && !sv[j]) focus_pos_fast(q[j], t, xf, yf);
+                    else focus_pos_strict(q[j], t, xf, yf);
+                    const double ex = xf;
+                    const double ey = SS(yf, fld.h_prime);
+                    if (want_e && valid[j]) {
+                        const size_t o = ((size_t)f * M + m) * NN + idx[j];
+                        A.ex[o] = ex; A.ey[o] = ey;
+                    }
+                    if (kept[j]) {
+                        const double dx = ex - cxm, dy = ey - cym;
+                        sx += dx; sxx = fma(dx, dx, sxx);
+                        sy += dy; syy = fma(dy, dy, syy);
+                    }
+                }
+                if (warp_kept) {
+#pragma unroll
+                    for (int d = 16; d >= 1; d >>= 1) {
+                        sx += __shfl_down_sync(0xffffffffu, sx, d);
+                        sxx += __shfl_down_sync(0xffffffffu, sxx, d);
+                        sy += __shfl_down_sync(0xffffffffu, sy, d);
+                        syy += __shfl_down_sync(0xffffffffu, syy, d);
+                    }
+                    if (lane == 0) {
+                        s_acc[warp][m][0] += sx; s_acc[warp][m][1] += sxx;
+                        s_acc[warp][m][2] += sy; s_acc[warp][m][3] += syy;
+                    }
+                }
+            }
+        }
+        if (A.tile_counts) {                    // ordered compaction: kept rays per 256-ray sub-tile
+#pragma unroll
+            for (int j = 0; j < RPT; j++) {
+                const int c = __syncthreads_count(kept[j]);
+                const unsigned sub = tile * RPT + j;
+                if (threadIdx.x == 0 && sub < nsub) A.tile_counts[(size_t)f * nsub + sub] = c;
+            }
+        }
+    }
+    RawPart p;
+    const int nflag_lo = *cnt_lo, nflag_hi = *cnt_hi;
+    p.n = *cnt_n; p.s1x = p.s2x = p.s1y = p.s2y = 0.0; p.rmax = s_rmax[threadIdx.x];
+    p.cx = p.cy = p.co = 0.0; p.s1o = p.s2o = 0.0; p.nvig = 0; p.nstrict = *cnt_strict;
+    p.nmiss = nflag_lo & 0xFFFF; p.ntir = nflag_lo >> 16; p.ndom = nflag_hi & 0xFFFF; p.nclip = nflag_hi >> 16;
+    raw_block_reduce<NWARPS>(p, s_part);         // its __syncthreads also orders the last s_acc updates
+    if (threadIdx.x == 0) {
+        if (ARITH != ORT_ARITH_STRICT) p.rmax = sqrt(p.rmax);
+        s_p0 = p;
+    }
+    __syncthreads();
+    for (int m = threadIdx.x; m < M; m += ORT_TILE) {
+        RawPart q = s_p0;
+        for (int w = 0; w < NWARPS; w++) {
+            q.s1x += s_acc[w][m][0]; q.s2x += s_acc[w][m][1];
+            q.s1y += s_acc[w][m][2]; q.s2y += s_acc[w][m][3];
+        }
+        q.cx = s_c[m][0]; q.cy = s_c[m][1];
+        A.partials[((size_t)f * M + m) * gridDim.x + blockIdx.x] = q;
+    }
+}
+
+// compaction of a focus sweep: one CTA per (tile, field); the foci of a field share its mask and tile offsets.
+// C.src / C.dst [0], [1] are ex, ey ([n_fields][n_foci][NN]); [2], [3] are r, theta ([n_fields][NN]).
+__global__ void __launch_bounds__(ORT_TILE) k_compact_focus(CompactArgs C, int n_foci)
+{
+    __shared__ int s_warp[ORT_TILE / 32];
+    const unsigned tile = blockIdx.x, f = blockIdx.y;
+    const unsigned ntiles = (C.NN + ORT_TILE - 1) / ORT_TILE;
+    const unsigned i = tile * ORT_TILE + threadIdx.x;
+    const size_t fbase = (size_t)f * C.NN;
+    const int m = (i < C.NN) ? C.mask[fbase + i] : 0;
+    const unsigned ball = __ballot_sync(0xffffffffu, m);
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    if (lane == 0) s_warp[warp] = __popc(ball);
+    __syncthreads();
+    int off = C.tile_offsets[(size_t)f * ntiles + tile];
+    {
+        const unsigned nchunks = (ntiles + SCAN_CHUNK - 1) / SCAN_CHUNK, mychunk = tile / SCAN_CHUNK;
+        const int* ct = C.tile_offsets + (size_t)gridDim.y * ntiles + (size_t)f * nchunks;
+        off += ct[mychunk];
+    }
+    for (int w = 0; w < warp; w++) off += s_warp[w];
+    off += __popc(ball & ((1u << lane) - 1u));
+    if (m) {
+        for (int a = 2; a < 4; a++)
+            if (C.src[a]) C.dst[a][fbase + off] = C.src[a][fbase + i];
+        for (int j = 0; j < n_foci; j++) {
+            const size_t b = ((size_t)f * n_foci + j) * C.NN;
+            for (int a = 0; a < 2; a++)
+                if (C.src[a]) C.dst[a][b + off] = C.src[a][b + i];
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------
 // arbitrary rays, all surfaces recorded
 // ------------------------------------------------------------------------------------------
 template <int ARITH, bool EXT>
@@ -1104,6 +1487,47 @@ cudaError_t launch_compact(int* tile_counts, const CompactArgs& C, int n_fields,
     cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess) return e;
     k_compact<<<dim3(ntiles, n_fields), ORT_TILE, 0, st>>>(C);
+    return cudaGetLastError();
+}
+
+// resident CTAs/SM of the k_focus instantiation of a k_grid variant (0 general, 2 SIMPLE, 4 SIMPLE-conic; FAST general
+// with and without MIRROR share their bounds); sizes the grid in ort_api.cu like grid_blocks_per_sm does k_grid's
+int focus_blocks_per_sm(int arith, int variant)
+{
+    int nb = 0;
+    cudaError_t e;
+    if (arith != ORT_ARITH_FAST) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_focus<ORT_ARITH_STRICT, ORT_STRICT_RPT, true, 0>, ORT_TILE, 0);
+    else if (variant == 2) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_focus<ORT_ARITH_FAST, ORT_SIMPLE_RPT, false, 1>, ORT_TILE, 0);
+    else if (variant == 4) e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_focus<ORT_ARITH_FAST, ORT_SC_RPT, false, 2>, ORT_TILE, 0);
+    else e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&nb, k_focus<ORT_ARITH_FAST, ORT_FAST_RPT, true, 0>, ORT_TILE, 0);
+    if (e != cudaSuccess || nb < 1) nb = 1;
+    return nb;
+}
+
+// the k_focus instantiation of the k_grid variant this prescription runs (grid_variant without extensions)
+cudaError_t launch_focus(const Presc& P, const FocusArgs& F, int arith, dim3 grid, cudaStream_t st)
+{
+    if (arith == ORT_ARITH_FAST) {
+        const int variant = grid_variant(P, arith, 0);
+        if (variant == 2) k_focus<ORT_ARITH_FAST, ORT_SIMPLE_RPT, false, 1><<<grid, ORT_TILE, 0, st>>>(P, F);
+        else if (variant == 4) k_focus<ORT_ARITH_FAST, ORT_SC_RPT, false, 2><<<grid, ORT_TILE, 0, st>>>(P, F);
+        else if (!P.has_mirror) k_focus<ORT_ARITH_FAST, ORT_FAST_RPT, false, 0><<<grid, ORT_TILE, 0, st>>>(P, F);
+        else k_focus<ORT_ARITH_FAST, ORT_FAST_RPT, true, 0><<<grid, ORT_TILE, 0, st>>>(P, F);
+    } else {
+        k_focus<ORT_ARITH_STRICT, ORT_STRICT_RPT, true, 0><<<grid, ORT_TILE, 0, st>>>(P, F);
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_compact_focus(int* tile_counts, const CompactArgs& C, int n_fields, int n_foci, cudaStream_t st)
+{
+    const unsigned ntiles = (C.NN + ORT_TILE - 1) / ORT_TILE;
+    const unsigned nchunks = (ntiles + SCAN_CHUNK - 1) / SCAN_CHUNK;
+    k_tile_scan<<<dim3(nchunks, n_fields), 256, 0, st>>>(tile_counts, tile_counts + (size_t)n_fields * ntiles, ntiles, nchunks);
+    k_chunk_scan<<<n_fields, 256, 0, st>>>(tile_counts + (size_t)n_fields * ntiles, nchunks);
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return e;
+    k_compact_focus<<<dim3(ntiles, n_fields), ORT_TILE, 0, st>>>(C, n_foci);
     return cudaGetLastError();
 }
 

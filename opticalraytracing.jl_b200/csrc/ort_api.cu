@@ -109,6 +109,8 @@ int ort_init(ort_ctx** out, int device)
     for (int v = 0; v < 5; v++) {
         ctx->bps[ORT_ARITH_STRICT][v] = grid_blocks_per_sm(ORT_ARITH_STRICT, v);
         ctx->bps[ORT_ARITH_FAST][v] = grid_blocks_per_sm(ORT_ARITH_FAST, v);
+        ctx->bps_focus[ORT_ARITH_STRICT][v] = focus_blocks_per_sm(ORT_ARITH_STRICT, v);
+        ctx->bps_focus[ORT_ARITH_FAST][v] = focus_blocks_per_sm(ORT_ARITH_FAST, v);
     }
     *out = ctx;
     return ORT_OK;
@@ -604,6 +606,200 @@ int ort_trace3d_grid(ort_ctx* ctx, const ort_field* fields, int n_fields, const 
         if (out->stats) memcpy(out->stats, hmerged, sizeof(ort_stats) * (size_t)n_fields);
         if (out->stats_local) memcpy(out->stats_local, hstats, sizeof(ort_stats) * (size_t)n_fields);
     } else if (out->stats) memcpy(out->stats, hstats, sizeof(ort_stats) * (size_t)n_fields);
+    return ORT_OK;
+}
+
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------
+// through-focus sweep (k_focus): the grid sweep at n_foci image planes, every ray traced once
+// ------------------------------------------------------------------------------------------
+static int focus_check(ort_ctx* ctx, const ort_field* fields, int n_fields, const void* ys, int ny, const void* xs, int nx,
+                       int stop, const double* foci, int n_foci, const ort_opts* opts, const ort_grid_out* out)
+{
+    if (!ctx) return ORT_EINVAL;
+    if (!opts || !out) return fail(ctx, ORT_EINVAL, "trace3d_focus: opts/out is NULL");
+    if (opts->ext) return fail(ctx, ORT_EUNSUPPORTED, "trace3d_focus: opts.ext = %d (no OPD / vignetting through focus)", opts->ext);
+    if (opts->gather_stats) return fail(ctx, ORT_EUNSUPPORTED, "trace3d_focus: opts.gather_stats is not supported");
+    if (ctx->have_layout && ctx->presc.poly) return fail(ctx, ORT_EUNSUPPORTED, "trace3d_focus: polynomial terms are set on the context");
+    const int rc = grid_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, opts, out);
+    if (rc) return rc;
+    if (n_foci < 1 || n_foci > ORT_MAX_FOCI) return fail(ctx, ORT_EINVAL, "trace3d_focus: n_foci = %d not in [1, %d]", n_foci, ORT_MAX_FOCI);
+    if (!foci) return fail(ctx, ORT_EINVAL, "trace3d_focus: foci is NULL");
+    for (int j = 0; j < n_foci; j++)
+        if (!isfinite(foci[j])) return fail(ctx, ORT_EINVAL, "trace3d_focus: foci[%d] is not finite", j);
+    const Presc& P = ctx->presc;
+    const SurfK& S = P.s[P.nsurf - 1];
+    if (!isinf(S.R) || S.K != 0.0) return fail(ctx, ORT_EINVAL, "trace3d_focus: the last row of the layout is not a plane");
+    if (stop > P.nsurf - 1) return fail(ctx, ORT_EINVAL, "trace3d_focus: stop = %d is the image plane (at most %d)", stop, P.nsurf - 1);
+    if (out->wx || out->wy || out->opd || out->stats_local)
+        return fail(ctx, ORT_EINVAL, "trace3d_focus: wx, wy, opd and stats_local must be NULL");
+    return ORT_OK;
+}
+
+// CTAs along x of a k_focus launch: ort_grid_dims's rule (8 waves, >= 16 tiles per CTA, <= 32 000 rays per thread for the
+// 16-bit flag counters) with k_focus's own rays per thread and resident CTAs/SM
+static int focus_dims(const ort_ctx* ctx, int arith, int n_fields, unsigned NN)
+{
+    const int variant = grid_variant(ctx->presc, arith, 0);
+    const unsigned nsub = (NN + ORT_TILE - 1) / ORT_TILE;
+    const unsigned rpt = (unsigned)grid_rays_per_thread(arith, variant);
+    const unsigned ntiles = (nsub + rpt - 1) / rpt;
+    long long slots = (long long)ctx->sm_count * ctx->bps_focus[arith][variant] / n_fields;
+    if (slots < 1) slots = 1;
+    long long gx = (long long)ntiles / 16;
+    if (gx < slots) gx = slots;
+    if (gx > slots * ORT_GRID_WAVES_DEFAULT) gx = slots * ORT_GRID_WAVES_DEFAULT;
+    const long long gmin = ((long long)nsub + 31999) / 32000;
+    if (gx < gmin) gx = gmin;
+    if (gx > (long long)ntiles) gx = ntiles;
+    if (gx < 1) gx = 1;
+    return (int)gx;
+}
+
+// k_focus + k_grid_finalize over n_fields * n_foci records (+ scan and compaction once when dst is given) on `st`
+static int focus_enqueue(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* d_ys, int ny, const double* d_xs,
+                         int nx, int stop, double a_stop, const double* foci, int n_foci, const ort_opts* opts,
+                         const ort_grid_out& full, const ort_grid_out* dst, ort_stats* d_stats, RawPart* d_partials,
+                         int* d_tiles, int gx, cudaStream_t st)
+{
+    const unsigned NN = (unsigned)((long long)ny * nx);
+    FocusArgs F;
+    memset(&F, 0, sizeof F);
+    GridArgs& A = F.G;
+    A.ys = d_ys; A.xs = d_xs; A.ny = ny; A.nx = nx; A.NN = NN; A.stop = stop;
+    A.ys_stride = opts->ys_per_field ? ny : 0;
+    A.a_stop = a_stop; A.a_stop2 = a_stop * a_stop;
+    A.ex = full.ex; A.ey = full.ey; A.r = full.r; A.theta = full.theta;
+    A.mask = full.mask; A.flags = full.flags;
+    A.partials = d_partials;
+    A.tile_counts = dst ? d_tiles : nullptr;
+    memcpy(A.fields, fields, sizeof(ort_field) * (size_t)n_fields);
+    F.n_foci = n_foci;
+    F.t_lo = F.t_hi = foci[0];
+    for (int j = 0; j < n_foci; j++) {
+        F.foci[j] = foci[j];
+        F.t_lo = fmin(F.t_lo, foci[j]); F.t_hi = fmax(F.t_hi, foci[j]);
+    }
+    const int arith = resolve_arith(ctx, opts->arith);
+    const int nrec = n_fields * n_foci;
+    if (NN > 0) {
+        ProfScope prof(ctx, st);
+        CK(launch_focus(ctx->presc, F, arith, dim3((unsigned)gx, (unsigned)n_fields), st));
+        ctx->launches++;
+    } else {
+        CK(cudaMemsetAsync(d_partials, 0, sizeof(RawPart) * (size_t)gx * nrec, st));
+    }
+    CK(launch_grid_finalize(d_partials, gx, nrec, d_stats, st));
+    ctx->launches++;
+    if (dst && NN > 0) {
+        CompactArgs C;
+        memset(&C, 0, sizeof C);
+        C.NN = NN; C.mask = full.mask; C.tile_offsets = d_tiles;
+        const double* src[4] = {full.ex, full.ey, full.r, full.theta};
+        double* dd[4] = {dst->ex, dst->ey, dst->r, dst->theta};
+        for (int a = 0; a < 4; a++) { C.src[a] = dd[a] ? src[a] : nullptr; C.dst[a] = dd[a]; }
+        CK(launch_compact_focus(d_tiles, C, n_fields, n_foci, st));
+        ctx->launches += 3;
+    }
+    return ORT_OK;
+}
+
+extern "C" {
+
+int ort_trace3d_focus_dev(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* d_ys, int ny,
+                          const double* d_xs, int nx, int stop, double a_stop, const double* foci, int n_foci,
+                          const ort_opts* opts, const ort_grid_out* d_out, void* stream)
+{
+    int rc = focus_check(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, foci, n_foci, opts, d_out);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    ScratchScope scratch(ctx, st);                  // before the first ENSURE: a poisoning memset is ordered like the work
+    const unsigned NN = (unsigned)((long long)ny * nx);
+    const int arith = resolve_arith(ctx, opts->arith);
+    const int gx = focus_dims(ctx, arith, n_fields, NN);
+    const size_t nrec = (size_t)n_fields * n_foci;
+    RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * nrec, d_partials);
+    ort_stats* d_stats = d_out->stats;
+    if (!d_stats) ENSURE(SL_STATS, sizeof(ort_stats) * nrec, d_stats);
+    if (!opts->compact)
+        return focus_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, n_foci, opts, *d_out, nullptr,
+                             d_stats, d_partials, nullptr, gx, st);
+    // compaction: trace into scratch, scatter into the caller's arrays
+    const size_t tot = (size_t)NN * n_fields;
+    ort_grid_out full = *d_out;
+    if (d_out->ex) ENSURE(SL_EX, tot * n_foci * 8, full.ex);
+    if (d_out->ey) ENSURE(SL_EY, tot * n_foci * 8, full.ey);
+    if (d_out->r) ENSURE(SL_R, tot * 8, full.r);
+    if (d_out->theta) ENSURE(SL_TH, tot * 8, full.theta);
+    if (!d_out->mask) ENSURE(SL_MASK, tot, full.mask);
+    const size_t ntiles = (size_t)(NN + ORT_TILE - 1) / ORT_TILE;
+    int* d_tiles; ENSURE(SL_TILES, sizeof(int) * (ntiles + ntiles / 2048 + 2) * n_fields, d_tiles);
+    return focus_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, n_foci, opts, full, d_out, d_stats,
+                         d_partials, d_tiles, gx, st);
+}
+
+int ort_trace3d_focus(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* ys, int ny,
+                      const double* xs, int nx, int stop, double a_stop, const double* foci, int n_foci,
+                      const ort_opts* opts, ort_grid_out* out)
+{
+    int rc = focus_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, foci, n_foci, opts, out);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    ScratchScope scratch(ctx, st);                  // before the first ENSURE (see ort_trace3d_focus_dev)
+    const unsigned NN = (unsigned)((long long)ny * nx);
+    const size_t tot = (size_t)NN * n_fields, nrec = (size_t)n_fields * n_foci;
+    const int arith = resolve_arith(ctx, opts->arith);
+    const int gx = focus_dims(ctx, arith, n_fields, NN);
+    const size_t nys = (size_t)ny * (opts->ys_per_field ? n_fields : 1);
+    double *d_ys, *d_xs;
+    ENSURE(SL_YS, sizeof(double) * nys, d_ys);
+    ENSURE(SL_XS, sizeof(double) * (size_t)nx, d_xs);
+    RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * nrec, d_partials);
+    ort_stats* d_stats; ENSURE(SL_STATS, sizeof(ort_stats) * nrec, d_stats);
+    ort_grid_out full; memset(&full, 0, sizeof full);
+    ort_grid_out comp; memset(&comp, 0, sizeof comp);
+    if (out->ex) ENSURE(SL_EX, tot * n_foci * 8, full.ex);
+    if (out->ey) ENSURE(SL_EY, tot * n_foci * 8, full.ey);
+    if (out->r) ENSURE(SL_R, tot * 8, full.r);
+    if (out->theta) ENSURE(SL_TH, tot * 8, full.theta);
+    if (out->mask || opts->compact) ENSURE(SL_MASK, tot, full.mask);
+    if (out->flags) ENSURE(SL_FLAGS, tot, full.flags);
+    int* d_tiles = nullptr;
+    if (opts->compact) {
+        const size_t ntiles = (size_t)(NN + ORT_TILE - 1) / ORT_TILE;
+        ENSURE(SL_TILES, sizeof(int) * (ntiles + ntiles / 2048 + 2) * n_fields, d_tiles);
+        if (out->ex) ENSURE(SL_CEX, tot * n_foci * 8, comp.ex);
+        if (out->ey) ENSURE(SL_CEY, tot * n_foci * 8, comp.ey);
+        if (out->r) ENSURE(SL_CR, tot * 8, comp.r);
+        if (out->theta) ENSURE(SL_CTH, tot * 8, comp.theta);
+    }
+    CK(cudaMemcpyAsync(d_ys, ys, sizeof(double) * nys, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_xs, xs, sizeof(double) * (size_t)nx, cudaMemcpyHostToDevice, st));
+    rc = focus_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, n_foci, opts, full,
+                       opts->compact ? &comp : nullptr, d_stats, d_partials, d_tiles, gx, st);
+    if (rc) return rc;
+    std::vector<ort_stats> hstats(nrec);
+    CK(cudaMemcpyAsync(hstats.data(), d_stats, sizeof(ort_stats) * nrec, cudaMemcpyDeviceToHost, st));
+    if (opts->compact) CK(cudaStreamSynchronize(st));                          // counts needed for the copy sizes
+    const ort_grid_out& src = opts->compact ? comp : full;
+    if (out->mask) CK(cudaMemcpyAsync(out->mask, full.mask, tot, cudaMemcpyDeviceToHost, st));
+    if (out->flags) CK(cudaMemcpyAsync(out->flags, full.flags, tot, cudaMemcpyDeviceToHost, st));
+    for (int f = 0; f < n_fields; f++) {
+        const size_t o = (size_t)f * NN;
+        const size_t cnt = opts->compact ? (size_t)hstats[(size_t)f * n_foci].n_kept : (size_t)NN;
+        if (out->r) CK(cudaMemcpyAsync(out->r + o, src.r + o, cnt * 8, cudaMemcpyDeviceToHost, st));
+        if (out->theta) CK(cudaMemcpyAsync(out->theta + o, src.theta + o, cnt * 8, cudaMemcpyDeviceToHost, st));
+        for (int j = 0; j < n_foci; j++) {
+            const size_t oj = ((size_t)f * n_foci + j) * NN;
+            if (out->ex) CK(cudaMemcpyAsync(out->ex + oj, src.ex + oj, cnt * 8, cudaMemcpyDeviceToHost, st));
+            if (out->ey) CK(cudaMemcpyAsync(out->ey + oj, src.ey + oj, cnt * 8, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    CK(cudaStreamSynchronize(st));
+    if (out->stats) memcpy(out->stats, hstats.data(), sizeof(ort_stats) * nrec);
     return ORT_OK;
 }
 

@@ -31,6 +31,7 @@ struct ort_ctx {
     bool have_layout;
     int fast_ok_layout;         // fast_ok as derived from R, t, n, K alone (polynomial terms force it to 0 while set)
     int bps[2][5];              // resident CTAs/SM of k_grid<STRICT|FAST, variant general|EXT|SIMPLE|SIMPLE x EXT|SIMPLE-conic> (grid_variant)
+    int bps_focus[2][5];        // the same for k_focus (variants 0, 2, 4; 1 and 3 unused)
     void* slot[SL_COUNT];
     size_t slot_bytes[SL_COUNT];
     // The scratch slots are shared by every entry point of the context.  Work that uses them is ordered across streams

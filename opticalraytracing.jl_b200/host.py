@@ -720,6 +720,83 @@ def full_trace_fields(surfaces, system, Hs, k_rays=SPOT_RAYS, focus=None, backen
     return out
 
 
+@dataclass
+class ThroughFocus:
+    """EXTENSION (no reference type): the spot of one field point through focus.  foci are image-plane distances from
+    the last lens vertex, full_trace's `focus` (src/PupilSampling.jl:85,111-114); rms[j] is the RealRayError RMS of
+    full_trace(..., focus = foci[j]).  The kept set is the same at every focus, so the mirrored sigma^2 is exactly
+    quadratic in the focus: best_focus / best_rms are the vertex of its least-squares parabola over all foci (NaN with
+    fewer than 3 distinct foci or a parabola that does not open upwards); bracketed: min(foci) <= best_focus <= max(foci)."""
+    H: float
+    foci: np.ndarray
+    rms: np.ndarray
+    n_kept: int
+    stats: np.ndarray = field(repr=False)
+    best_focus: float
+    best_rms: float
+    bracketed: bool
+    spots: Optional[list] = field(default=None, repr=False)    # per focus (x, y), mirrored as in RealRayError
+
+
+def best_focus_fit(foci, rms):
+    """vertex of the least-squares parabola sigma^2 = A d^2 + B d + C, d = f - mean(foci) -> (best_focus, best_rms)"""
+    f = np.asarray(foci, dtype=np.float64)
+    s2 = np.asarray(rms, dtype=np.float64) ** 2
+    if len(np.unique(f)) < 3 or not np.all(np.isfinite(s2)):
+        return float("nan"), float("nan")
+    fm = float(f.mean())
+    d = f - fm
+    (A, B, Cc), *_ = np.linalg.lstsq(np.column_stack([d * d, d, np.ones_like(d)]), s2, rcond=None)
+    if not A > 0.0:
+        return float("nan"), float("nan")
+    return fm - B / (2.0 * A), math.sqrt(max(Cc - B * B / (4.0 * A), 0.0))
+
+
+def through_focus(surfaces, system, Hs, foci, k_rays=SPOT_RAYS, spots=False, backend=None, arith=_lib.FAST):
+    """EXTENSION: full_trace's spot at every focus of `foci` for every field point of Hs, each pupil grid traced once
+    (ort_trace3d_focus: one device call for all fields and foci, chunked by MAX_FIELDS) -> list of ThroughFocus.
+    Equivalent to full_trace_fields(surfaces, system, Hs, k_rays, focus=f) at each f, except that a ray whose image
+    position is NaN at one focus is dropped at all of them (only a ray with k3 = 0 after the last surface can be)."""
+    be = _be(backend)
+    layout = _as_layout(surfaces)
+    if layout.P is not None:
+        raise NotImplementedError("through_focus: polynomial terms are not supported (ort_trace3d_focus rejects them)")
+    foci = np.atleast_1d(np.asarray(foci, dtype=np.float64))
+    if foci.ndim != 1 or not 1 <= len(foci) <= _lib.MAX_FOCI:
+        raise ValueError(f"through_focus: between 1 and {_lib.MAX_FOCI} foci")
+    if not np.all(np.isfinite(foci)):
+        raise ValueError("through_focus: foci must be finite")
+    p = _full_trace_setup(layout, system, Hs, k_rays, None, backend)
+    be.set_layout(p["ext"], p["K"])
+    k2 = k_rays // 2                                                             # :116
+    xs = jl_range(0.0, p["y_EP"], k2)                                            # :122
+    ys = np.stack([jl_range(p["y1"][j], p["y2"][j], k_rays) for j in range(len(p["Hs"]))])      # :121
+    if p["z0"] is None:
+        flds = [dict(mode=0, u=float(p["u"][j]), v=math.tan(0.0), h_prime=float(p["h_prime"][j]))
+                for j in range(len(p["Hs"]))]
+    else:
+        flds = [dict(mode=1, ybar=float(p["ybar"]), z0=float(p["z0"]), h_prime=float(p["h_prime"][j]))
+                for j in range(len(p["Hs"]))]
+    want = ("ex", "ey", "stats") if spots else ("stats",)
+    out = []
+    for j0 in range(0, len(flds), _lib.MAX_FIELDS):
+        sl = slice(j0, j0 + _lib.MAX_FIELDS)
+        r = be.trace3d_focus(flds[sl], ys[sl], xs, p["stop"], p["a_stop"], foci, arith=arith, compact=spots,
+                            want=want)            # statistics only: no compaction, two launches
+        for j, H in enumerate(p["Hs"][sl]):
+            st = r["stats"][j].copy()
+            rms = np.array([rms_from_stats(st[m]) for m in range(len(foci))])
+            n = int(st[0]["n_kept"])
+            bf, br = best_focus_fit(foci, rms)
+            sp = None
+            if spots:
+                sp = [(np.concatenate([r["ex"][j][m][:n], -r["ex"][j][m][:n]]), np.concatenate([r["ey"][j][m][:n]] * 2))
+                      for m in range(len(foci))]
+            out.append(ThroughFocus(float(H), foci.copy(), rms, n, st, bf, br,
+                                    bool(foci.min() <= bf <= foci.max()), sp))
+    return out
+
+
 def _mirror(r, f, nu, H):
     """take advantage of symmetry -- src/PupilSampling.jl:139-146; RMS = sigma(:169-173) evaluated
     from the kernel's mergeable moments (mirrored x has mean exactly 0)."""
