@@ -80,6 +80,10 @@ class GridOut(C.Structure):
                 ("flags", C.c_void_p), ("stats", C.c_void_p), ("stats_local", C.c_void_p)]
 
 
+GRID_OUT_NAMES = tuple(name for name, _ in GridOut._fields_)
+RAY_OUT_NAMES = GRID_OUT_NAMES[:9]          # the per-ray members: every one but the statistics records
+
+
 _lib = None
 
 
@@ -264,23 +268,12 @@ def trace3d_grid_multi(contexts, fields, ys, xs, stop, a_stop, arith=FAST, compa
     if per_field and ys.shape[0] != nf:
         raise ValueError("ys must be (ny,) or (n_fields, ny)")
     ny, nx = ys.shape[-1], len(xs)
-    NN = ny * nx
-    res = dict(out) if out else {}
     if "opd" in want:
         ext |= EXT_OPD
-    for name in ("ex", "ey", "r", "theta", "wx", "wy", "opd"):
-        if name in want and name not in res:
-            res[name] = np.empty((nf, NN), dtype=np.float64)
-    for name in ("mask", "flags"):
-        if name in want and name not in res:
-            res[name] = np.zeros((nf, NN), dtype=np.uint8)
     stats = np.zeros(nf, dtype=STATS_DTYPE)
     local = np.zeros((len(contexts), nf), dtype=STATS_DTYPE)
-    go = GridOut(*[(res[k].ctypes.data if k in res and res[k] is not None else None)
-                   for k in ("ex", "ey", "r", "theta", "wx", "wy", "opd", "mask", "flags")],
-                 stats.ctypes.data, local.ctypes.data)
-    nu, lam = wavegrad if wavegrad else (0.0, 1.0)
-    op = Opts(int(arith), int(bool(compact)), int(per_field), int(ext), float(nu), float(lam), float(opd_scale), 0, 0)
+    res, go = _host_out(want, out, nf, ny * nx, stats, local)
+    op = _opts(arith, compact, per_field, ext, wavegrad, opd_scale)
     arr = (C.c_void_p * len(contexts))(*[c.h for c in contexts])
     rc = L.ort_trace3d_grid_multi(arr, len(contexts), farr, nf, _vp(ys), ny, _vp(xs), nx, int(stop), float(a_stop),
                                   C.byref(op), C.byref(go))
@@ -288,6 +281,27 @@ def trace3d_grid_multi(contexts, fields, ys, xs, stop, a_stop, arith=FAST, compa
         raise OrtError(rc, L.ort_last_error(contexts[0].h).decode())
     res["stats"], res["stats_local"] = stats, local
     return res
+
+
+def _host_out(want, out, nf, NN, stats, local=None, foci=None):
+    """The result dict of a host-pointer sweep and the GridOut over it: the arrays of `out`, and new ones for the other
+    per-ray members named in `want`, (n_fields, ny*nx) each.  foci = M: a through-focus sweep, whose ex, ey are
+    (n_fields, M, ny*nx) and which has no wx, wy, opd."""
+    res = dict(out) if out else {}
+    for name in RAY_OUT_NAMES:
+        if name not in want or name in res or (foci is not None and name in ("wx", "wy", "opd")):
+            continue
+        shape = (nf, foci, NN) if foci is not None and name in ("ex", "ey") else (nf, NN)
+        res[name] = np.zeros(shape, dtype=np.uint8) if name in ("mask", "flags") else np.empty(shape, dtype=np.float64)
+    go = GridOut(*[(res[k].ctypes.data if res.get(k) is not None else None) for k in RAY_OUT_NAMES],
+                 stats.ctypes.data, None if local is None else local.ctypes.data)
+    return res, go
+
+
+def _opts(arith, compact, ys_per_field, ext=0, wavegrad=None, opd_scale=1.0, gather=False):
+    nu, lam = wavegrad if wavegrad else (0.0, 1.0)
+    return Opts(int(arith), int(bool(compact)), int(bool(ys_per_field)), int(ext), float(nu), float(lam), float(opd_scale),
+                int(bool(gather)), 0)
 
 
 def make_fields(fields):
@@ -455,24 +469,12 @@ class Context:
         if per_field and ys.shape[0] != nf:
             raise ValueError("ys must be (ny,) or (n_fields, ny)")
         ny, nx = ys.shape[-1], len(xs)
-        NN = ny * nx
-        res = dict(out) if out else {}
         if "opd" in want:
             ext |= EXT_OPD
-        for name in ("ex", "ey", "r", "theta", "wx", "wy", "opd"):
-            if name in want and name not in res:
-                res[name] = np.empty((nf, NN), dtype=np.float64)
-        for name in ("mask", "flags"):
-            if name in want and name not in res:
-                res[name] = np.zeros((nf, NN), dtype=np.uint8)
         stats = np.zeros(nf, dtype=STATS_DTYPE)
         local = np.zeros(nf, dtype=STATS_DTYPE) if gather else None
-        go = GridOut(*[(res[k].ctypes.data if k in res and res[k] is not None else None)
-                       for k in ("ex", "ey", "r", "theta", "wx", "wy", "opd", "mask", "flags")],
-                     stats.ctypes.data, local.ctypes.data if gather else None)
-        nu, lam = wavegrad if wavegrad else (0.0, 1.0)
-        op = Opts(int(arith), int(bool(compact)), int(per_field), int(ext), float(nu), float(lam), float(opd_scale),
-                  int(bool(gather)), 0)
+        res, go = _host_out(want, out, nf, ny * nx, stats, local)
+        op = _opts(arith, compact, per_field, ext, wavegrad, opd_scale, gather)
         self._ck(self.L.ort_trace3d_grid(self.h, farr, nf, _vp(ys), ny, _vp(xs), nx, int(stop),
                                          float(a_stop), C.byref(op), C.byref(go)))
         res["stats"] = stats
@@ -486,13 +488,10 @@ class Context:
         merge of the statistics records over the communicator behind the sweep, on the same stream (ptrs['stats'] =
         merged, ptrs['stats_local'] = this rank's)."""
         farr, nf = make_fields(fields)
-        go = GridOut(*[ptrs.get(k) for k in ("ex", "ey", "r", "theta", "wx", "wy", "opd", "mask", "flags", "stats",
-                                             "stats_local")])
+        go = GridOut(*[ptrs.get(k) for k in GRID_OUT_NAMES])
         if ptrs.get("opd"):
             ext |= EXT_OPD
-        nu, lam = wavegrad if wavegrad else (0.0, 1.0)
-        op = Opts(int(arith), int(bool(compact)), int(bool(ys_per_field)), int(ext), float(nu), float(lam),
-                  float(opd_scale), int(bool(gather)), 0)
+        op = _opts(arith, compact, ys_per_field, ext, wavegrad, opd_scale, gather)
         self._ck(self.L.ort_trace3d_grid_dev(self.h, farr, nf, C.c_void_p(d_ys), int(ny), C.c_void_p(d_xs),
                                              int(nx), int(stop), float(a_stop), C.byref(op), C.byref(go),
                                              C.c_void_p(stream)))
@@ -511,21 +510,9 @@ class Context:
         foci = _d(np.atleast_1d(foci))
         M = len(foci)
         ny, nx = ys.shape[-1], len(xs)
-        NN = ny * nx
-        res = {}
-        for name in ("ex", "ey"):
-            if name in want:
-                res[name] = np.empty((nf, M, NN), dtype=np.float64)
-        for name in ("r", "theta"):
-            if name in want:
-                res[name] = np.empty((nf, NN), dtype=np.float64)
-        for name in ("mask", "flags"):
-            if name in want:
-                res[name] = np.zeros((nf, NN), dtype=np.uint8)
         stats = np.zeros((nf, M), dtype=STATS_DTYPE)
-        go = GridOut(*[(res[k].ctypes.data if k in res else None)
-                       for k in ("ex", "ey", "r", "theta", "wx", "wy", "opd", "mask", "flags")], stats.ctypes.data, None)
-        op = Opts(int(arith), int(bool(compact)), int(per_field), 0, 0.0, 1.0, 1.0, 0, 0)
+        res, go = _host_out(want, None, nf, ny * nx, stats, foci=M)
+        op = _opts(arith, compact, per_field)
         self._ck(self.L.ort_trace3d_focus(self.h, farr, nf, _vp(ys), ny, _vp(xs), nx, int(stop), float(a_stop), _p(foci), M,
                                           C.byref(op), C.byref(go)))
         res["stats"] = stats
@@ -537,9 +524,8 @@ class Context:
         [n_fields][M][ny*nx], 'r', 'theta', 'mask', 'flags' [n_fields][ny*nx], 'stats' [n_fields][M]."""
         farr, nf = make_fields(fields)
         foci = _d(np.atleast_1d(foci))
-        go = GridOut(*[ptrs.get(k) for k in ("ex", "ey", "r", "theta", "wx", "wy", "opd", "mask", "flags", "stats",
-                                             "stats_local")])
-        op = Opts(int(arith), int(bool(compact)), int(bool(ys_per_field)), 0, 0.0, 1.0, 1.0, 0, 0)
+        go = GridOut(*[ptrs.get(k) for k in GRID_OUT_NAMES])
+        op = _opts(arith, compact, ys_per_field)
         self._ck(self.L.ort_trace3d_focus_dev(self.h, farr, nf, C.c_void_p(d_ys), int(ny), C.c_void_p(d_xs), int(nx),
                                               int(stop), float(a_stop), _p(foci), len(foci), C.byref(op), C.byref(go),
                                               C.c_void_p(stream)))

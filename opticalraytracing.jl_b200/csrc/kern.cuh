@@ -181,6 +181,8 @@ int grid_blocks_per_sm(int arith, int variant);
 cudaError_t launch_grid(const Presc& P, const GridArgs& A, int arith, dim3 grid, cudaStream_t st, const PolyK* Q = nullptr);
 cudaError_t launch_grid_finalize(const RawPart* partials, int nparts, int n_fields, ort_stats* stats,
                                  cudaStream_t st);
+// ints per field of the tile-count buffer of launch_compact / launch_compact_focus: the counts and the chunk totals
+size_t compact_tile_ints(unsigned NN);
 cudaError_t launch_compact(int* tile_counts, const CompactArgs& C, int n_fields, cudaStream_t st);
 int focus_blocks_per_sm(int arith, int variant);
 cudaError_t launch_focus(const Presc& P, const FocusArgs& F, int arith, dim3 grid, cudaStream_t st);

@@ -546,17 +546,16 @@ __global__ void __launch_bounds__(256) k_chunk_scan(int* chunk_tot, unsigned nch
     }
 }
 
-// order-preserving scatter of up to 7 arrays: one CTA per (tile, field)
-__global__ void __launch_bounds__(ORT_TILE) k_compact(CompactArgs C)
+// Index of thread tid's ray among the kept rays of field f (m: the ray is kept), in a compaction kernel of one CTA per
+// (tile, field).  Every thread of the CTA calls it: it synchronises the CTA.  The kernel passes tid = threadIdx.x and
+// ntiles: read or computed in here they compile to other code (threadIdx.x loses the bound of the kernel's launch
+// bounds, and the loop over the preceding warps unrolls differently: 30 registers instead of 22).
+__device__ __forceinline__ int compact_offset(const CompactArgs& C, unsigned tile, unsigned f, unsigned ntiles, unsigned tid,
+                                              int m)
 {
     __shared__ int s_warp[ORT_TILE / 32];
-    const unsigned tile = blockIdx.x, f = blockIdx.y;
-    const unsigned ntiles = (C.NN + ORT_TILE - 1) / ORT_TILE;
-    const unsigned i = tile * ORT_TILE + threadIdx.x;
-    const size_t fbase = (size_t)f * C.NN;
-    const int m = (i < C.NN) ? C.mask[fbase + i] : 0;
     const unsigned ball = __ballot_sync(0xffffffffu, m);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+    const int lane = tid & 31, warp = tid >> 5;
     if (lane == 0) s_warp[warp] = __popc(ball);
     __syncthreads();
     int off = C.tile_offsets[(size_t)f * ntiles + tile];
@@ -566,7 +565,18 @@ __global__ void __launch_bounds__(ORT_TILE) k_compact(CompactArgs C)
         off += ct[mychunk];
     }
     for (int w = 0; w < warp; w++) off += s_warp[w];
-    off += __popc(ball & ((1u << lane) - 1u));
+    return off + __popc(ball & ((1u << lane) - 1u));
+}
+
+// order-preserving scatter of up to 7 arrays: one CTA per (tile, field)
+__global__ void __launch_bounds__(ORT_TILE) k_compact(CompactArgs C)
+{
+    const unsigned tile = blockIdx.x, f = blockIdx.y;
+    const unsigned ntiles = (C.NN + ORT_TILE - 1) / ORT_TILE;
+    const unsigned i = tile * ORT_TILE + threadIdx.x;
+    const size_t fbase = (size_t)f * C.NN;
+    const int m = (i < C.NN) ? C.mask[fbase + i] : 0;
+    const int off = compact_offset(C, tile, f, ntiles, threadIdx.x, m);
     if (m) {
 #pragma unroll
         for (int a = 0; a < 7; a++)
@@ -927,24 +937,12 @@ k_focus(const __grid_constant__ Presc P, const __grid_constant__ FocusArgs F)
 // C.src / C.dst [0], [1] are ex, ey ([n_fields][n_foci][NN]); [2], [3] are r, theta ([n_fields][NN]).
 __global__ void __launch_bounds__(ORT_TILE) k_compact_focus(CompactArgs C, int n_foci)
 {
-    __shared__ int s_warp[ORT_TILE / 32];
     const unsigned tile = blockIdx.x, f = blockIdx.y;
     const unsigned ntiles = (C.NN + ORT_TILE - 1) / ORT_TILE;
     const unsigned i = tile * ORT_TILE + threadIdx.x;
     const size_t fbase = (size_t)f * C.NN;
     const int m = (i < C.NN) ? C.mask[fbase + i] : 0;
-    const unsigned ball = __ballot_sync(0xffffffffu, m);
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) s_warp[warp] = __popc(ball);
-    __syncthreads();
-    int off = C.tile_offsets[(size_t)f * ntiles + tile];
-    {
-        const unsigned nchunks = (ntiles + SCAN_CHUNK - 1) / SCAN_CHUNK, mychunk = tile / SCAN_CHUNK;
-        const int* ct = C.tile_offsets + (size_t)gridDim.y * ntiles + (size_t)f * nchunks;
-        off += ct[mychunk];
-    }
-    for (int w = 0; w < warp; w++) off += s_warp[w];
-    off += __popc(ball & ((1u << lane) - 1u));
+    const int off = compact_offset(C, tile, f, ntiles, threadIdx.x, m);
     if (m) {
         for (int a = 2; a < 4; a++)
             if (C.src[a]) C.dst[a][fbase + off] = C.src[a][fbase + i];
@@ -1477,14 +1475,25 @@ cudaError_t launch_grid_finalize(const RawPart* partials, int nparts, int n_fiel
     return cudaGetLastError();
 }
 
+size_t compact_tile_ints(unsigned NN)
+{
+    const size_t ntiles = (NN + ORT_TILE - 1) / ORT_TILE;
+    return ntiles + ntiles / SCAN_CHUNK + 2;
+}
+
+// the two scan levels over the [n_fields][ntiles] tile counts; the chunk totals live right behind them
+static cudaError_t launch_tile_scan(int* tile_counts, unsigned ntiles, int n_fields, cudaStream_t st)
+{
+    const unsigned nchunks = (ntiles + SCAN_CHUNK - 1) / SCAN_CHUNK;
+    k_tile_scan<<<dim3(nchunks, n_fields), 256, 0, st>>>(tile_counts, tile_counts + (size_t)n_fields * ntiles, ntiles, nchunks);
+    k_chunk_scan<<<n_fields, 256, 0, st>>>(tile_counts + (size_t)n_fields * ntiles, nchunks);
+    return cudaGetLastError();
+}
+
 cudaError_t launch_compact(int* tile_counts, const CompactArgs& C, int n_fields, cudaStream_t st)
 {
     const unsigned ntiles = (C.NN + ORT_TILE - 1) / ORT_TILE;
-    const unsigned nchunks = (ntiles + SCAN_CHUNK - 1) / SCAN_CHUNK;
-    // chunk totals live right behind the [n_fields][ntiles] counts (the API layer sizes the buffer for it)
-    k_tile_scan<<<dim3(nchunks, n_fields), 256, 0, st>>>(tile_counts, tile_counts + (size_t)n_fields * ntiles, ntiles, nchunks);
-    k_chunk_scan<<<n_fields, 256, 0, st>>>(tile_counts + (size_t)n_fields * ntiles, nchunks);
-    cudaError_t e = cudaGetLastError();
+    cudaError_t e = launch_tile_scan(tile_counts, ntiles, n_fields, st);
     if (e != cudaSuccess) return e;
     k_compact<<<dim3(ntiles, n_fields), ORT_TILE, 0, st>>>(C);
     return cudaGetLastError();
@@ -1522,10 +1531,7 @@ cudaError_t launch_focus(const Presc& P, const FocusArgs& F, int arith, dim3 gri
 cudaError_t launch_compact_focus(int* tile_counts, const CompactArgs& C, int n_fields, int n_foci, cudaStream_t st)
 {
     const unsigned ntiles = (C.NN + ORT_TILE - 1) / ORT_TILE;
-    const unsigned nchunks = (ntiles + SCAN_CHUNK - 1) / SCAN_CHUNK;
-    k_tile_scan<<<dim3(nchunks, n_fields), 256, 0, st>>>(tile_counts, tile_counts + (size_t)n_fields * ntiles, ntiles, nchunks);
-    k_chunk_scan<<<n_fields, 256, 0, st>>>(tile_counts + (size_t)n_fields * ntiles, nchunks);
-    cudaError_t e = cudaGetLastError();
+    cudaError_t e = launch_tile_scan(tile_counts, ntiles, n_fields, st);
     if (e != cudaSuccess) return e;
     k_compact_focus<<<dim3(ntiles, n_fields), ORT_TILE, 0, st>>>(C, n_foci);
     return cudaGetLastError();

@@ -3,6 +3,7 @@
 // entry points.  No torch types, no exceptions across the boundary, no CPU fallback.
 #include <math.h>
 #include <stdarg.h>
+#include <stddef.h>
 #include <stdio.h>
 #include <string.h>
 
@@ -49,7 +50,7 @@ int ort_ensure(ort_ctx* ctx, int id, size_t bytes, void** out)
     // SL_POLY is the one slot whose content outlives the call that fills it.
     static const bool poison = [] { const char* e = getenv("ORT_POISON_SCRATCH"); return e && atoi(e) != 0; }();
     if (poison && id != SL_POLY) {
-        cudaError_t e = cudaMemsetAsync(ctx->slot[id], 0xFF, bytes, ctx->scratch_now ? ctx->scratch_now : ctx->stream);
+        cudaError_t e = cudaMemsetAsync(ctx->slot[id], 0xFF, bytes, ctx->scratch_now);
         if (e != cudaSuccess) return fail(ctx, ORT_ECUDA, "poison memset -> %s", cudaGetErrorString(e));
     }
     return ORT_OK;
@@ -100,6 +101,7 @@ int ort_init(ort_ctx** out, int device)
     CKI(cudaSetDevice(device));
     CKI(cudaStreamCreateWithFlags(&ctx->stream, cudaStreamNonBlocking));
     CKI(cudaStreamCreateWithFlags(&ctx->copy_stream, cudaStreamNonBlocking));
+    ctx->scratch_now = ctx->stream;
     CKI(cudaEventCreate(&ctx->ev_a));
     CKI(cudaEventCreate(&ctx->ev_b));
     CKI(cudaEventCreateWithFlags(&ctx->ev_scratch, cudaEventDisableTiming));
@@ -356,7 +358,7 @@ int ort_set_apertures(ort_ctx* ctx, int n, const double* a)
 }  // extern "C"
 
 // ------------------------------------------------------------------------------------------
-// pupil-grid sweep
+// pupil-grid sweep (k_grid) and through-focus sweep (k_focus)
 // ------------------------------------------------------------------------------------------
 int ort_grid_check(ort_ctx* ctx, const ort_field* fields, int n_fields, const void* ys, int ny,
                       const void* xs, int nx, int stop, const ort_opts* opts, const ort_grid_out* out)
@@ -376,17 +378,98 @@ int ort_grid_check(ort_ctx* ctx, const ort_field* fields, int n_fields, const vo
     return ORT_OK;
 }
 
-// Enqueue trace (+ compaction) + finalize for fields [0, n_fields) on `st`.  All pointers are
-// device pointers.  `full` receives the full-grid trace outputs; when compacting, `full` is
-// scratch and `dst` the compacted destination.
+// The per-ray members of ort_grid_out and how a sweep stores them.  The compacted members come first, in the index order
+// of CompactArgs.src / dst; mask and flags always cover the full grid.  A per-focus member of a through-focus sweep holds
+// one block of NN rays per (field, focus), [n_fields][n_foci][NN].
+struct OutMember {
+    size_t off;                 // offsetof in ort_grid_out
+    int slot, cslot;            // scratch slots of the full-grid and of the compacted array
+    size_t bytes;               // per ray
+    bool compacted, per_focus;
+};
+static const OutMember k_members[] = {
+    {offsetof(ort_grid_out, ex), SL_EX, SL_CEX, 8, true, true},
+    {offsetof(ort_grid_out, ey), SL_EY, SL_CEY, 8, true, true},
+    {offsetof(ort_grid_out, r), SL_R, SL_CR, 8, true, false},
+    {offsetof(ort_grid_out, theta), SL_TH, SL_CTH, 8, true, false},
+    {offsetof(ort_grid_out, wx), SL_WX, SL_CWX, 8, true, false},
+    {offsetof(ort_grid_out, wy), SL_WY, SL_CWY, 8, true, false},
+    {offsetof(ort_grid_out, opd), SL_OPD, SL_COPD, 8, true, false},
+    {offsetof(ort_grid_out, mask), SL_MASK, -1, 1, false, false},
+    {offsetof(ort_grid_out, flags), SL_FLAGS, -1, 1, false, false},
+};
+static const int N_COMPACTED = 7;
+static_assert(sizeof(CompactArgs::src) / sizeof(CompactArgs::src[0]) == N_COMPACTED, "one CompactArgs entry per compacted member");
+
+static char* member(const ort_grid_out& o, const OutMember& m) { char* p; memcpy(&p, (const char*)&o + m.off, sizeof p); return p; }
+static void set_member(ort_grid_out& o, const OutMember& m, void* p) { memcpy((char*)&o + m.off, &p, sizeof p); }
+
+// the members of a grid sweep's outputs from ray i of the first field on
+static ort_grid_out from_ray(const ort_grid_out& g, size_t i)
+{
+    ort_grid_out o = g;
+    for (const OutMember& m : k_members)
+        if (char* p = member(g, m)) set_member(o, m, p + i * m.bytes);
+    return o;
+}
+
+// Scratch of a sweep's per-ray outputs; call it inside the entry point's ScratchScope, so that a poisoning memset is
+// ordered like the work.  Host form (dev false): every member `out` wants is traced into its slot of *full -- the mask
+// also when compacting -- and, when compacting, scattered into its slot of *comp.  Device form: the caller's arrays are
+// the results (*full = *comp = *out); when compacting, the members that are compacted are traced into scratch, and so is
+// the mask when the caller gives none, while flags are written in place.  opd is wanted only with ORT_EXT_OPD.
+// *d_tiles: the tile counts of the compaction, or NULL.
+int ort_sweep_scratch(ort_ctx* ctx, const ort_grid_out* out, const ort_opts* opts, bool dev, unsigned NN, int n_fields,
+                      int n_foci, ort_grid_out* full, ort_grid_out* comp, int** d_tiles)
+{
+    *d_tiles = nullptr;
+    if (dev) { *full = *out; *comp = *out; }
+    else { memset(full, 0, sizeof *full); memset(comp, 0, sizeof *comp); }
+    if (dev && !opts->compact) return ORT_OK;
+    const size_t tot = (size_t)NN * n_fields;
+    for (const OutMember& m : k_members) {
+        const size_t bytes = tot * m.bytes * (m.per_focus ? n_foci : 1);
+        const bool want = member(*out, m) && (m.slot != SL_OPD || (opts->ext & ORT_EXT_OPD));
+        const bool mask = m.slot == SL_MASK;
+        const bool traced = dev ? (m.compacted ? want : mask && !want) : want || (mask && opts->compact);
+        void* p = nullptr;
+        if (traced) ENSURE(m.slot, bytes, p);
+        if (traced || (dev && m.compacted)) set_member(*full, m, p);
+        if (!dev && opts->compact && m.compacted && want) { ENSURE(m.cslot, bytes, p); set_member(*comp, m, p); }
+    }
+    if (opts->compact) ENSURE(SL_TILES, sizeof(int) * compact_tile_ints(NN) * n_fields, *d_tiles);
+    return ORT_OK;
+}
+
+// Device-to-host copies on `st` of one kind of member -- the compacted kind (rays) or mask and flags -- that `out` wants
+// and `src` holds: n rays from ray src_o of src to ray dst_o of out, offsets of a per-field array.  A per-focus member
+// copies its n_foci blocks of the field, block j from / to ray o * n_foci + j * NN.
+int ort_copy_out(ort_ctx* ctx, const ort_grid_out* out, const ort_grid_out& src, bool rays, size_t dst_o, size_t src_o,
+                 size_t n, int n_foci, unsigned NN, cudaStream_t st)
+{
+    for (const OutMember& m : k_members) {
+        char *d = member(*out, m), *s = member(src, m);
+        if (m.compacted != rays || !d || !s) continue;
+        const size_t nb = m.per_focus ? (size_t)n_foci : 1;
+        for (size_t j = 0; j < nb; j++)
+            CK(cudaMemcpyAsync(d + (dst_o * nb + j * NN) * m.bytes, s + (src_o * nb + j * NN) * m.bytes, n * m.bytes,
+                               cudaMemcpyDeviceToHost, st));
+    }
+    return ORT_OK;
+}
+
+// Enqueue on `st` the sweep of fields [0, n_fields): k_grid, or with foci k_focus at n_foci image planes; then
+// k_grid_finalize over the n_fields * n_foci records and, when dst is given, the tile scan and the compaction of the
+// members of `full` that dst holds.  All pointers are device pointers; a grid sweep passes foci = NULL, n_foci = 1.
 int ort_grid_enqueue(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* d_ys, int ny,
-                        const double* d_xs, int nx, int stop, double a_stop, const ort_opts* opts,
-                        const ort_grid_out& full, const ort_grid_out* dst, ort_stats* d_stats,
+                        const double* d_xs, int nx, int stop, double a_stop, const double* foci, int n_foci,
+                        const ort_opts* opts, const ort_grid_out& full, const ort_grid_out* dst, ort_stats* d_stats,
                         RawPart* d_partials, int* d_tiles, int gx, cudaStream_t st)
 {
     const unsigned NN = (unsigned)((long long)ny * nx);
-    GridArgs A;
-    memset(&A, 0, sizeof A);
+    FocusArgs F;
+    memset(&F, 0, sizeof F);
+    GridArgs& A = F.G;
     A.ys = d_ys; A.xs = d_xs; A.ny = ny; A.nx = nx; A.NN = NN; A.stop = stop;
     A.ys_stride = opts->ys_per_field ? ny : 0;
     A.a_stop = a_stop; A.a_stop2 = a_stop * a_stop;
@@ -398,43 +481,63 @@ int ort_grid_enqueue(ort_ctx* ctx, const ort_field* fields, int n_fields, const 
     A.partials = d_partials;
     A.tile_counts = dst ? d_tiles : nullptr;
     memcpy(A.fields, fields, sizeof(ort_field) * (size_t)n_fields);
+    if (foci) {
+        F.n_foci = n_foci;
+        F.t_lo = F.t_hi = foci[0];
+        for (int j = 0; j < n_foci; j++) {
+            F.foci[j] = foci[j];
+            F.t_lo = fmin(F.t_lo, foci[j]); F.t_hi = fmax(F.t_hi, foci[j]);
+        }
+    }
     const int arith = resolve_arith(ctx, opts->arith);
+    const int nrec = n_fields * n_foci;
+    const dim3 grid((unsigned)gx, (unsigned)n_fields);
     if (NN > 0) {
         ProfScope prof(ctx, st);
-        CK(launch_grid(ctx->presc, A, arith, dim3((unsigned)gx, (unsigned)n_fields), st, ctx->have_polyk ? &ctx->polyk : nullptr));
+        CK(foci ? launch_focus(ctx->presc, F, arith, grid, st)
+                : launch_grid(ctx->presc, A, arith, grid, st, ctx->have_polyk ? &ctx->polyk : nullptr));
         ctx->launches++;
     } else {
-        CK(cudaMemsetAsync(d_partials, 0, sizeof(RawPart) * (size_t)gx * n_fields, st));
+        CK(cudaMemsetAsync(d_partials, 0, sizeof(RawPart) * (size_t)gx * nrec, st));
     }
-    CK(launch_grid_finalize(d_partials, gx, n_fields, d_stats, st));
+    CK(launch_grid_finalize(d_partials, gx, nrec, d_stats, st));
     ctx->launches++;
     if (dst && NN > 0) {
         CompactArgs C;
         memset(&C, 0, sizeof C);
         C.NN = NN; C.mask = full.mask; C.tile_offsets = d_tiles;
-        const double* src[7] = {full.ex, full.ey, full.r, full.theta, full.wx, full.wy, A.opd};
-        double* dd[7] = {dst->ex, dst->ey, dst->r, dst->theta, dst->wx, dst->wy, A.opd ? dst->opd : nullptr};
-        for (int a = 0; a < 7; a++) { C.src[a] = dd[a] ? src[a] : nullptr; C.dst[a] = dd[a]; }
-        CK(launch_compact(d_tiles, C, n_fields, st));
+        for (int a = 0; a < N_COMPACTED; a++) {
+            const OutMember& m = k_members[a];
+            if (member(full, m) && member(*dst, m)) { C.src[a] = (const double*)member(full, m); C.dst[a] = (double*)member(*dst, m); }
+        }
+        CK(foci ? launch_compact_focus(d_tiles, C, n_fields, n_foci, st) : launch_compact(d_tiles, C, n_fields, st));
         ctx->launches += 3;
     }
     return ORT_OK;
 }
 
-int ort_grid_dims(const ort_ctx* ctx, int arith, int ext, int n_fields, unsigned NN)
+// Several waves of CTAs instead of one persistent wave: the warp schedulers favour the older of the resident CTAs, so
+// with one wave of equal shares the CTAs of an SM finish far apart and the SM idles at half occupancy in between
+// (ncu: 3.4 of 4 warps per scheduler active on average).  With 8 waves the block scheduler refills the slot:
+// 2.23 ms vs 2.34 (4, 16 waves: 2.25, 2.23; 32: 2.26 -- every CTA first traces its field's centre ray).
+// ORT_GRID_WAVES overrides the grid sweep's count (tuning).
+int ort_grid_waves()
 {
-    const int variant = grid_variant(ctx->presc, arith, ext);
+    static const int waves = [] { const char* e = getenv("ORT_GRID_WAVES"); const int w = e ? atoi(e) : ORT_GRID_WAVES_DEFAULT; return w < 1 ? 1 : w; }();
+    return waves;
+}
+
+// CTAs along x of a sweep launch: at most `waves` waves of the resident CTAs/SM in bps (ctx->bps for k_grid,
+// ctx->bps_focus for k_focus).  A CTA keeps at least 16 tiles so that its prologue stays amortised; the per-CTA partial
+// sums still belong to a fixed set of tiles, so the statistics stay bit-reproducible.
+int ort_grid_dims(const ort_ctx* ctx, const int (&bps)[2][5], int waves, const ort_opts* opts, int n_fields, unsigned NN)
+{
+    const int arith = resolve_arith(ctx, opts->arith);
+    const int variant = grid_variant(ctx->presc, arith, (opts->ext & 3) || ctx->presc.poly);
     const unsigned nsub = (NN + ORT_TILE - 1) / ORT_TILE;
     const unsigned rpt = (unsigned)grid_rays_per_thread(arith, variant);
     const unsigned ntiles = (nsub + rpt - 1) / rpt;
-    // Several waves of CTAs instead of one persistent wave: the warp schedulers favour the older of the resident CTAs, so
-    // with one wave of equal shares the CTAs of an SM finish far apart and the SM idles at half occupancy in between
-    // (ncu: 3.4 of 4 warps per scheduler active on average).  With 8 waves the block scheduler refills the slot:
-    // 2.23 ms vs 2.34 (4, 16 waves: 2.25, 2.23; 32: 2.26 -- every CTA first traces its field's centre ray).  A CTA
-    // keeps at least 16 tiles so that prologue stays amortised; the per-CTA partial sums still belong to a fixed set
-    // of tiles, so the statistics stay bit-reproducible.  ORT_GRID_WAVES overrides (tuning).
-    static const int waves = [] { const char* e = getenv("ORT_GRID_WAVES"); const int w = e ? atoi(e) : ORT_GRID_WAVES_DEFAULT; return w < 1 ? 1 : w; }();
-    long long slots = (long long)ctx->sm_count * ctx->bps[arith][variant] / n_fields;
+    long long slots = (long long)ctx->sm_count * bps[arith][variant] / n_fields;
     if (slots < 1) slots = 1;
     long long gx = (long long)ntiles / 16;
     if (gx < slots) gx = slots;
@@ -459,33 +562,16 @@ int ort_trace3d_grid_dev(ort_ctx* ctx, const ort_field* fields, int n_fields, co
     cudaStream_t st = (cudaStream_t)stream;
     ScratchScope scratch(ctx, st);
     const unsigned NN = (unsigned)((long long)ny * nx);
-    const int arith = resolve_arith(ctx, opts->arith);
-    const int gx = grid_dims(ctx, arith, (opts->ext & 3) || ctx->presc.poly, n_fields, NN);
+    const int gx = grid_dims(ctx, ctx->bps, ort_grid_waves(), opts, n_fields, NN);
     RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * n_fields, d_partials);
     // with opts.gather_stats out->stats receives the records merged over all ranks, out->stats_local this rank's own
     const bool gather = opts->gather_stats != 0;
     ort_stats* d_stats = gather ? d_out->stats_local : d_out->stats;
     if (!d_stats) ENSURE(SL_STATS, sizeof(ort_stats) * (size_t)n_fields, d_stats);
-    if (!opts->compact) {
-        rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, opts, *d_out, nullptr,
-                          d_stats, d_partials, nullptr, gx, st);
-    } else {
-        // compaction: trace into scratch, scatter into the caller's arrays
-        const size_t tot = (size_t)NN * n_fields;
-        ort_grid_out full = *d_out;
-        if (d_out->ex) ENSURE(SL_EX, tot * 8, full.ex);
-        if (d_out->ey) ENSURE(SL_EY, tot * 8, full.ey);
-        if (d_out->r) ENSURE(SL_R, tot * 8, full.r);
-        if (d_out->theta) ENSURE(SL_TH, tot * 8, full.theta);
-        if (d_out->wx) ENSURE(SL_WX, tot * 8, full.wx);
-        if (d_out->wy) ENSURE(SL_WY, tot * 8, full.wy);
-        if (d_out->opd) ENSURE(SL_OPD, tot * 8, full.opd);
-        if (!d_out->mask) ENSURE(SL_MASK, tot, full.mask);
-        const size_t tiles_per_field = (size_t)(NN + ORT_TILE - 1) / ORT_TILE, tile_stride = tiles_per_field + tiles_per_field / 2048 + 2;
-        int* d_tiles; ENSURE(SL_TILES, sizeof(int) * tile_stride * n_fields, d_tiles);
-        rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, opts, full, d_out, d_stats,
-                          d_partials, d_tiles, gx, st);
-    }
+    ort_grid_out full, comp; int* d_tiles;
+    if ((rc = ort_sweep_scratch(ctx, d_out, opts, true, NN, n_fields, 1, &full, &comp, &d_tiles))) return rc;
+    rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, nullptr, 1, opts, full,
+                      opts->compact ? &comp : nullptr, d_stats, d_partials, d_tiles, gx, st);
     if (rc || !gather) return rc;
     ort_stats* d_merged = d_out->stats;
     if (!d_merged) ENSURE(SL_MERGED, sizeof(ort_stats) * (size_t)n_fields, d_merged);
@@ -499,99 +585,58 @@ int ort_trace3d_grid(ort_ctx* ctx, const ort_field* fields, int n_fields, const 
     int rc = grid_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, opts, out);
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream, cs = ctx->copy_stream;
+    ScratchScope scratch(ctx, st);
     const unsigned NN = (unsigned)((long long)ny * nx);
     const size_t tot = (size_t)NN * n_fields;
-    const int arith = resolve_arith(ctx, opts->arith);
     // one launch per field so the D2H of field f overlaps the trace of field f+1
-    const int gx = grid_dims(ctx, arith, (opts->ext & 3) || ctx->presc.poly, 1, NN);
+    const int gx = grid_dims(ctx, ctx->bps, ort_grid_waves(), opts, 1, NN);
     double *d_ys, *d_xs;
     const size_t nys = (size_t)ny * (opts->ys_per_field ? n_fields : 1);
     ENSURE(SL_YS, sizeof(double) * nys, d_ys);
     ENSURE(SL_XS, sizeof(double) * (size_t)nx, d_xs);
     RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * n_fields, d_partials);
     ort_stats* d_stats; ENSURE(SL_STATS, sizeof(ort_stats) * (size_t)n_fields, d_stats);
-    const unsigned ntiles = (NN + ORT_TILE - 1) / ORT_TILE;
-    int* d_tiles = nullptr;
-    ort_grid_out full; memset(&full, 0, sizeof full);
-    ort_grid_out comp; memset(&comp, 0, sizeof comp);
-    if (out->ex) ENSURE(SL_EX, tot * 8, full.ex);
-    if (out->ey) ENSURE(SL_EY, tot * 8, full.ey);
-    if (out->r) ENSURE(SL_R, tot * 8, full.r);
-    if (out->theta) ENSURE(SL_TH, tot * 8, full.theta);
-    if (out->wx) ENSURE(SL_WX, tot * 8, full.wx);
-    if (out->wy) ENSURE(SL_WY, tot * 8, full.wy);
-    if (out->opd) ENSURE(SL_OPD, tot * 8, full.opd);
-    if (out->mask || opts->compact) ENSURE(SL_MASK, tot, full.mask);
-    if (out->flags) ENSURE(SL_FLAGS, tot, full.flags);
-    if (opts->compact) {
-        ENSURE(SL_TILES, sizeof(int) * ((size_t)ntiles + ntiles / 2048 + 2) * n_fields, d_tiles);
-        if (out->ex) ENSURE(SL_CEX, tot * 8, comp.ex);
-        if (out->ey) ENSURE(SL_CEY, tot * 8, comp.ey);
-        if (out->r) ENSURE(SL_CR, tot * 8, comp.r);
-        if (out->theta) ENSURE(SL_CTH, tot * 8, comp.theta);
-        if (out->wx) ENSURE(SL_CWX, tot * 8, comp.wx);
-        if (out->wy) ENSURE(SL_CWY, tot * 8, comp.wy);
-        if (out->opd) ENSURE(SL_COPD, tot * 8, comp.opd);
-    }
-    cudaStream_t st = ctx->stream, cs = ctx->copy_stream;
-    ScratchScope scratch(ctx, st);
+    ort_grid_out full, comp; int* d_tiles;
+    if ((rc = ort_sweep_scratch(ctx, out, opts, false, NN, n_fields, 1, &full, &comp, &d_tiles))) return rc;
     CK(cudaMemcpyAsync(d_ys, ys, sizeof(double) * nys, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_xs, xs, sizeof(double) * (size_t)nx, cudaMemcpyHostToDevice, st));
     ort_stats hstats[ORT_MAX_FIELDS];
+    const ort_grid_out& src = opts->compact ? comp : full;         // of the compacted kind of member
     // Large sweeps: one launch sequence per field, so the D2H of field f overlaps the trace of field f+1.
     // Small sweeps are launch-latency bound: all fields in ONE launch sequence (fields = grid dimension y).
     const bool per_field = n_fields > 1 && tot > ((size_t)1 << 21);
     if (!per_field) {
-        const int gxa = grid_dims(ctx, arith, (opts->ext & 3) || ctx->presc.poly, n_fields, NN);     // <= gx: partials slot is large enough
-        rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, opts, full,
+        const int gxa = grid_dims(ctx, ctx->bps, ort_grid_waves(), opts, n_fields, NN);     // <= gx: partials slot is large enough
+        rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, nullptr, 1, opts, full,
                           opts->compact ? &comp : nullptr, d_stats, d_partials, d_tiles, gxa, st);
         if (rc) return rc;
         CK(cudaMemcpyAsync(hstats, d_stats, sizeof(ort_stats) * (size_t)n_fields, cudaMemcpyDeviceToHost, st));
         if (opts->compact) CK(cudaStreamSynchronize(st));                        // counts needed for the copy sizes
-        const ort_grid_out& src = opts->compact ? comp : full;
-        if (out->mask) CK(cudaMemcpyAsync(out->mask, full.mask, tot, cudaMemcpyDeviceToHost, st));
-        if (out->flags) CK(cudaMemcpyAsync(out->flags, full.flags, tot, cudaMemcpyDeviceToHost, st));
+        if ((rc = ort_copy_out(ctx, out, full, false, 0, 0, tot, 1, NN, st))) return rc;
         for (int f = 0; f < n_fields; f++) {
             const size_t o = (size_t)f * NN;
             const size_t cnt = opts->compact ? (size_t)hstats[f].n_kept : (size_t)NN;
-            if (out->ex) CK(cudaMemcpyAsync(out->ex + o, src.ex + o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->ey) CK(cudaMemcpyAsync(out->ey + o, src.ey + o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->r) CK(cudaMemcpyAsync(out->r + o, src.r + o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->theta) CK(cudaMemcpyAsync(out->theta + o, src.theta + o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->wx) CK(cudaMemcpyAsync(out->wx + o, src.wx + o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->wy) CK(cudaMemcpyAsync(out->wy + o, src.wy + o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->opd && (opts->ext & ORT_EXT_OPD)) CK(cudaMemcpyAsync(out->opd + o, src.opd + o, cnt * 8, cudaMemcpyDeviceToHost, st));
+            if ((rc = ort_copy_out(ctx, out, src, true, o, o, cnt, 1, NN, st))) return rc;
         }
     }
     for (int f = 0; per_field && f < n_fields; f++) {
         const size_t o = (size_t)f * NN;
-        ort_grid_out ff = full, cc = comp;
-#define OFF(p) if (p) p += o
-        OFF(ff.ex); OFF(ff.ey); OFF(ff.r); OFF(ff.theta); OFF(ff.wx); OFF(ff.wy); OFF(ff.opd); OFF(ff.mask); OFF(ff.flags);
-        OFF(cc.ex); OFF(cc.ey); OFF(cc.r); OFF(cc.theta); OFF(cc.wx); OFF(cc.wy); OFF(cc.opd);
-#undef OFF
-        rc = grid_enqueue(ctx, fields + f, 1, d_ys + (opts->ys_per_field ? (size_t)f * ny : 0), ny, d_xs, nx, stop, a_stop, opts, ff,
-                          opts->compact ? &cc : nullptr, d_stats + f, d_partials + (size_t)f * gx,
-                          d_tiles ? d_tiles + (size_t)f * ((size_t)ntiles + ntiles / 2048 + 2) : nullptr, gx, st);
+        const ort_grid_out ff = from_ray(full, o), cc = from_ray(comp, o);
+        rc = grid_enqueue(ctx, fields + f, 1, d_ys + (opts->ys_per_field ? (size_t)f * ny : 0), ny, d_xs, nx, stop, a_stop,
+                          nullptr, 1, opts, ff, opts->compact ? &cc : nullptr, d_stats + f, d_partials + (size_t)f * gx,
+                          d_tiles ? d_tiles + (size_t)f * compact_tile_ints(NN) : nullptr, gx, st);
         if (rc) return rc;
         CK(cudaEventRecord(ctx->ev_field[f], st));
         CK(cudaStreamWaitEvent(cs, ctx->ev_field[f], 0));
         CK(cudaMemcpyAsync(&hstats[f], d_stats + f, sizeof(ort_stats), cudaMemcpyDeviceToHost, cs));
-        if (out->mask) CK(cudaMemcpyAsync(out->mask + o, ff.mask, NN, cudaMemcpyDeviceToHost, cs));
-        if (out->flags) CK(cudaMemcpyAsync(out->flags + o, ff.flags, NN, cudaMemcpyDeviceToHost, cs));
+        if ((rc = ort_copy_out(ctx, out, full, false, o, o, NN, 1, NN, cs))) return rc;
         size_t cnt = NN;
-        const ort_grid_out& src = opts->compact ? cc : ff;
         if (opts->compact) {           // copy only the kept prefix: needs this field's count
             CK(cudaStreamSynchronize(cs));
             cnt = (size_t)hstats[f].n_kept;
         }
-        if (out->ex) CK(cudaMemcpyAsync(out->ex + o, src.ex, cnt * 8, cudaMemcpyDeviceToHost, cs));
-        if (out->ey) CK(cudaMemcpyAsync(out->ey + o, src.ey, cnt * 8, cudaMemcpyDeviceToHost, cs));
-        if (out->r) CK(cudaMemcpyAsync(out->r + o, src.r, cnt * 8, cudaMemcpyDeviceToHost, cs));
-        if (out->theta) CK(cudaMemcpyAsync(out->theta + o, src.theta, cnt * 8, cudaMemcpyDeviceToHost, cs));
-        if (out->wx) CK(cudaMemcpyAsync(out->wx + o, src.wx, cnt * 8, cudaMemcpyDeviceToHost, cs));
-        if (out->wy) CK(cudaMemcpyAsync(out->wy + o, src.wy, cnt * 8, cudaMemcpyDeviceToHost, cs));
-        if (out->opd && (opts->ext & ORT_EXT_OPD)) CK(cudaMemcpyAsync(out->opd + o, src.opd, cnt * 8, cudaMemcpyDeviceToHost, cs));
+        if ((rc = ort_copy_out(ctx, out, src, true, o, o, cnt, 1, NN, cs))) return rc;
     }
     ort_stats hmerged[ORT_MAX_FIELDS];
     if (opts->gather_stats) {               // the statistics of the whole sharded grid: all-gather + rank-order merge
@@ -611,9 +656,6 @@ int ort_trace3d_grid(ort_ctx* ctx, const ort_field* fields, int n_fields, const 
 
 }  // extern "C"
 
-// ------------------------------------------------------------------------------------------
-// through-focus sweep (k_focus): the grid sweep at n_foci image planes, every ray traced once
-// ------------------------------------------------------------------------------------------
 static int focus_check(ort_ctx* ctx, const ort_field* fields, int n_fields, const void* ys, int ny, const void* xs, int nx,
                        int stop, const double* foci, int n_foci, const ort_opts* opts, const ort_grid_out* out)
 {
@@ -637,74 +679,6 @@ static int focus_check(ort_ctx* ctx, const ort_field* fields, int n_fields, cons
     return ORT_OK;
 }
 
-// CTAs along x of a k_focus launch: ort_grid_dims's rule (8 waves, >= 16 tiles per CTA, <= 32 000 rays per thread for the
-// 16-bit flag counters) with k_focus's own rays per thread and resident CTAs/SM
-static int focus_dims(const ort_ctx* ctx, int arith, int n_fields, unsigned NN)
-{
-    const int variant = grid_variant(ctx->presc, arith, 0);
-    const unsigned nsub = (NN + ORT_TILE - 1) / ORT_TILE;
-    const unsigned rpt = (unsigned)grid_rays_per_thread(arith, variant);
-    const unsigned ntiles = (nsub + rpt - 1) / rpt;
-    long long slots = (long long)ctx->sm_count * ctx->bps_focus[arith][variant] / n_fields;
-    if (slots < 1) slots = 1;
-    long long gx = (long long)ntiles / 16;
-    if (gx < slots) gx = slots;
-    if (gx > slots * ORT_GRID_WAVES_DEFAULT) gx = slots * ORT_GRID_WAVES_DEFAULT;
-    const long long gmin = ((long long)nsub + 31999) / 32000;
-    if (gx < gmin) gx = gmin;
-    if (gx > (long long)ntiles) gx = ntiles;
-    if (gx < 1) gx = 1;
-    return (int)gx;
-}
-
-// k_focus + k_grid_finalize over n_fields * n_foci records (+ scan and compaction once when dst is given) on `st`
-static int focus_enqueue(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* d_ys, int ny, const double* d_xs,
-                         int nx, int stop, double a_stop, const double* foci, int n_foci, const ort_opts* opts,
-                         const ort_grid_out& full, const ort_grid_out* dst, ort_stats* d_stats, RawPart* d_partials,
-                         int* d_tiles, int gx, cudaStream_t st)
-{
-    const unsigned NN = (unsigned)((long long)ny * nx);
-    FocusArgs F;
-    memset(&F, 0, sizeof F);
-    GridArgs& A = F.G;
-    A.ys = d_ys; A.xs = d_xs; A.ny = ny; A.nx = nx; A.NN = NN; A.stop = stop;
-    A.ys_stride = opts->ys_per_field ? ny : 0;
-    A.a_stop = a_stop; A.a_stop2 = a_stop * a_stop;
-    A.ex = full.ex; A.ey = full.ey; A.r = full.r; A.theta = full.theta;
-    A.mask = full.mask; A.flags = full.flags;
-    A.partials = d_partials;
-    A.tile_counts = dst ? d_tiles : nullptr;
-    memcpy(A.fields, fields, sizeof(ort_field) * (size_t)n_fields);
-    F.n_foci = n_foci;
-    F.t_lo = F.t_hi = foci[0];
-    for (int j = 0; j < n_foci; j++) {
-        F.foci[j] = foci[j];
-        F.t_lo = fmin(F.t_lo, foci[j]); F.t_hi = fmax(F.t_hi, foci[j]);
-    }
-    const int arith = resolve_arith(ctx, opts->arith);
-    const int nrec = n_fields * n_foci;
-    if (NN > 0) {
-        ProfScope prof(ctx, st);
-        CK(launch_focus(ctx->presc, F, arith, dim3((unsigned)gx, (unsigned)n_fields), st));
-        ctx->launches++;
-    } else {
-        CK(cudaMemsetAsync(d_partials, 0, sizeof(RawPart) * (size_t)gx * nrec, st));
-    }
-    CK(launch_grid_finalize(d_partials, gx, nrec, d_stats, st));
-    ctx->launches++;
-    if (dst && NN > 0) {
-        CompactArgs C;
-        memset(&C, 0, sizeof C);
-        C.NN = NN; C.mask = full.mask; C.tile_offsets = d_tiles;
-        const double* src[4] = {full.ex, full.ey, full.r, full.theta};
-        double* dd[4] = {dst->ex, dst->ey, dst->r, dst->theta};
-        for (int a = 0; a < 4; a++) { C.src[a] = dd[a] ? src[a] : nullptr; C.dst[a] = dd[a]; }
-        CK(launch_compact_focus(d_tiles, C, n_fields, n_foci, st));
-        ctx->launches += 3;
-    }
-    return ORT_OK;
-}
-
 extern "C" {
 
 int ort_trace3d_focus_dev(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* d_ys, int ny,
@@ -715,29 +689,17 @@ int ort_trace3d_focus_dev(ort_ctx* ctx, const ort_field* fields, int n_fields, c
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = (cudaStream_t)stream;
-    ScratchScope scratch(ctx, st);                  // before the first ENSURE: a poisoning memset is ordered like the work
+    ScratchScope scratch(ctx, st);
     const unsigned NN = (unsigned)((long long)ny * nx);
-    const int arith = resolve_arith(ctx, opts->arith);
-    const int gx = focus_dims(ctx, arith, n_fields, NN);
+    const int gx = grid_dims(ctx, ctx->bps_focus, ORT_GRID_WAVES_DEFAULT, opts, n_fields, NN);
     const size_t nrec = (size_t)n_fields * n_foci;
     RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * nrec, d_partials);
     ort_stats* d_stats = d_out->stats;
     if (!d_stats) ENSURE(SL_STATS, sizeof(ort_stats) * nrec, d_stats);
-    if (!opts->compact)
-        return focus_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, n_foci, opts, *d_out, nullptr,
-                             d_stats, d_partials, nullptr, gx, st);
-    // compaction: trace into scratch, scatter into the caller's arrays
-    const size_t tot = (size_t)NN * n_fields;
-    ort_grid_out full = *d_out;
-    if (d_out->ex) ENSURE(SL_EX, tot * n_foci * 8, full.ex);
-    if (d_out->ey) ENSURE(SL_EY, tot * n_foci * 8, full.ey);
-    if (d_out->r) ENSURE(SL_R, tot * 8, full.r);
-    if (d_out->theta) ENSURE(SL_TH, tot * 8, full.theta);
-    if (!d_out->mask) ENSURE(SL_MASK, tot, full.mask);
-    const size_t ntiles = (size_t)(NN + ORT_TILE - 1) / ORT_TILE;
-    int* d_tiles; ENSURE(SL_TILES, sizeof(int) * (ntiles + ntiles / 2048 + 2) * n_fields, d_tiles);
-    return focus_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, n_foci, opts, full, d_out, d_stats,
-                         d_partials, d_tiles, gx, st);
+    ort_grid_out full, comp; int* d_tiles;
+    if ((rc = ort_sweep_scratch(ctx, d_out, opts, true, NN, n_fields, n_foci, &full, &comp, &d_tiles))) return rc;
+    return grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, n_foci, opts, full,
+                        opts->compact ? &comp : nullptr, d_stats, d_partials, d_tiles, gx, st);
 }
 
 int ort_trace3d_focus(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* ys, int ny,
@@ -748,55 +710,32 @@ int ort_trace3d_focus(ort_ctx* ctx, const ort_field* fields, int n_fields, const
     if (rc) return rc;
     CK(cudaSetDevice(ctx->device));
     cudaStream_t st = ctx->stream;
-    ScratchScope scratch(ctx, st);                  // before the first ENSURE (see ort_trace3d_focus_dev)
+    ScratchScope scratch(ctx, st);
     const unsigned NN = (unsigned)((long long)ny * nx);
     const size_t tot = (size_t)NN * n_fields, nrec = (size_t)n_fields * n_foci;
-    const int arith = resolve_arith(ctx, opts->arith);
-    const int gx = focus_dims(ctx, arith, n_fields, NN);
+    const int gx = grid_dims(ctx, ctx->bps_focus, ORT_GRID_WAVES_DEFAULT, opts, n_fields, NN);
     const size_t nys = (size_t)ny * (opts->ys_per_field ? n_fields : 1);
     double *d_ys, *d_xs;
     ENSURE(SL_YS, sizeof(double) * nys, d_ys);
     ENSURE(SL_XS, sizeof(double) * (size_t)nx, d_xs);
     RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * nrec, d_partials);
     ort_stats* d_stats; ENSURE(SL_STATS, sizeof(ort_stats) * nrec, d_stats);
-    ort_grid_out full; memset(&full, 0, sizeof full);
-    ort_grid_out comp; memset(&comp, 0, sizeof comp);
-    if (out->ex) ENSURE(SL_EX, tot * n_foci * 8, full.ex);
-    if (out->ey) ENSURE(SL_EY, tot * n_foci * 8, full.ey);
-    if (out->r) ENSURE(SL_R, tot * 8, full.r);
-    if (out->theta) ENSURE(SL_TH, tot * 8, full.theta);
-    if (out->mask || opts->compact) ENSURE(SL_MASK, tot, full.mask);
-    if (out->flags) ENSURE(SL_FLAGS, tot, full.flags);
-    int* d_tiles = nullptr;
-    if (opts->compact) {
-        const size_t ntiles = (size_t)(NN + ORT_TILE - 1) / ORT_TILE;
-        ENSURE(SL_TILES, sizeof(int) * (ntiles + ntiles / 2048 + 2) * n_fields, d_tiles);
-        if (out->ex) ENSURE(SL_CEX, tot * n_foci * 8, comp.ex);
-        if (out->ey) ENSURE(SL_CEY, tot * n_foci * 8, comp.ey);
-        if (out->r) ENSURE(SL_CR, tot * 8, comp.r);
-        if (out->theta) ENSURE(SL_CTH, tot * 8, comp.theta);
-    }
+    ort_grid_out full, comp; int* d_tiles;
+    if ((rc = ort_sweep_scratch(ctx, out, opts, false, NN, n_fields, n_foci, &full, &comp, &d_tiles))) return rc;
     CK(cudaMemcpyAsync(d_ys, ys, sizeof(double) * nys, cudaMemcpyHostToDevice, st));
     CK(cudaMemcpyAsync(d_xs, xs, sizeof(double) * (size_t)nx, cudaMemcpyHostToDevice, st));
-    rc = focus_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, n_foci, opts, full,
-                       opts->compact ? &comp : nullptr, d_stats, d_partials, d_tiles, gx, st);
+    rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, foci, n_foci, opts, full,
+                      opts->compact ? &comp : nullptr, d_stats, d_partials, d_tiles, gx, st);
     if (rc) return rc;
     std::vector<ort_stats> hstats(nrec);
     CK(cudaMemcpyAsync(hstats.data(), d_stats, sizeof(ort_stats) * nrec, cudaMemcpyDeviceToHost, st));
     if (opts->compact) CK(cudaStreamSynchronize(st));                          // counts needed for the copy sizes
     const ort_grid_out& src = opts->compact ? comp : full;
-    if (out->mask) CK(cudaMemcpyAsync(out->mask, full.mask, tot, cudaMemcpyDeviceToHost, st));
-    if (out->flags) CK(cudaMemcpyAsync(out->flags, full.flags, tot, cudaMemcpyDeviceToHost, st));
+    if ((rc = ort_copy_out(ctx, out, full, false, 0, 0, tot, n_foci, NN, st))) return rc;
     for (int f = 0; f < n_fields; f++) {
         const size_t o = (size_t)f * NN;
         const size_t cnt = opts->compact ? (size_t)hstats[(size_t)f * n_foci].n_kept : (size_t)NN;
-        if (out->r) CK(cudaMemcpyAsync(out->r + o, src.r + o, cnt * 8, cudaMemcpyDeviceToHost, st));
-        if (out->theta) CK(cudaMemcpyAsync(out->theta + o, src.theta + o, cnt * 8, cudaMemcpyDeviceToHost, st));
-        for (int j = 0; j < n_foci; j++) {
-            const size_t oj = ((size_t)f * n_foci + j) * NN;
-            if (out->ex) CK(cudaMemcpyAsync(out->ex + oj, src.ex + oj, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->ey) CK(cudaMemcpyAsync(out->ey + oj, src.ey + oj, cnt * 8, cudaMemcpyDeviceToHost, st));
-        }
+        if ((rc = ort_copy_out(ctx, out, src, true, o, o, cnt, n_foci, NN, st))) return rc;
     }
     CK(cudaStreamSynchronize(st));
     if (out->stats) memcpy(out->stats, hstats.data(), sizeof(ort_stats) * nrec);

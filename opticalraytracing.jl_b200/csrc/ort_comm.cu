@@ -251,11 +251,9 @@ static int grid_multi_impl(ort_ctx** ctxs, int n, const ort_field* fields, int n
     o1.gather_stats = 0;                                    // the gather is driven from here, grouped over the contexts
     int rc = ort_grid_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, opts ? &o1 : nullptr, out);
     if (rc) return rc;
-    const int arith = ort_resolve_arith(ctx, o1.arith);
-    const bool ext = (o1.ext & 3) || ctx->presc.poly;
     const size_t NNt = (size_t)ny * nx;                     // whole grid, per field
     struct Dev {
-        long long lo, hi; unsigned NN; size_t tot;
+        long long lo, hi; unsigned NN;
         ort_grid_out full, comp;
         ort_stats *d_stats, *d_merged, *d_ranks;
     } D[ORT_MAX_GPUS];
@@ -269,7 +267,7 @@ static int grid_multi_impl(ort_ctx** ctxs, int n, const ort_field* fields, int n
         memset(&V, 0, sizeof V);
         comm_range(ny, d, n, &V.lo, &V.hi);
         const int nyd = (int)(V.hi - V.lo);
-        V.NN = (unsigned)((long long)nyd * nx); V.tot = (size_t)V.NN * n_fields;
+        V.NN = (unsigned)((long long)nyd * nx);
         ctx = c;                                            // CK / ENSURE report into the context they act on
         CK(cudaSetDevice(c->device));
         if (d > 0) {                                        // the layout of ctxs[0] on every context
@@ -285,7 +283,7 @@ static int grid_multi_impl(ort_ctx** ctxs, int n, const ort_field* fields, int n
         }
         cudaStream_t st = c->stream;
         ScratchScope scratch(c, st);
-        const int gx = ort_grid_dims(c, arith, ext, n_fields, V.NN);
+        const int gx = ort_grid_dims(c, c->bps, ort_grid_waves(), &o1, n_fields, V.NN);
         double *d_ys, *d_xs;
         const size_t nys = (size_t)nyd * (o1.ys_per_field ? n_fields : 1);
         ENSURE(SL_YS, sizeof(double) * nys, d_ys);
@@ -294,35 +292,16 @@ static int grid_multi_impl(ort_ctx** ctxs, int n, const ort_field* fields, int n
         ENSURE(SL_STATS, sizeof(ort_stats) * (size_t)n_fields, V.d_stats);
         ENSURE(SL_MERGED, sizeof(ort_stats) * (size_t)n_fields, V.d_merged);
         ENSURE(SL_GATHER, sizeof(ort_stats) * (size_t)n_fields * n, V.d_ranks);
-        if (out->ex) ENSURE(SL_EX, V.tot * 8, V.full.ex);
-        if (out->ey) ENSURE(SL_EY, V.tot * 8, V.full.ey);
-        if (out->r) ENSURE(SL_R, V.tot * 8, V.full.r);
-        if (out->theta) ENSURE(SL_TH, V.tot * 8, V.full.theta);
-        if (out->wx) ENSURE(SL_WX, V.tot * 8, V.full.wx);
-        if (out->wy) ENSURE(SL_WY, V.tot * 8, V.full.wy);
-        if (out->opd) ENSURE(SL_OPD, V.tot * 8, V.full.opd);
-        if (out->mask || o1.compact) ENSURE(SL_MASK, V.tot, V.full.mask);
-        if (out->flags) ENSURE(SL_FLAGS, V.tot, V.full.flags);
-        int* d_tiles = nullptr;
-        if (o1.compact) {
-            const unsigned ntiles = (V.NN + ORT_TILE - 1) / ORT_TILE;
-            ENSURE(SL_TILES, sizeof(int) * ((size_t)ntiles + ntiles / 2048 + 2) * n_fields, d_tiles);
-            if (out->ex) ENSURE(SL_CEX, V.tot * 8, V.comp.ex);
-            if (out->ey) ENSURE(SL_CEY, V.tot * 8, V.comp.ey);
-            if (out->r) ENSURE(SL_CR, V.tot * 8, V.comp.r);
-            if (out->theta) ENSURE(SL_CTH, V.tot * 8, V.comp.theta);
-            if (out->wx) ENSURE(SL_CWX, V.tot * 8, V.comp.wx);
-            if (out->wy) ENSURE(SL_CWY, V.tot * 8, V.comp.wy);
-            if (out->opd) ENSURE(SL_COPD, V.tot * 8, V.comp.opd);
-        }
+        int* d_tiles;
+        if ((rc = ort_sweep_scratch(c, out, &o1, false, V.NN, n_fields, 1, &V.full, &V.comp, &d_tiles))) return rc;
         if (o1.ys_per_field)
             for (int f = 0; f < n_fields; f++)
                 CK(cudaMemcpyAsync(d_ys + (size_t)f * nyd, ys + (size_t)f * ny + V.lo, sizeof(double) * (size_t)nyd, cudaMemcpyHostToDevice, st));
         else
             CK(cudaMemcpyAsync(d_ys, ys + V.lo, sizeof(double) * (size_t)nyd, cudaMemcpyHostToDevice, st));
         CK(cudaMemcpyAsync(d_xs, xs, sizeof(double) * (size_t)nx, cudaMemcpyHostToDevice, st));
-        rc = ort_grid_enqueue(c, fields, n_fields, d_ys, nyd, d_xs, nx, stop, a_stop, &o1, V.full, o1.compact ? &V.comp : nullptr,
-                              V.d_stats, d_partials, d_tiles, gx, st);
+        rc = ort_grid_enqueue(c, fields, n_fields, d_ys, nyd, d_xs, nx, stop, a_stop, nullptr, 1, &o1, V.full,
+                              o1.compact ? &V.comp : nullptr, V.d_stats, d_partials, d_tiles, gx, st);
         if (rc) return rc;
     }
     // ---- the one exchange: grouped all-gather of the records, rank-order merge on every device ----------------
@@ -357,22 +336,14 @@ static int grid_multi_impl(ort_ctx** ctxs, int n, const ort_field* fields, int n
         for (int f = 0; f < n_fields; f++) {
             const size_t src_o = (size_t)f * V.NN;
             const size_t grid_o = (size_t)f * NNt + (size_t)V.lo * nx;            // this shard's rows inside the whole grid
-            if (out->mask) CK(cudaMemcpyAsync(out->mask + grid_o, V.full.mask + src_o, V.NN, cudaMemcpyDeviceToHost, st));
-            if (out->flags) CK(cudaMemcpyAsync(out->flags + grid_o, V.full.flags + src_o, V.NN, cudaMemcpyDeviceToHost, st));
+            if ((rc = ort_copy_out(c, out, V.full, false, grid_o, src_o, V.NN, 1, V.NN, st))) return rc;
             size_t dst_o = grid_o, cnt = V.NN;
             if (o1.compact) {                                // behind the kept rays of the preceding shards
                 dst_o = (size_t)f * NNt;
                 for (int e = 0; e < d; e++) dst_o += (size_t)hstats[e][f].n_kept;
                 cnt = (size_t)hstats[d][f].n_kept;
             }
-            const ort_grid_out& S = o1.compact ? V.comp : V.full;
-            if (out->ex) CK(cudaMemcpyAsync(out->ex + dst_o, S.ex + src_o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->ey) CK(cudaMemcpyAsync(out->ey + dst_o, S.ey + src_o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->r) CK(cudaMemcpyAsync(out->r + dst_o, S.r + src_o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->theta) CK(cudaMemcpyAsync(out->theta + dst_o, S.theta + src_o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->wx) CK(cudaMemcpyAsync(out->wx + dst_o, S.wx + src_o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->wy) CK(cudaMemcpyAsync(out->wy + dst_o, S.wy + src_o, cnt * 8, cudaMemcpyDeviceToHost, st));
-            if (out->opd && (o1.ext & ORT_EXT_OPD)) CK(cudaMemcpyAsync(out->opd + dst_o, S.opd + src_o, cnt * 8, cudaMemcpyDeviceToHost, st));
+            if ((rc = ort_copy_out(c, out, o1.compact ? V.comp : V.full, true, dst_o, src_o, cnt, 1, V.NN, st))) return rc;
         }
     }
     for (int d = 0; d < n; d++) { ctx = ctxs[d]; CK(cudaSetDevice(ctx->device)); CK(cudaStreamSynchronize(ctx->stream)); }

@@ -39,7 +39,8 @@ struct ort_ctx {
     cudaEvent_t ev_scratch;
     cudaStream_t scratch_stream;
     bool scratch_busy;
-    cudaStream_t scratch_now;   // stream of the entry point that is running (ScratchScope), for ORT_POISON_SCRATCH
+    cudaStream_t scratch_now;   // stream of the entry point that is running (ScratchScope; NULL is the default stream), for
+                                // ORT_POISON_SCRATCH; ctx->stream until the first one
     long long launches;
     int prof_on;
     long long prof_n;               // event pairs recorded since the last read
@@ -53,7 +54,6 @@ struct ort_ctx {
 int ort_fail(ort_ctx* c, int code, const char* fmt, ...);
 int ort_ensure(ort_ctx* ctx, int id, size_t bytes, void** out);
 int ort_resolve_arith(const ort_ctx* ctx, int arith);
-int ort_grid_dims(const ort_ctx* ctx, int arith, int ext, int n_fields, unsigned NN);
 
 #define fail ort_fail
 #define CK(call)                                                                              \
@@ -99,9 +99,16 @@ struct ProfScope {
 // shared between ort_api.cu and ort_comm.cu
 int ort_grid_check(ort_ctx* ctx, const ort_field* fields, int n_fields, const void* ys, int ny, const void* xs, int nx,
                    int stop, const ort_opts* opts, const ort_grid_out* out);
+int ort_grid_waves();
+int ort_grid_dims(const ort_ctx* ctx, const int (&bps)[2][5], int waves, const ort_opts* opts, int n_fields, unsigned NN);
 int ort_grid_enqueue(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* d_ys, int ny, const double* d_xs,
-                     int nx, int stop, double a_stop, const ort_opts* opts, const ort_grid_out& full, const ort_grid_out* dst,
-                     ort_stats* d_stats, RawPart* d_partials, int* d_tiles, int gx, cudaStream_t st);
+                     int nx, int stop, double a_stop, const double* foci, int n_foci, const ort_opts* opts,
+                     const ort_grid_out& full, const ort_grid_out* dst, ort_stats* d_stats, RawPart* d_partials, int* d_tiles,
+                     int gx, cudaStream_t st);
+int ort_sweep_scratch(ort_ctx* ctx, const ort_grid_out* out, const ort_opts* opts, bool dev, unsigned NN, int n_fields,
+                      int n_foci, ort_grid_out* full, ort_grid_out* comp, int** d_tiles);
+int ort_copy_out(ort_ctx* ctx, const ort_grid_out* out, const ort_grid_out& src, bool rays, size_t dst_o, size_t src_o,
+                 size_t n, int n_foci, unsigned NN, cudaStream_t st);
 // all-gather of the per-field records of this rank + rank-order merge, enqueued on st (ort_comm.cu).  d_local: [n_fields]
 // on the device; d_merged: [n_fields] (may alias nothing else); d_ranks: optional [world][n_fields] receive buffer.
 int ort_comm_gather_stats(ort_ctx* ctx, const ort_stats* d_local, int n_fields, ort_stats* d_merged, ort_stats* d_ranks,

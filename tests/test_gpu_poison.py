@@ -10,7 +10,8 @@ import sys
 import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-FILES = ["tests/test_gpu_trace3d.py", "tests/test_gpu_first_order.py", "tests/test_gpu_random_systems.py"]
+FILES = ["tests/test_gpu_trace3d.py", "tests/test_gpu_first_order.py", "tests/test_gpu_random_systems.py",
+         "tests/test_gpu_sweep_outputs.py"]
 
 
 @pytest.mark.gpu
