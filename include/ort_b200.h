@@ -40,7 +40,8 @@ extern "C" {
 #endif
 
 #define ORT_VERSION 200 /* 0.2.0: communicator inside the library, ort_opts.gather_stats, ort_grid_out.stats_local;
-                           ort_trace3d_focus / ort_trace3d_focus_dev (through-focus sweep) added without a version change */
+                           ort_trace3d_focus / ort_trace3d_focus_dev (through-focus sweep) and ort_spot_energy_dev /
+                           ort_trace3d_energy (encircled energy) added without a version change */
 
 /* status codes */
 #define ORT_OK            0
@@ -233,6 +234,63 @@ int ort_trace3d_focus(ort_ctx *ctx, const ort_field *fields, int n_fields, const
 int ort_trace3d_focus_dev(ort_ctx *ctx, const ort_field *fields /* host */, int n_fields, const double *d_ys, int ny,
                           const double *d_xs, int nx, int stop, double a_stop, const double *foci /* host */, int n_foci,
                           const ort_opts *opts, const ort_grid_out *d_out /* device pointers inside */, void *stream);
+
+/* ---- EXTENSION (no reference method): geometric encircled / ensquared energy of the spot, computed on the device from
+ *      the outputs of a grid or through-focus sweep.  These are the figures a spot_diagram summarises; unlike the RMS they
+ *      are order statistics of every kept ray, so they cannot be built from the mergeable moments of ort_stats.
+ *      A SET is one field of a grid sweep or one (field, focus) of a through-focus sweep: set s = f * n_foci + j, the
+ *      layout of stats[f][j] and ex[f][j][.].  Its kept rays are those with mask == 1, or the first stats[s].n_kept
+ *      entries of a compacted segment; n = stats[s].n_kept.
+ *        centre (cx, cy)   ORT_CENTER_CENTROID: (0, stats[s].mean_y), the centroid of the MIRRORED spot that
+ *                          RealRayError and its RMS describe (mirrored x has mean exactly 0).
+ *                          ORT_CENTER_PARAXIAL: (0, 0), i.e. the point (0, h') -- ey is already yf - h'.
+ *        distance d        dy = __dadd_rn(ey, -cy);
+ *                          ORT_ENERGY_CIRCLE: d = __dsqrt_rn(__dadd_rn(__dmul_rn(ex, ex), __dmul_rn(dy, dy))), never
+ *                          contracted, so numpy.sqrt(ex*ex + dy*dy) gives the same bits;
+ *                          ORT_ENERGY_SQUARE: d = max(|ex|, |dy|), the half-width of the smallest centred square.
+ *                          A ray and its mirror image (-ex, ey) have the same d, so every fraction over the n traced rays
+ *                          is exactly that of the 2n-point mirrored spot.
+ *        counts[s][k]      #{kept i : d_i <= radii[k]} (int64) for radii[0..n_radii), finite, >= 0, strictly ascending,
+ *                          n_radii <= ORT_MAX_RADII.  The encircled-energy curve is counts / n (the caller divides).
+ *        radius[s][i]      for fracs[0..n_fracs), 0 < q <= 1, n_fracs <= ORT_MAX_FRACS: with
+ *                          k = clamp(ceil(__dmul_rn(q, (double)n)), 1, n), the k-th smallest d of the set (1-based), a bit
+ *                          pattern that occurs among its d values; NaN when n = 0.
+ *      A NaN d (a kept ray never has one) sorts after +Inf and lies within no radius.  Every result is exact -- integer
+ *      counts and an element of the input -- so it is bit-identical run to run and equal to a numpy sort / searchsorted
+ *      on the same arrays.  n_radii = 0 or n_fracs = 0 is allowed, not both. */
+#define ORT_MAX_RADII 1024
+#define ORT_MAX_FRACS 8
+#define ORT_ENERGY_CIRCLE   0
+#define ORT_ENERGY_SQUARE   1
+#define ORT_CENTER_CENTROID 0
+#define ORT_CENTER_PARAXIAL 1
+typedef struct ort_energy_req {
+    int32_t metric, center;   /* ORT_ENERGY_*, ORT_CENTER_* */
+    int32_t n_radii, n_fracs;
+    const double *radii, *fracs;  /* host */
+} ort_energy_req;
+typedef struct ort_spot_sets {
+    int32_t n_sets, sets_per_mask;  /* sets_per_mask: 1 for a grid sweep, n_foci for a focus sweep (its mask is per field) */
+    int64_t stride;                 /* ny*nx: set s starts at s*stride, its mask row at (s / sets_per_mask)*stride */
+    const double *ex, *ey;
+    const uint8_t *mask;            /* NULL = compacted segments */
+    const ort_stats *stats;         /* [n_sets]; all device pointers */
+} ort_spot_sets;
+/* Device form (enqueue only on `stream`): the sets already in HBM, e.g. the outputs of ort_trace3d_grid_dev /
+ * ort_trace3d_focus_dev.  d_counts [n_sets][n_radii] (may be NULL when n_radii = 0), d_radius [n_sets][n_fracs] (may be
+ * NULL when n_fracs = 0).  ORT_EINVAL before anything is enqueued for: a NULL array, radii not finite / negative / not
+ * strictly ascending, q outside (0, 1], counts above the maxima, both zero, n_sets outside [1, ORT_MAX_FIELDS *
+ * ORT_MAX_FOCI], sets_per_mask < 1, stride <= 0 or >= 2^31, an unknown metric or centre.  Launches the same number of
+ * kernels whatever n, n_radii, n_fracs and n_sets; integer atomics only. */
+int ort_spot_energy_dev(ort_ctx *ctx, const ort_spot_sets *sets /* host struct */, const ort_energy_req *req,
+                        int64_t *d_counts, double *d_radius, void *stream);
+/* Host form: the grid sweep of the layout (n_foci = 0; polynomial terms and opts.ext accepted as by ort_trace3d_grid) or
+ * the through-focus sweep at foci[0..n_foci) (as ort_trace3d_focus), full grid into the context's scratch, then the
+ * energy on it; only stats [n_sets] (may be NULL), counts [n_sets][n_radii] and radius [n_sets][n_fracs] cross PCIe.
+ * opts.compact must be 0 (ORT_EINVAL); opts.gather_stats is ORT_EUNSUPPORTED. */
+int ort_trace3d_energy(ort_ctx *ctx, const ort_field *fields, int n_fields, const double *ys, int ny, const double *xs,
+                       int nx, int stop, double a_stop, const double *foci, int n_foci /* 0 = grid sweep of the layout */,
+                       const ort_opts *opts, const ort_energy_req *req, ort_stats *stats, int64_t *counts, double *radius);
 
 /* ---- 3-D skew trace of N arbitrary rays, all surfaces recorded: replaces
  *      raytrace(surfaces, y, x, U, V, Vector{RealRay}) src/PupilSampling.jl:34-65 for a batch.

@@ -261,6 +261,72 @@ function through_focus(::B200, surfaces::Layout, system::SystemOrRayBasis, H::Fl
     return (rms = rms, n_kept = n_kept, best_focus = best_focus, best_rms = best_rms)
 end
 
+# --- encircled energy of the spot (EXTENSION, no reference method) --------------------------------
+# full_trace's prelude (:85-114), then ONE ccall (ort_trace3d_energy) that sweeps the pupil grid full-grid on the device --
+# at `focus`, or through focus at `foci` -- and computes the encircled (metric = ORT_ENERGY_CIRCLE) or ensquared
+# (ORT_ENERGY_SQUARE) energy there: fraction[j, k] of the mirrored spot within radii[k] of the centre, and radius[j, i],
+# the k-th smallest distance with k = clamp(ceil(fractions[i] n), 1, n).  Only these numbers cross PCIe.
+# Like the rest of this file it cannot be run in the repository that ships it (no Julia there); the Python host's
+# encircled_energy is the tested form of the same calls.
+struct OrtEnergyReq
+    metric::Int32; center::Int32; n_radii::Int32; n_fracs::Int32
+    radii::Ptr{Float64}; fracs::Ptr{Float64}
+end
+const ORT_ENERGY_CIRCLE, ORT_ENERGY_SQUARE = Int32(0), Int32(1)
+const ORT_CENTER_CENTROID, ORT_CENTER_PARAXIAL = Int32(0), Int32(1)
+
+function encircled_energy(::B200, surfaces::Layout, system::SystemOrRayBasis, H::Float64;
+                          radii::Vector{Float64} = Float64[], fractions::Vector{Float64} = [0.5, 0.8, 0.9],
+                          k_rays::Int = spot_rays, focus = nothing, foci::Union{Nothing, Vector{Float64}} = nothing,
+                          metric = ORT_ENERGY_CIRCLE, center = ORT_CENTER_CENTROID, arith = ORT_ARITH_FAST)
+    require_conic(surfaces)
+    H = abs(H)
+    H ≤ 1.0 || throw(DomainError(H, "Domain: |H| ≤ 1.0"))
+    focus === nothing && (focus = system.marginal.z[end] - system.marginal.z[end-1])   # :87
+    stop = system.stop
+    a_stop = abs(system.a[stop])
+    real_chief = trace_chief_ray(surfaces, system)
+    real_marginal = trace_marginal_ray(surfaces, system)
+    EP_t = real_chief.z[1]
+    Ū = real_chief.u[1]
+    U = H * Ū
+    u = tan(U)
+    y_EP = abs(real_marginal.y[1])
+    y1, y2 = (±(y_EP) - u * EP_t for (±) ∈ (+, -))
+    y1, y2 = trace_edge_rays(surfaces, y1, y2, U, stop, a_stop)
+    if typeof(system) <: System
+        field = OrtField(0, 0, u, tan(0.0), 0.0, 1.0, u * system.f, 0.0, 0.0, 0.0, 0.0)
+    else
+        z0 = system.marginal.z[1]
+        ȳ = system.chief.y[2] + system.chief.u[1] * z0
+        field = OrtField(1, 0, 0.0, 0.0, ȳ, z0, system.chief.y[end], 0.0, 0.0, 0.0, 0.0)
+    end
+    R = [surfaces.R; Inf]; t = [surfaces.t; 0.0]; n = [surfaces.n; 1.0]; K = [surfaces.K; 0.0]
+    t[end-1] = focus                                 # :114 (replaced by each of foci inside the library)
+    set_layout(R, t, n, K)
+    ys = collect(range(y1, y2, k_rays))              # :121
+    xs = collect(range(0.0, y_EP, div(k_rays, 2)))   # :122
+    M = foci === nothing ? 1 : length(foci)
+    stats = [OrtStats(0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0) for _ in 1:M]
+    counts = zeros(Int64, length(radii), M)          # [M][R] in C order
+    radius = zeros(Float64, length(fractions), M)
+    opts = Ref(OrtOpts(arith, 0, 0, 0, 0.0, 1.0, 1.0, 0, 0))
+    GC.@preserve stats counts radius radii fractions begin
+        req = Ref(OrtEnergyReq(metric, center, length(radii), length(fractions),
+                               isempty(radii) ? C_NULL : pointer(radii), isempty(fractions) ? C_NULL : pointer(fractions)))
+        check(ccall((:ort_trace3d_energy, LIB), Cint,
+                    (Ptr{Cvoid}, Ref{OrtField}, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint, Float64, Ptr{Float64},
+                     Cint, Ref{OrtOpts}, Ref{OrtEnergyReq}, Ptr{OrtStats}, Ptr{Int64}, Ptr{Float64}),
+                    ctx(), Ref(field), 1, ys, length(ys), xs, length(xs), stop, a_stop,
+                    foci === nothing ? C_NULL : foci, foci === nothing ? 0 : M, opts, req, pointer(stats),
+                    isempty(radii) ? C_NULL : pointer(counts), isempty(fractions) ? C_NULL : pointer(radius)))
+    end
+    n_kept = stats[1].n_kept
+    fraction = n_kept == 0 ? fill(NaN, M, length(radii)) : permutedims(counts) ./ n_kept
+    return (foci = foci === nothing ? [Float64(focus)] : foci, fraction = fraction, radius = permutedims(radius),
+            n_kept = n_kept)
+end
+
 # --- batched 2-D meridional real rays: src/RayTracing.jl:145-173 ------------------------------
 # Returns (y, U, ts), each rows × N, for N rays in one kernel launch.
 function raytrace(surfaces::Layout{T}, ys::Vector{Float64}, Us::Vector{Float64}, ::Type{RealRay}) where T

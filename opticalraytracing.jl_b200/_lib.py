@@ -19,13 +19,17 @@ EXT_OPD, EXT_VIGNETTE = 1, 2
 STRICT, FAST = 0, 1
 AIM_NOUT = 24
 VIG_TAIL = 12
+MAX_RADII, MAX_FRACS = 1024, 8
+ENERGY_CIRCLE, ENERGY_SQUARE = 0, 1
+CENTER_CENTROID, CENTER_PARAXIAL = 0, 1
 
 # every symbol include/ort_b200.h declares (tests check the .so exports exactly these)
 SYMBOLS = [
     "ort_version", "ort_init", "ort_free", "ort_last_error", "ort_sync", "ort_device_info",
     "ort_host_alloc", "ort_host_free", "ort_device_numa", "ort_bind_host_thread", "ort_launch_count", "ort_profile_enable", "ort_profile_read",
     "ort_set_layout", "ort_set_apertures", "ort_set_polynomials",
-    "ort_trace3d_grid", "ort_trace3d_grid_dev", "ort_trace3d_focus", "ort_trace3d_focus_dev", "ort_trace3d_rays", "ort_trace3d_rays_opl", "ort_trace3d_rays_dev", "ort_trace2d_batch", "ort_aim2d",
+    "ort_trace3d_grid", "ort_trace3d_grid_dev", "ort_trace3d_focus", "ort_trace3d_focus_dev",
+    "ort_spot_energy_dev", "ort_trace3d_energy", "ort_trace3d_rays", "ort_trace3d_rays_opl", "ort_trace3d_rays_dev", "ort_trace2d_batch", "ort_aim2d",
     "ort_paraxial_batch", "ort_paraxial_batch_dev", "ort_transfer_batch", "ort_transfer_batch_dev",
     "ort_trace3d_candidates", "ort_trace3d_candidates_dev", "ort_aim_candidates", "ort_aim_candidates_dev", "ort_aim_fields",
     "ort_trace3d_candidates_aimed", "ort_trace3d_candidates_aimed_dev", "ort_vignetting_candidates",
@@ -81,6 +85,19 @@ class GridOut(C.Structure):
 
 
 GRID_OUT_NAMES = tuple(name for name, _ in GridOut._fields_)
+
+
+class EnergyReq(C.Structure):
+    _fields_ = [("metric", C.c_int32), ("center", C.c_int32), ("n_radii", C.c_int32), ("n_fracs", C.c_int32),
+                ("radii", C.c_void_p), ("fracs", C.c_void_p)]
+
+
+class SpotSets(C.Structure):
+    _fields_ = [("n_sets", C.c_int32), ("sets_per_mask", C.c_int32), ("stride", C.c_int64), ("ex", C.c_void_p),
+                ("ey", C.c_void_p), ("mask", C.c_void_p), ("stats", C.c_void_p)]
+
+
+SPOT_SETS_NAMES = tuple(name for name, _ in SpotSets._fields_)
 RAY_OUT_NAMES = GRID_OUT_NAMES[:9]          # the per-ray members: every one but the statistics records
 
 
@@ -124,6 +141,10 @@ def load():
     L.ort_trace3d_grid_dev.argtypes = grid_args + [C.c_void_p]
     L.ort_trace3d_focus.argtypes = grid_args[:9] + [_dp, C.c_int] + grid_args[9:]
     L.ort_trace3d_focus_dev.argtypes = grid_args[:9] + [_dp, C.c_int] + grid_args[9:] + [C.c_void_p]
+    L.ort_spot_energy_dev.argtypes = [C.c_void_p, C.POINTER(SpotSets), C.POINTER(EnergyReq), C.c_void_p, C.c_void_p,
+                                      C.c_void_p]
+    L.ort_trace3d_energy.argtypes = grid_args[:9] + [_dp, C.c_int, C.POINTER(Opts), C.POINTER(EnergyReq), C.c_void_p,
+                                                     C.c_void_p, C.c_void_p]
     L.ort_trace3d_rays.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p]
     L.ort_trace3d_rays_opl.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p, _dp]
     L.ort_trace3d_rays_dev.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 6
@@ -302,6 +323,21 @@ def _opts(arith, compact, ys_per_field, ext=0, wavegrad=None, opd_scale=1.0, gat
     nu, lam = wavegrad if wavegrad else (0.0, 1.0)
     return Opts(int(arith), int(bool(compact)), int(bool(ys_per_field)), int(ext), float(nu), float(lam), float(opd_scale),
                 int(bool(gather)), 0)
+
+
+_METRICS = {"circle": ENERGY_CIRCLE, "square": ENERGY_SQUARE}
+_CENTERS = {"centroid": CENTER_CENTROID, "paraxial": CENTER_PARAXIAL}
+
+
+def _energy_req(radii, fracs, metric, center):
+    """EnergyReq over float64 copies of radii and fracs (returned too: they must outlive the call).  metric / center are
+    the names ("circle" / "square", "centroid" / "paraxial") or the ORT_* codes; the library validates the values."""
+    r = _d(np.atleast_1d(np.asarray(radii, dtype=np.float64)) if radii is not None else np.empty(0))
+    q = _d(np.atleast_1d(np.asarray(fracs, dtype=np.float64)) if fracs is not None else np.empty(0))
+    m = _METRICS[metric] if isinstance(metric, str) else int(metric)
+    c = _CENTERS[center] if isinstance(center, str) else int(center)
+    req = EnergyReq(m, c, len(r), len(q), r.ctypes.data if len(r) else None, q.ctypes.data if len(q) else None)
+    return req, r, q
 
 
 def make_fields(fields):
@@ -529,6 +565,41 @@ class Context:
         self._ck(self.L.ort_trace3d_focus_dev(self.h, farr, nf, C.c_void_p(d_ys), int(ny), C.c_void_p(d_xs), int(nx),
                                               int(stop), float(a_stop), _p(foci), len(foci), C.byref(op), C.byref(go),
                                               C.c_void_p(stream)))
+
+    # ---- encircled energy ----------------------------------------------------------------
+    def spot_energy_dev(self, sets, radii=None, fracs=None, metric="circle", center="centroid", d_counts=0, d_radius=0,
+                        stream=0):
+        """Encircled / ensquared energy of spot sets already in HBM (ort_spot_energy_dev, enqueue only).  sets: dict with
+        n_sets, sets_per_mask, stride and the device addresses ex, ey, mask (0 = compacted segments), stats.  d_counts:
+        int64 [n_sets][len(radii)], d_radius: float64 [n_sets][len(fracs)] (device addresses)."""
+        ss = SpotSets(*[sets.get(k) or 0 for k in SPOT_SETS_NAMES])
+        req, _r, _q = _energy_req(radii, fracs, metric, center)
+        self._ck(self.L.ort_spot_energy_dev(self.h, C.byref(ss), C.byref(req), C.c_void_p(d_counts or 0),
+                                            C.c_void_p(d_radius or 0), C.c_void_p(stream)))
+
+    def trace3d_energy(self, fields, ys, xs, stop, a_stop, radii=None, fracs=None, foci=None, arith=FAST, metric="circle",
+                       center="centroid", ext=0):
+        """The grid sweep (foci None) or the through-focus sweep at foci, full grid on the device, and the energy of every
+        set on it (ort_trace3d_energy); no spot crosses PCIe.  Returns dict(stats, counts, radius): (n_fields[, M]),
+        (n_fields[, M], len(radii)) int64, (n_fields[, M], len(fracs)) float64."""
+        farr, nf = make_fields(fields)
+        ys, xs = _d(ys), _d(xs)
+        per_field = ys.ndim == 2
+        if per_field and ys.shape[0] != nf:
+            raise ValueError("ys must be (ny,) or (n_fields, ny)")
+        fo = None if foci is None else _d(np.atleast_1d(foci))
+        M = 0 if fo is None else len(fo)
+        req, r, q = _energy_req(radii, fracs, metric, center)
+        lead = (nf,) if fo is None else (nf, M)
+        stats = np.zeros(lead, dtype=STATS_DTYPE)
+        counts = np.zeros(lead + (len(r),), dtype=np.int64)
+        radius = np.zeros(lead + (len(q),), dtype=np.float64)
+        op = _opts(arith, False, per_field, ext)
+        self._ck(self.L.ort_trace3d_energy(self.h, farr, nf, _vp(ys), ys.shape[-1], _vp(xs), len(xs), int(stop),
+                                           float(a_stop), _p(fo), M, C.byref(op), C.byref(req), stats.ctypes.data,
+                                           counts.ctypes.data if len(r) else None,
+                                           radius.ctypes.data if len(q) else None))
+        return dict(stats=stats, counts=counts, radius=radius)
 
     # ---- arbitrary rays ------------------------------------------------------------------
     def trace3d_rays(self, y0, x0, u0, v0, arith=STRICT, opl=False):

@@ -36,6 +36,34 @@ struct FocusArgs {                          // through-focus sweep (k_focus)
     double foci[ORT_MAX_FOCI];
 };
 
+// Encircled energy (kern_energy.cu): per-set selection state in device scratch, written by k_energy_init and
+// k_energy_select, read by the pass kernels
+struct EnergyState {
+    unsigned long long prefix[ORT_MAX_FRACS];   // key bits selected so far, per fraction
+    unsigned long long rank[ORT_MAX_FRACS];     // 0-based rank of the wanted key among the keys with that prefix
+    long long n;                                // kept rays
+    unsigned src_n;                             // keys in candidate list `src`
+    unsigned cnt;                               // keys appended to candidate list `dst` by the running pass
+    int src, dst;                               // candidate list the next pass reads / writes: -1 = the sweep outputs / none
+    int active;                                 // bit f: fraction f is selecting (n > 0)
+    int pad;
+};
+
+struct EnergyArgs {
+    int n_sets, sets_per_mask;
+    long long stride;
+    const double *ex, *ey; const uint8_t* mask; const ort_stats* stats;
+    int metric, center, n_radii, n_fracs;
+    EnergyState* state;                         // [n_sets]
+    unsigned* hist;                             // [n_sets][energy_hist_words(n_fracs)]
+    unsigned long long* bins;                   // [n_sets][n_radii + 1]
+    unsigned long long* cand[2];                // [n_sets][cap] each
+    unsigned cap;                               // candidate-list capacity per set
+    long long* counts;                          // [n_sets][n_radii]
+    double* radius;                             // [n_sets][n_fracs]
+    double fracs[ORT_MAX_FRACS];
+};
+
 struct CompactArgs {
     unsigned NN;
     const uint8_t* mask;
@@ -187,6 +215,11 @@ cudaError_t launch_compact(int* tile_counts, const CompactArgs& C, int n_fields,
 int focus_blocks_per_sm(int arith, int variant);
 cudaError_t launch_focus(const Presc& P, const FocusArgs& F, int arith, dim3 grid, cudaStream_t st);
 cudaError_t launch_compact_focus(int* tile_counts, const CompactArgs& C, int n_fields, int n_foci, cudaStream_t st);
+// encircled energy: hist words per set, candidate-list capacity per set, and the launch sequence (*launches kernels,
+// the same number whatever the sizes)
+size_t energy_hist_words(int n_fracs);
+unsigned energy_cand_cap(long long stride, int n_sets);
+cudaError_t launch_energy(const EnergyArgs& A, const double* radii, int sm_count, cudaStream_t st, int* launches);
 cudaError_t launch_rays(const Presc& P, const RaysArgs& A, int arith, cudaStream_t st);
 cudaError_t launch_candidates(const CandArgs& A, int arith, cudaStream_t st, int sm_count);
 cudaError_t launch_trace2d(const Presc& P, const Trace2dArgs& A, cudaStream_t st);

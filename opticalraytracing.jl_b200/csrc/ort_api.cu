@@ -742,6 +742,142 @@ int ort_trace3d_focus(ort_ctx* ctx, const ort_field* fields, int n_fields, const
     return ORT_OK;
 }
 
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------
+// encircled / ensquared energy of the spot (kern_energy.cu)
+// ------------------------------------------------------------------------------------------
+static int energy_req_check(ort_ctx* ctx, const ort_energy_req* req, const void* counts, const void* radius)
+{
+    if (!req) return fail(ctx, ORT_EINVAL, "spot_energy: req is NULL");
+    if (req->metric != ORT_ENERGY_CIRCLE && req->metric != ORT_ENERGY_SQUARE)
+        return fail(ctx, ORT_EINVAL, "spot_energy: metric = %d", req->metric);
+    if (req->center != ORT_CENTER_CENTROID && req->center != ORT_CENTER_PARAXIAL)
+        return fail(ctx, ORT_EINVAL, "spot_energy: center = %d", req->center);
+    if (req->n_radii < 0 || req->n_radii > ORT_MAX_RADII)
+        return fail(ctx, ORT_EINVAL, "spot_energy: n_radii = %d not in [0, %d]", req->n_radii, ORT_MAX_RADII);
+    if (req->n_fracs < 0 || req->n_fracs > ORT_MAX_FRACS)
+        return fail(ctx, ORT_EINVAL, "spot_energy: n_fracs = %d not in [0, %d]", req->n_fracs, ORT_MAX_FRACS);
+    if (!req->n_radii && !req->n_fracs) return fail(ctx, ORT_EINVAL, "spot_energy: neither radii nor fractions");
+    if (req->n_radii && (!req->radii || !counts)) return fail(ctx, ORT_EINVAL, "spot_energy: radii or counts is NULL");
+    if (req->n_fracs && (!req->fracs || !radius)) return fail(ctx, ORT_EINVAL, "spot_energy: fracs or radius is NULL");
+    for (int k = 0; k < req->n_radii; k++) {
+        const double r = req->radii[k];
+        if (!isfinite(r) || !(r >= 0.0)) return fail(ctx, ORT_EINVAL, "spot_energy: radii[%d] = %g is not finite and >= 0", k, r);
+        if (k && !(r > req->radii[k - 1])) return fail(ctx, ORT_EINVAL, "spot_energy: radii are not strictly ascending at %d", k);
+    }
+    for (int i = 0; i < req->n_fracs; i++) {
+        const double q = req->fracs[i];
+        if (!(q > 0.0 && q <= 1.0)) return fail(ctx, ORT_EINVAL, "spot_energy: fracs[%d] = %g not in (0, 1]", i, q);
+    }
+    return ORT_OK;
+}
+
+static int energy_sets_check(ort_ctx* ctx, const ort_spot_sets* S)
+{
+    if (!S) return fail(ctx, ORT_EINVAL, "spot_energy: sets is NULL");
+    if (S->n_sets < 1 || S->n_sets > ORT_MAX_FIELDS * ORT_MAX_FOCI)
+        return fail(ctx, ORT_EINVAL, "spot_energy: n_sets = %d not in [1, %d]", S->n_sets, ORT_MAX_FIELDS * ORT_MAX_FOCI);
+    if (S->sets_per_mask < 1) return fail(ctx, ORT_EINVAL, "spot_energy: sets_per_mask = %d", S->sets_per_mask);
+    if (S->stride <= 0 || S->stride >= (1LL << 31))
+        return fail(ctx, ORT_EINVAL, "spot_energy: stride = %lld not in [1, 2^31)", (long long)S->stride);
+    if (!S->ex || !S->ey || !S->stats) return fail(ctx, ORT_EINVAL, "spot_energy: ex, ey or stats is NULL");
+    return ORT_OK;
+}
+
+// Enqueue the energy kernels over `sets` on st (inside the entry point's ScratchScope); one ProfScope around all of them
+static int energy_enqueue(ort_ctx* ctx, const ort_spot_sets& S, const ort_energy_req* req, int64_t* d_counts,
+                          double* d_radius, cudaStream_t st)
+{
+    EnergyArgs A;
+    memset(&A, 0, sizeof A);
+    A.n_sets = S.n_sets; A.sets_per_mask = S.sets_per_mask; A.stride = S.stride;
+    A.ex = S.ex; A.ey = S.ey; A.mask = S.mask; A.stats = S.stats;
+    A.metric = req->metric; A.center = req->center; A.n_radii = req->n_radii; A.n_fracs = req->n_fracs;
+    for (int i = 0; i < req->n_fracs; i++) A.fracs[i] = req->fracs[i];
+    A.cap = energy_cand_cap(S.stride, S.n_sets);
+    const size_t ns = (size_t)S.n_sets;
+    ENSURE(SL_EN_STATE, sizeof(EnergyState) * ns, A.state);
+    ENSURE(SL_EN_HIST, sizeof(unsigned) * energy_hist_words(req->n_fracs) * ns, A.hist);
+    ENSURE(SL_EN_BINS, sizeof(unsigned long long) * (size_t)(req->n_radii + 1) * ns, A.bins);
+    ENSURE(SL_EN_CAND0, sizeof(unsigned long long) * A.cap * ns, A.cand[0]);
+    ENSURE(SL_EN_CAND1, sizeof(unsigned long long) * A.cap * ns, A.cand[1]);
+    A.counts = (long long*)d_counts; A.radius = d_radius;
+    int n = 0;
+    {
+        ProfScope prof(ctx, st);
+        CK(launch_energy(A, req->radii, ctx->sm_count, st, &n));
+    }
+    ctx->launches += n;
+    return ORT_OK;
+}
+
+extern "C" {
+
+int ort_spot_energy_dev(ort_ctx* ctx, const ort_spot_sets* sets, const ort_energy_req* req, int64_t* d_counts,
+                        double* d_radius, void* stream)
+{
+    if (!ctx) return ORT_EINVAL;
+    int rc = energy_sets_check(ctx, sets);
+    if (rc || (rc = energy_req_check(ctx, req, d_counts, d_radius))) return rc;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    ScratchScope scratch(ctx, st);
+    return energy_enqueue(ctx, *sets, req, d_counts, d_radius, st);
+}
+
+int ort_trace3d_energy(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* ys, int ny, const double* xs,
+                       int nx, int stop, double a_stop, const double* foci, int n_foci, const ort_opts* opts,
+                       const ort_energy_req* req, ort_stats* stats, int64_t* counts, double* radius)
+{
+    if (!ctx) return ORT_EINVAL;
+    if (!opts) return fail(ctx, ORT_EINVAL, "trace3d_energy: opts is NULL");
+    if (opts->gather_stats) return fail(ctx, ORT_EUNSUPPORTED, "trace3d_energy: opts.gather_stats is not supported");
+    if (opts->compact) return fail(ctx, ORT_EINVAL, "trace3d_energy: opts.compact must be 0");
+    if (n_foci < 0) return fail(ctx, ORT_EINVAL, "trace3d_energy: n_foci = %d", n_foci);
+    // the members the energy reads; ort_sweep_scratch traces each one a host call wants into its scratch slot
+    static double tag; static uint8_t mtag;
+    ort_grid_out want;
+    memset(&want, 0, sizeof want);
+    want.ex = want.ey = &tag; want.mask = &mtag; want.stats = nullptr;
+    int rc = n_foci ? focus_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, foci, n_foci, opts, &want)
+                    : grid_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, opts, &want);
+    if (rc || (rc = energy_req_check(ctx, req, counts, radius))) return rc;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    ScratchScope scratch(ctx, st);
+    const int M = n_foci ? n_foci : 1;
+    const unsigned NN = (unsigned)((long long)ny * nx);
+    const size_t nrec = (size_t)n_fields * M;
+    const int gx = n_foci ? grid_dims(ctx, ctx->bps_focus, ORT_GRID_WAVES_DEFAULT, opts, n_fields, NN)
+                          : grid_dims(ctx, ctx->bps, ort_grid_waves(), opts, n_fields, NN);
+    const size_t nys = (size_t)ny * (opts->ys_per_field ? n_fields : 1);
+    double *d_ys, *d_xs;
+    ENSURE(SL_YS, sizeof(double) * nys, d_ys);
+    ENSURE(SL_XS, sizeof(double) * (size_t)nx, d_xs);
+    RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * nrec, d_partials);
+    ort_stats* d_stats; ENSURE(SL_STATS, sizeof(ort_stats) * nrec, d_stats);
+    int64_t* d_counts; ENSURE(SL_EN_COUNTS, sizeof(int64_t) * nrec * (size_t)req->n_radii, d_counts);
+    double* d_radius; ENSURE(SL_EN_RADIUS, sizeof(double) * nrec * (size_t)req->n_fracs, d_radius);
+    ort_grid_out full, comp; int* d_tiles;
+    if ((rc = ort_sweep_scratch(ctx, &want, opts, false, NN, n_fields, M, &full, &comp, &d_tiles))) return rc;
+    CK(cudaMemcpyAsync(d_ys, ys, sizeof(double) * nys, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_xs, xs, sizeof(double) * (size_t)nx, cudaMemcpyHostToDevice, st));
+    rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, n_foci ? foci : nullptr, M, opts, full,
+                      nullptr, d_stats, d_partials, nullptr, gx, st);
+    if (rc) return rc;
+    ort_spot_sets S;
+    memset(&S, 0, sizeof S);
+    S.n_sets = (int32_t)nrec; S.sets_per_mask = M; S.stride = NN;
+    S.ex = full.ex; S.ey = full.ey; S.mask = full.mask; S.stats = d_stats;
+    if ((rc = energy_enqueue(ctx, S, req, d_counts, d_radius, st))) return rc;
+    if (stats) CK(cudaMemcpyAsync(stats, d_stats, sizeof(ort_stats) * nrec, cudaMemcpyDeviceToHost, st));
+    if (req->n_radii) CK(cudaMemcpyAsync(counts, d_counts, sizeof(int64_t) * nrec * req->n_radii, cudaMemcpyDeviceToHost, st));
+    if (req->n_fracs) CK(cudaMemcpyAsync(radius, d_radius, sizeof(double) * nrec * req->n_fracs, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return ORT_OK;
+}
+
 // ------------------------------------------------------------------------------------------
 // arbitrary rays / 2-D / paraxial / transfer / candidates: host wrappers stage through scratch
 // ------------------------------------------------------------------------------------------

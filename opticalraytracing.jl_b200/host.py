@@ -673,6 +673,20 @@ def _full_trace_setup(surfaces, system, H, k_rays, focus, backend):
                 nu=system.marginal.nu[-1], P=P_ext)
 
 
+def _sweep_inputs(p, k_rays):
+    """the pupil grid (xs, one ys per field) and the field records of a sweep from _full_trace_setup's prelude"""
+    k2 = k_rays // 2                                                             # :116
+    xs = jl_range(0.0, p["y_EP"], k2)                                            # :122
+    ys = np.stack([jl_range(p["y1"][j], p["y2"][j], k_rays) for j in range(len(p["Hs"]))])      # :121
+    if p["z0"] is None:
+        flds = [dict(mode=0, u=float(p["u"][j]), v=math.tan(0.0), h_prime=float(p["h_prime"][j]))
+                for j in range(len(p["Hs"]))]
+    else:
+        flds = [dict(mode=1, ybar=float(p["ybar"]), z0=float(p["z0"]), h_prime=float(p["h_prime"][j]))
+                for j in range(len(p["Hs"]))]
+    return xs, ys, flds
+
+
 def full_trace(*args, backend=None, arith=_lib.FAST):
     """full_trace(system, H[, k_rays, focus]) / full_trace(surfaces, system, H[, k_rays, focus]) /
     full_trace(surfaces, raybasis[, k_rays, focus]) -- src/PupilSampling.jl:85-163.
@@ -702,15 +716,7 @@ def full_trace_fields(surfaces, system, Hs, k_rays=SPOT_RAYS, focus=None, backen
     be.set_layout(p["ext"], p["K"])
     if p["P"] is not None:
         be.set_polynomials(p["P"])
-    k2 = k_rays // 2                                                             # :116
-    xs = jl_range(0.0, p["y_EP"], k2)                                            # :122
-    ys = np.stack([jl_range(p["y1"][j], p["y2"][j], k_rays) for j in range(len(p["Hs"]))])      # :121
-    if p["z0"] is None:
-        flds = [dict(mode=0, u=float(p["u"][j]), v=math.tan(0.0), h_prime=float(p["h_prime"][j]))
-                for j in range(len(p["Hs"]))]
-    else:
-        flds = [dict(mode=1, ybar=float(p["ybar"]), z0=float(p["z0"]), h_prime=float(p["h_prime"][j]))
-                for j in range(len(p["Hs"]))]
+    xs, ys, flds = _sweep_inputs(p, k_rays)
     out = []
     for j0 in range(0, len(flds), _lib.MAX_FIELDS):
         sl = slice(j0, j0 + _lib.MAX_FIELDS)
@@ -768,15 +774,7 @@ def through_focus(surfaces, system, Hs, foci, k_rays=SPOT_RAYS, spots=False, bac
         raise ValueError("through_focus: foci must be finite")
     p = _full_trace_setup(layout, system, Hs, k_rays, None, backend)
     be.set_layout(p["ext"], p["K"])
-    k2 = k_rays // 2                                                             # :116
-    xs = jl_range(0.0, p["y_EP"], k2)                                            # :122
-    ys = np.stack([jl_range(p["y1"][j], p["y2"][j], k_rays) for j in range(len(p["Hs"]))])      # :121
-    if p["z0"] is None:
-        flds = [dict(mode=0, u=float(p["u"][j]), v=math.tan(0.0), h_prime=float(p["h_prime"][j]))
-                for j in range(len(p["Hs"]))]
-    else:
-        flds = [dict(mode=1, ybar=float(p["ybar"]), z0=float(p["z0"]), h_prime=float(p["h_prime"][j]))
-                for j in range(len(p["Hs"]))]
+    xs, ys, flds = _sweep_inputs(p, k_rays)
     want = ("ex", "ey", "stats") if spots else ("stats",)
     out = []
     for j0 in range(0, len(flds), _lib.MAX_FIELDS):
@@ -794,6 +792,71 @@ def through_focus(surfaces, system, Hs, foci, k_rays=SPOT_RAYS, spots=False, bac
                       for m in range(len(foci))]
             out.append(ThroughFocus(float(H), foci.copy(), rms, n, st, bf, br,
                                     bool(foci.min() <= bf <= foci.max()), sp))
+    return out
+
+
+@dataclass
+class EncircledEnergy:
+    """EXTENSION (no reference type): geometric encircled (metric "circle") or ensquared ("square") energy of the spot of
+    one field point, the figures a spot_diagram summarises.  Row j is the image plane foci[j] (one row, full_trace's
+    focus, for a grid sweep).  fraction[j][k] is the share of the mirrored spot within radii[k] of the centre (NaN when no
+    ray is kept); radius[j][i] the smallest radius that holds fractions[i] of it, an exact element of the ray distances
+    (NaN when no ray is kept).  Centre and distance as in include/ort_b200.h (ort_spot_energy_dev)."""
+    H: float
+    foci: np.ndarray
+    radii: np.ndarray
+    fraction: np.ndarray
+    fractions: np.ndarray
+    radius: np.ndarray
+    n_kept: int
+    stats: np.ndarray = field(repr=False)
+
+
+def encircled_energy(surfaces, system, Hs, radii=None, fractions=(0.5, 0.8, 0.9), k_rays=SPOT_RAYS, focus=None, foci=None,
+                     metric="circle", center="centroid", backend=None, arith=_lib.FAST):
+    """EXTENSION: encircled (or ensquared) energy of full_trace's spot for every field point of Hs -> list of
+    EncircledEnergy.  The pupil grid is swept on the device -- at `focus` (full_trace's, default the paraxial one), or
+    with `foci` at up to MAX_FOCI image planes in one pass as through_focus does -- and the curve over `radii` and the
+    energy radii of `fractions` are computed there (ort_trace3d_energy); only those numbers cross PCIe.
+    center "centroid" measures from the centroid of the mirrored spot, (0, mean y); "paraxial" from (0, h')."""
+    be = _be(backend)
+    layout = _as_layout(surfaces)
+    r = np.empty(0) if radii is None else np.atleast_1d(np.asarray(radii, dtype=np.float64))
+    q = np.empty(0) if fractions is None else np.atleast_1d(np.asarray(fractions, dtype=np.float64))
+    if r.ndim != 1 or len(r) > _lib.MAX_RADII or not np.all(np.isfinite(r)) or np.any(r < 0) or np.any(np.diff(r) <= 0):
+        raise ValueError(f"encircled_energy: radii must be finite, >= 0 and strictly ascending, at most {_lib.MAX_RADII}")
+    if q.ndim != 1 or len(q) > _lib.MAX_FRACS or not np.all((q > 0) & (q <= 1)):
+        raise ValueError(f"encircled_energy: fractions must lie in (0, 1], at most {_lib.MAX_FRACS}")
+    if not len(r) and not len(q):
+        raise ValueError("encircled_energy: neither radii nor fractions")
+    if metric not in ("circle", "square") or center not in ("centroid", "paraxial"):
+        raise ValueError("encircled_energy: metric is 'circle' or 'square', center 'centroid' or 'paraxial'")
+    if foci is not None:
+        if focus is not None:
+            raise ValueError("encircled_energy: give focus or foci, not both")
+        if layout.P is not None:
+            raise NotImplementedError("encircled_energy: polynomial terms are not supported through focus")
+        foci = np.atleast_1d(np.asarray(foci, dtype=np.float64))
+        if foci.ndim != 1 or not 1 <= len(foci) <= _lib.MAX_FOCI or not np.all(np.isfinite(foci)):
+            raise ValueError(f"encircled_energy: between 1 and {_lib.MAX_FOCI} finite foci")
+    p = _full_trace_setup(layout, system, Hs, k_rays, focus, backend)
+    be.set_layout(p["ext"], p["K"])
+    if p["P"] is not None:
+        be.set_polynomials(p["P"])
+    xs, ys, flds = _sweep_inputs(p, k_rays)
+    fo = np.array([float(p["focus"])]) if foci is None else foci
+    out = []
+    for j0 in range(0, len(flds), _lib.MAX_FIELDS):
+        sl = slice(j0, j0 + _lib.MAX_FIELDS)
+        e = be.trace3d_energy(flds[sl], ys[sl], xs, p["stop"], p["a_stop"], radii=r, fracs=q, foci=foci, arith=arith,
+                              metric=metric, center=center)
+        for j, H in enumerate(p["Hs"][sl]):
+            st = e["stats"][j].reshape(-1).copy()
+            cnt = e["counts"][j].reshape(len(fo), len(r))
+            n = int(st[0]["n_kept"])
+            frac = cnt / n if n else np.full(cnt.shape, np.nan)
+            out.append(EncircledEnergy(float(H), fo.copy(), r.copy(), frac, q.copy(),
+                                       e["radius"][j].reshape(len(fo), len(q)).copy(), n, st))
     return out
 
 
