@@ -41,7 +41,8 @@ extern "C" {
 
 #define ORT_VERSION 200 /* 0.2.0: communicator inside the library, ort_opts.gather_stats, ort_grid_out.stats_local;
                            ort_trace3d_focus / ort_trace3d_focus_dev (through-focus sweep) and ort_spot_energy_dev /
-                           ort_trace3d_energy (encircled energy) added without a version change */
+                           ort_trace3d_energy (encircled energy) and ort_wavefront_zernike_dev / ort_trace3d_zernike
+                           (Zernike fit of the wavefront) added without a version change */
 
 /* status codes */
 #define ORT_OK            0
@@ -291,6 +292,57 @@ int ort_spot_energy_dev(ort_ctx *ctx, const ort_spot_sets *sets /* host struct *
 int ort_trace3d_energy(ort_ctx *ctx, const ort_field *fields, int n_fields, const double *ys, int ny, const double *xs,
                        int nx, int stop, double a_stop, const double *foci, int n_foci /* 0 = grid sweep of the layout */,
                        const ort_opts *opts, const ort_energy_req *req, ort_stats *stats, int64_t *counts, double *radius);
+
+/* ---- EXTENSION (no reference method): Zernike decomposition of the ray-traced wavefront, fitted on the device from the
+ *      outputs of a grid sweep with ORT_EXT_OPD (the OPD map that Wavefront.opd of the Python host holds).
+ *      Basis: ANSI Z80.28 / OSA, single index j = (n(n+2) + m)/2 for n = 0 .. n_max, m = -n, -n+2, .., n;
+ *        Z_j(rho, theta) = N_n^m R_n^|m|(rho) x {cos m theta (m > 0); sin |m| theta (m < 0); 1 (m = 0)},
+ *        N_n^m = sqrt(2(n+1) / (1 + delta_m0)): every term has unit RMS over the unit disk.  This ordering is the library's;
+ *        J = (n_max+1)(n_max+2)/2 terms.
+ *      Pupil coordinates: the sweep's own r and theta (hypot and atan2(y, x) at the stop surface, theta from the sagittal
+ *        +x axis); rho = r / r_norm with r_norm = req.r_norm if > 0, else stats[s].r_max (the reference's rho = r / max(r),
+ *        src/PupilSampling.jl:142).
+ *      A SET is one field of a grid sweep; its kept rays are those with mask == 1, or the first stats[s].n_kept entries of
+ *        a compacted segment.  The fit is the least-squares fit of opd over the MIRRORED wavefront, 2n points (r, theta)
+ *        and (r, pi - theta) with the same opd.  Under that mirror cos m theta (m even) and sin m theta (m odd) are
+ *        symmetric and every other term antisymmetric; over mirrored pairs the cross terms of the two classes cancel
+ *        exactly, so the device fits only the J_s symmetric terms from the n traced rays (25 at n_max = 8, 49 at 12) and
+ *        returns the antisymmetric coefficients as exactly 0.0.  In exact arithmetic this is the full-basis fit of the
+ *        2n-point set.  The fit solves the normal equations G c = b, G = sum z z^T, b = sum z opd, by Cholesky.
+ *      Outputs per set s:
+ *        coef[s][J]     ANSI order, in the units of opd;
+ *        resid[s][2]    RMS and PV (max - min) of opd - sum_j c_j Z_j over the kept rays, from a second pass over them;
+ *        status[s]      0 ok; 1 n_kept < J_s (including 0); 2 G not numerically positive definite: a Cholesky pivot
+ *                       <= 1e-10 x its diagonal entry of G; 3 a kept ray has a non-finite opd.  For status != 0 coef and
+ *                       resid are NaN.
+ *      Determinism: no floating-point atomics, per-CTA partial sums folded in a fixed order, so the results are
+ *      bit-identical run to run on one device.  They are not bit-equal to a numpy fit, and the full-grid (masked) and
+ *      compacted forms of the same sweep may differ in the last bits (their rays fall into different partial sums). */
+#define ORT_ZERN_MAX_ORDER 12
+typedef struct ort_zernike_req {
+    int32_t n_max, reserved;        /* 0 .. ORT_ZERN_MAX_ORDER */
+    double  r_norm;                 /* > 0: pupil radius of rho = 1; 0: stats[s].r_max of each set */
+} ort_zernike_req;
+typedef struct ort_wave_sets {
+    int32_t n_sets, reserved;
+    int64_t stride;                 /* ny*nx: set s starts at s*stride */
+    const double *opd, *r, *theta;
+    const uint8_t *mask;            /* NULL = compacted segments */
+    const ort_stats *stats;         /* [n_sets]; all device pointers */
+} ort_wave_sets;
+/* Device form (enqueue only on `stream`): the sets already in HBM, e.g. the outputs of ort_trace3d_grid_dev with
+ * ORT_EXT_OPD.  d_coef [n_sets][J], d_resid [n_sets][2], d_status [n_sets].  ORT_EINVAL before anything is enqueued
+ * for: a NULL array, n_max outside [0, ORT_ZERN_MAX_ORDER], r_norm negative or not finite, n_sets outside
+ * [1, ORT_MAX_FIELDS], stride <= 0 or >= 2^31.  Launches four kernels whatever n, n_max and n_sets. */
+int ort_wavefront_zernike_dev(ort_ctx *ctx, const ort_wave_sets *sets /* host struct */, const ort_zernike_req *req,
+                              double *d_coef, double *d_resid, int32_t *d_status, void *stream);
+/* Host form: the grid sweep of the layout (polynomial terms and vignetting accepted as by ort_trace3d_grid) full grid
+ * into the context's scratch with opd, r, theta, mask and stats, then the fit on it; only stats [n_fields] (may be NULL),
+ * coef [n_fields][J], resid [n_fields][2] and status [n_fields] cross PCIe.  opts.ext must hold ORT_EXT_OPD and
+ * opts.compact must be 0 (ORT_EINVAL); opts.gather_stats is ORT_EUNSUPPORTED. */
+int ort_trace3d_zernike(ort_ctx *ctx, const ort_field *fields, int n_fields, const double *ys, int ny, const double *xs,
+                        int nx, int stop, double a_stop, const ort_opts *opts, const ort_zernike_req *req,
+                        ort_stats *stats, double *coef, double *resid, int32_t *status);
 
 /* ---- 3-D skew trace of N arbitrary rays, all surfaces recorded: replaces
  *      raytrace(surfaces, y, x, U, V, Vector{RealRay}) src/PupilSampling.jl:34-65 for a batch.

@@ -327,6 +327,76 @@ function encircled_energy(::B200, surfaces::Layout, system::SystemOrRayBasis, H:
             n_kept = n_kept)
 end
 
+# --- Zernike decomposition of the wavefront (EXTENSION, no reference method) ------------------------------
+# The OPD sweep of the Python host's wavefront() -- full_trace's prelude, the chief ray through the centre of the stop,
+# the reference sphere centred on its image point with radius image plane - paraxial exit pupil -- then ONE ccall
+# (ort_trace3d_zernike) that sweeps the pupil grid with ORT_EXT_OPD on the device and fits ANSI Zernike terms n <= n_max
+# to the mirrored OPD map there (coefficients in waves, ANSI order j = (n(n+2) + m)/2).  Only coef, the residual RMS /
+# PV and the status cross PCIe.  norm = :stop puts the stop rim at rho = 1, :rmax the largest kept r (RealRayError.r).
+# Like the rest of this file it cannot be run in the repository that ships it (no Julia there); the Python host's
+# zernike is the tested form of the same calls.
+struct OrtZernikeReq
+    n_max::Int32; reserved::Int32; r_norm::Float64
+end
+const ORT_EXT_OPD, ORT_EXT_VIGNETTE = Int32(1), Int32(2)
+
+function zernike(::B200, surfaces::Layout, system::System, H::Float64; n_max::Int = 8, k_rays::Int = spot_rays,
+                 focus = nothing, λ = 587.5618e-6, vignette::Bool = false, norm::Symbol = :stop, arith = ORT_ARITH_FAST)
+    require_conic(surfaces)
+    0 ≤ n_max ≤ 12 || throw(DomainError(n_max, "0 ≤ n_max ≤ 12"))
+    norm ∈ (:stop, :rmax) || throw(ArgumentError("norm is :stop or :rmax"))
+    H = abs(H)
+    H ≤ 1.0 || throw(DomainError(H, "Domain: |H| ≤ 1.0"))
+    focus === nothing && (focus = system.marginal.z[end] - system.marginal.z[end-1])   # :87
+    stop = system.stop
+    a_stop = abs(system.a[stop])
+    real_chief = trace_chief_ray(surfaces, system)
+    real_marginal = trace_marginal_ray(surfaces, system)
+    EP_t = real_chief.z[1]
+    U = H * real_chief.u[1]
+    u = tan(U)
+    y_EP = abs(real_marginal.y[1])
+    y1, y2 = trace_edge_rays(surfaces, y_EP - u * EP_t, -y_EP - u * EP_t, U, stop, a_stop)
+    # chief ray: the entrance height that meets the stop at y = 0 (2-D secant solve on the bare layout)
+    set_layout([surfaces.R; Inf], [surfaces.t; 0.0], [surfaces.n; 1.0], [surfaces.K; 0.0])
+    y_c = Ref(-u * EP_t)
+    check(ccall((:ort_aim2d, LIB), Cint, (Ptr{Cvoid}, Int64, Ref{Float64}, Ref{Float64}, Ref{Float64}, Cint, Cint, Cint,
+                                          Float64, Cint, Ref{Float64}, Ptr{Int32}),
+                ctx(), 1, Ref(-u * EP_t), Ref(U), Ref(0.0), stop, 0, 1, a_stop, 0, y_c, C_NULL))
+    # the extended layout: image plane at `focus`, in the last medium (no refraction onto it)
+    R = [surfaces.R; Inf]; t = [surfaces.t; 0.0]; n = [surfaces.n; surfaces.n[end]]; K = [surfaces.K; 0.0]
+    t[end-1] = focus                                 # :114
+    set_layout(R, t, n, K)
+    a = vignette ? Float64.(system.a) : Float64[]
+    check(ccall((:ort_set_apertures, LIB), Cint, (Ptr{Cvoid}, Cint, Ptr{Float64}), ctx(), length(a),
+                isempty(a) ? C_NULL : a))
+    rows1 = length(R) - 1
+    xv = zeros(rows1); yv = zeros(rows1); opl = zeros(1)
+    check(ccall((:ort_trace3d_rays_opl, LIB), Cint,
+                (Ptr{Cvoid}, Int64, Ref{Float64}, Ref{Float64}, Ref{Float64}, Ref{Float64}, Cint, Ptr{Float64},
+                 Ptr{Float64}, Ptr{Float64}, Ptr{UInt8}, Ptr{Float64}),
+                ctx(), 1, y_c, Ref(0.0), Ref(u), Ref(0.0), ORT_ARITH_STRICT, xv, yv, C_NULL, C_NULL, opl))
+    Rr = focus - system.XP.t                         # image plane - paraxial exit pupil
+    opl_ref = opl[1] + surfaces.n[1] * (y_c[] * u / sqrt(u^2 + 1)) - surfaces.n[end] * Rr
+    field = OrtField(0, 0, u, 0.0, 0.0, 0.0, u * system.f, 0.0, yv[end], Rr, opl_ref)
+    ys = collect(range(y1, y2, k_rays))              # :121
+    xs = collect(range(0.0, y_EP, div(k_rays, 2)))   # :122
+    J = (n_max + 1) * (n_max + 2) ÷ 2
+    stats = [OrtStats(0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0)]
+    coef = zeros(J); resid = zeros(2); status = zeros(Int32, 1)
+    opts = Ref(OrtOpts(arith, 0, 0, ORT_EXT_OPD | (vignette ? ORT_EXT_VIGNETTE : Int32(0)), 0.0, 1.0, -1.0 / λ, 0, 0))
+    req = Ref(OrtZernikeReq(n_max, 0, norm == :stop ? a_stop : 0.0))
+    check(ccall((:ort_trace3d_zernike, LIB), Cint,
+                (Ptr{Cvoid}, Ref{OrtField}, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint, Float64, Ref{OrtOpts},
+                 Ref{OrtZernikeReq}, Ptr{OrtStats}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}),
+                ctx(), Ref(field), 1, ys, length(ys), xs, length(xs), stop, a_stop, opts, req, stats, coef, resid,
+                status))
+    check(ccall((:ort_set_apertures, LIB), Cint, (Ptr{Cvoid}, Cint, Ptr{Float64}), ctx(), 0, C_NULL))
+    nm = [(nn, m) for nn in 0:n_max for m in -nn:2:nn]
+    return (n = first.(nm), m = last.(nm), coef = coef, rms_resid = resid[1], pv_resid = resid[2],
+            status = Int(status[1]), n_kept = stats[1].n_kept)
+end
+
 # --- batched 2-D meridional real rays: src/RayTracing.jl:145-173 ------------------------------
 # Returns (y, U, ts), each rows × N, for N rays in one kernel launch.
 function raytrace(surfaces::Layout{T}, ys::Vector{Float64}, Us::Vector{Float64}, ::Type{RealRay}) where T

@@ -22,6 +22,7 @@ VIG_TAIL = 12
 MAX_RADII, MAX_FRACS = 1024, 8
 ENERGY_CIRCLE, ENERGY_SQUARE = 0, 1
 CENTER_CENTROID, CENTER_PARAXIAL = 0, 1
+ZERN_MAX_ORDER = 12
 
 # every symbol include/ort_b200.h declares (tests check the .so exports exactly these)
 SYMBOLS = [
@@ -29,7 +30,8 @@ SYMBOLS = [
     "ort_host_alloc", "ort_host_free", "ort_device_numa", "ort_bind_host_thread", "ort_launch_count", "ort_profile_enable", "ort_profile_read",
     "ort_set_layout", "ort_set_apertures", "ort_set_polynomials",
     "ort_trace3d_grid", "ort_trace3d_grid_dev", "ort_trace3d_focus", "ort_trace3d_focus_dev",
-    "ort_spot_energy_dev", "ort_trace3d_energy", "ort_trace3d_rays", "ort_trace3d_rays_opl", "ort_trace3d_rays_dev", "ort_trace2d_batch", "ort_aim2d",
+    "ort_spot_energy_dev", "ort_trace3d_energy", "ort_wavefront_zernike_dev", "ort_trace3d_zernike",
+    "ort_trace3d_rays", "ort_trace3d_rays_opl", "ort_trace3d_rays_dev", "ort_trace2d_batch", "ort_aim2d",
     "ort_paraxial_batch", "ort_paraxial_batch_dev", "ort_transfer_batch", "ort_transfer_batch_dev",
     "ort_trace3d_candidates", "ort_trace3d_candidates_dev", "ort_aim_candidates", "ort_aim_candidates_dev", "ort_aim_fields",
     "ort_trace3d_candidates_aimed", "ort_trace3d_candidates_aimed_dev", "ort_vignetting_candidates",
@@ -98,6 +100,23 @@ class SpotSets(C.Structure):
 
 
 SPOT_SETS_NAMES = tuple(name for name, _ in SpotSets._fields_)
+
+
+class ZernikeReq(C.Structure):
+    _fields_ = [("n_max", C.c_int32), ("reserved", C.c_int32), ("r_norm", C.c_double)]
+
+
+class WaveSets(C.Structure):
+    _fields_ = [("n_sets", C.c_int32), ("reserved", C.c_int32), ("stride", C.c_int64), ("opd", C.c_void_p),
+                ("r", C.c_void_p), ("theta", C.c_void_p), ("mask", C.c_void_p), ("stats", C.c_void_p)]
+
+
+WAVE_SETS_NAMES = tuple(name for name, _ in WaveSets._fields_)
+
+
+def zernike_terms(n_max):
+    """J = (n_max + 1)(n_max + 2) / 2 coefficients per set, in ANSI order"""
+    return (int(n_max) + 1) * (int(n_max) + 2) // 2
 RAY_OUT_NAMES = GRID_OUT_NAMES[:9]          # the per-ray members: every one but the statistics records
 
 
@@ -145,6 +164,10 @@ def load():
                                       C.c_void_p]
     L.ort_trace3d_energy.argtypes = grid_args[:9] + [_dp, C.c_int, C.POINTER(Opts), C.POINTER(EnergyReq), C.c_void_p,
                                                      C.c_void_p, C.c_void_p]
+    L.ort_wavefront_zernike_dev.argtypes = [C.c_void_p, C.POINTER(WaveSets), C.POINTER(ZernikeReq), C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_void_p]
+    L.ort_trace3d_zernike.argtypes = grid_args[:9] + [C.POINTER(Opts), C.POINTER(ZernikeReq), C.c_void_p, C.c_void_p,
+                                                      C.c_void_p, C.c_void_p]
     L.ort_trace3d_rays.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p]
     L.ort_trace3d_rays_opl.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p, _dp]
     L.ort_trace3d_rays_dev.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 6
@@ -600,6 +623,37 @@ class Context:
                                            counts.ctypes.data if len(r) else None,
                                            radius.ctypes.data if len(q) else None))
         return dict(stats=stats, counts=counts, radius=radius)
+
+    # ---- Zernike fit of the wavefront -----------------------------------------------------
+    def wavefront_zernike_dev(self, sets, n_max, r_norm=0.0, d_coef=0, d_resid=0, d_status=0, stream=0):
+        """Zernike fit of wavefront sets already in HBM (ort_wavefront_zernike_dev, enqueue only).  sets: dict with n_sets,
+        stride and the device addresses opd, r, theta, mask (0 = compacted segments), stats.  d_coef: float64
+        [n_sets][zernike_terms(n_max)], d_resid: float64 [n_sets][2], d_status: int32 [n_sets] (device addresses)."""
+        ws = WaveSets(*[sets.get(k) or 0 for k in WAVE_SETS_NAMES])
+        req = ZernikeReq(int(n_max), 0, float(r_norm))
+        self._ck(self.L.ort_wavefront_zernike_dev(self.h, C.byref(ws), C.byref(req), C.c_void_p(d_coef or 0),
+                                                  C.c_void_p(d_resid or 0), C.c_void_p(d_status or 0),
+                                                  C.c_void_p(stream)))
+
+    def trace3d_zernike(self, fields, ys, xs, stop, a_stop, n_max, r_norm=0.0, arith=FAST, ext=EXT_OPD, opd_scale=1.0):
+        """The grid sweep with ORT_EXT_OPD full grid on the device and the Zernike fit of every field on it
+        (ort_trace3d_zernike); no ray crosses PCIe.  Returns dict(stats (n_fields,), coef (n_fields, J) float64,
+        resid (n_fields, 2) float64 = RMS, PV, status (n_fields,) int32)."""
+        farr, nf = make_fields(fields)
+        ys, xs = _d(ys), _d(xs)
+        per_field = ys.ndim == 2
+        if per_field and ys.shape[0] != nf:
+            raise ValueError("ys must be (ny,) or (n_fields, ny)")
+        stats = np.zeros(nf, dtype=STATS_DTYPE)
+        coef = np.zeros((nf, zernike_terms(max(int(n_max), 0))), dtype=np.float64)
+        resid = np.zeros((nf, 2), dtype=np.float64)
+        status = np.zeros(nf, dtype=np.int32)
+        req = ZernikeReq(int(n_max), 0, float(r_norm))
+        op = _opts(arith, False, per_field, ext, opd_scale=opd_scale)
+        self._ck(self.L.ort_trace3d_zernike(self.h, farr, nf, _vp(ys), ys.shape[-1], _vp(xs), len(xs), int(stop),
+                                            float(a_stop), C.byref(op), C.byref(req), stats.ctypes.data,
+                                            coef.ctypes.data, resid.ctypes.data, status.ctypes.data))
+        return dict(stats=stats, coef=coef, resid=resid, status=status)
 
     # ---- arbitrary rays ------------------------------------------------------------------
     def trace3d_rays(self, y0, x0, u0, v0, arith=STRICT, opl=False):

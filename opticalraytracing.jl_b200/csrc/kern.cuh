@@ -64,6 +64,22 @@ struct EnergyArgs {
     double fracs[ORT_MAX_FRACS];
 };
 
+// Zernike fit of the wavefront (kern_zernike.cu)
+struct ZernArgs {
+    int n_sets, n_max;
+    long long stride;
+    const double *opd, *r, *theta; const uint8_t* mask; const ort_stats* stats;
+    double r_norm;                              // 0: stats[s].r_max
+    int js, jp, nblk, R;                        // fitted terms, Gram row (js + 1 padded to 4), 4 x 4 Gram blocks, ray groups
+    int gx, gx_resid;                           // CTAs per set of k_zern_gram and of k_zern_resid
+    double* gpart;                              // [n_sets][gx][zern_gram_record]: per-CTA Gram blocks, non-finite flag
+    double* rpart;                              // [n_sets][gx_resid][3]: per-CTA sum of squares, min, max of the residual
+    double* csym;                               // [n_sets][49]: the fitted coefficients in column order
+    double* coef;                               // [n_sets][(n_max + 1)(n_max + 2) / 2]
+    double* resid;                              // [n_sets][2]
+    int* status;                                // [n_sets]
+};
+
 struct CompactArgs {
     unsigned NN;
     const uint8_t* mask;
@@ -220,6 +236,12 @@ cudaError_t launch_compact_focus(int* tile_counts, const CompactArgs& C, int n_f
 size_t energy_hist_words(int n_fracs);
 unsigned energy_cand_cap(long long stride, int n_sets);
 cudaError_t launch_energy(const EnergyArgs& A, const double* radii, int sm_count, cudaStream_t st, int* launches);
+// Zernike fit: zern_dims fills js .. gx_resid from n_sets, n_max and stride; zern_gram_record is the doubles per gpart
+// record; launch_zernike enqueues the four kernels
+int zern_fitted_terms(int n_max);
+cudaError_t zern_dims(ZernArgs& A, int sm_count);
+size_t zern_gram_record(const ZernArgs& A);
+cudaError_t launch_zernike(const ZernArgs& A, cudaStream_t st, int* launches);
 cudaError_t launch_rays(const Presc& P, const RaysArgs& A, int arith, cudaStream_t st);
 cudaError_t launch_candidates(const CandArgs& A, int arith, cudaStream_t st, int sm_count);
 cudaError_t launch_trace2d(const Presc& P, const Trace2dArgs& A, cudaStream_t st);

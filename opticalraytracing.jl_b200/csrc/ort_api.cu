@@ -878,6 +878,120 @@ int ort_trace3d_energy(ort_ctx* ctx, const ort_field* fields, int n_fields, cons
     return ORT_OK;
 }
 
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------
+// Zernike fit of the wavefront (kern_zernike.cu)
+// ------------------------------------------------------------------------------------------
+static int zernike_req_check(ort_ctx* ctx, const ort_zernike_req* req, const void* coef, const void* resid,
+                             const void* status)
+{
+    if (!req) return fail(ctx, ORT_EINVAL, "zernike: req is NULL");
+    if (req->n_max < 0 || req->n_max > ORT_ZERN_MAX_ORDER)
+        return fail(ctx, ORT_EINVAL, "zernike: n_max = %d not in [0, %d]", req->n_max, ORT_ZERN_MAX_ORDER);
+    if (!isfinite(req->r_norm) || req->r_norm < 0.0)
+        return fail(ctx, ORT_EINVAL, "zernike: r_norm = %g is not finite and >= 0", req->r_norm);
+    if (!coef || !resid || !status) return fail(ctx, ORT_EINVAL, "zernike: coef, resid or status is NULL");
+    return ORT_OK;
+}
+
+// Enqueue the four fit kernels over `sets` on st (inside the entry point's ScratchScope); one ProfScope around them
+static int zernike_enqueue(ort_ctx* ctx, const ort_wave_sets& S, const ort_zernike_req* req, double* d_coef,
+                           double* d_resid, int32_t* d_status, cudaStream_t st)
+{
+    ZernArgs A;
+    memset(&A, 0, sizeof A);
+    A.n_sets = S.n_sets; A.n_max = req->n_max; A.stride = S.stride;
+    A.opd = S.opd; A.r = S.r; A.theta = S.theta; A.mask = S.mask; A.stats = S.stats;
+    A.r_norm = req->r_norm;
+    CK(zern_dims(A, ctx->sm_count));
+    const size_t ns = (size_t)S.n_sets;
+    ENSURE(SL_ZN_GPART, sizeof(double) * zern_gram_record(A) * (size_t)A.gx * ns, A.gpart);
+    ENSURE(SL_ZN_RPART, sizeof(double) * 3 * (size_t)A.gx_resid * ns, A.rpart);
+    ENSURE(SL_ZN_CSYM, sizeof(double) * zern_fitted_terms(ORT_ZERN_MAX_ORDER) * ns, A.csym);
+    A.coef = d_coef; A.resid = d_resid; A.status = (int*)d_status;
+    int n = 0;
+    {
+        ProfScope prof(ctx, st);
+        CK(launch_zernike(A, st, &n));
+    }
+    ctx->launches += n;
+    return ORT_OK;
+}
+
+extern "C" {
+
+int ort_wavefront_zernike_dev(ort_ctx* ctx, const ort_wave_sets* sets, const ort_zernike_req* req, double* d_coef,
+                              double* d_resid, int32_t* d_status, void* stream)
+{
+    if (!ctx) return ORT_EINVAL;
+    if (!sets) return fail(ctx, ORT_EINVAL, "wavefront_zernike: sets is NULL");
+    if (sets->n_sets < 1 || sets->n_sets > ORT_MAX_FIELDS)
+        return fail(ctx, ORT_EINVAL, "wavefront_zernike: n_sets = %d not in [1, %d]", sets->n_sets, ORT_MAX_FIELDS);
+    if (sets->stride <= 0 || sets->stride >= (1LL << 31))
+        return fail(ctx, ORT_EINVAL, "wavefront_zernike: stride = %lld not in [1, 2^31)", (long long)sets->stride);
+    if (!sets->opd || !sets->r || !sets->theta || !sets->stats)
+        return fail(ctx, ORT_EINVAL, "wavefront_zernike: opd, r, theta or stats is NULL");
+    int rc = zernike_req_check(ctx, req, d_coef, d_resid, d_status);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    ScratchScope scratch(ctx, st);
+    return zernike_enqueue(ctx, *sets, req, d_coef, d_resid, d_status, st);
+}
+
+int ort_trace3d_zernike(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* ys, int ny, const double* xs,
+                        int nx, int stop, double a_stop, const ort_opts* opts, const ort_zernike_req* req,
+                        ort_stats* stats, double* coef, double* resid, int32_t* status)
+{
+    if (!ctx) return ORT_EINVAL;
+    if (!opts) return fail(ctx, ORT_EINVAL, "trace3d_zernike: opts is NULL");
+    if (opts->gather_stats) return fail(ctx, ORT_EUNSUPPORTED, "trace3d_zernike: opts.gather_stats is not supported");
+    if (opts->compact) return fail(ctx, ORT_EINVAL, "trace3d_zernike: opts.compact must be 0");
+    if (!(opts->ext & ORT_EXT_OPD)) return fail(ctx, ORT_EINVAL, "trace3d_zernike: opts.ext must hold ORT_EXT_OPD");
+    // the members the fit reads; ort_sweep_scratch traces each one a host call wants into its scratch slot
+    static double tag; static uint8_t mtag;
+    ort_grid_out want;
+    memset(&want, 0, sizeof want);
+    want.opd = want.r = want.theta = &tag; want.mask = &mtag;
+    int rc = grid_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, opts, &want);
+    if (rc || (rc = zernike_req_check(ctx, req, coef, resid, status))) return rc;
+    if ((long long)ny * nx == 0) return fail(ctx, ORT_EINVAL, "trace3d_zernike: empty grid");
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    ScratchScope scratch(ctx, st);
+    const unsigned NN = (unsigned)((long long)ny * nx);
+    const size_t nf = (size_t)n_fields, J = (size_t)(req->n_max + 1) * (req->n_max + 2) / 2;
+    const int gx = grid_dims(ctx, ctx->bps, ort_grid_waves(), opts, n_fields, NN);
+    const size_t nys = (size_t)ny * (opts->ys_per_field ? n_fields : 1);
+    double *d_ys, *d_xs;
+    ENSURE(SL_YS, sizeof(double) * nys, d_ys);
+    ENSURE(SL_XS, sizeof(double) * (size_t)nx, d_xs);
+    RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * nf, d_partials);
+    ort_stats* d_stats; ENSURE(SL_STATS, sizeof(ort_stats) * nf, d_stats);
+    double* d_coef; ENSURE(SL_ZN_COEF, sizeof(double) * nf * J, d_coef);
+    double* d_resid; ENSURE(SL_ZN_RESID, sizeof(double) * nf * 2, d_resid);
+    int32_t* d_status; ENSURE(SL_ZN_STATUS, sizeof(int32_t) * nf, d_status);
+    ort_grid_out full, comp; int* d_tiles;
+    if ((rc = ort_sweep_scratch(ctx, &want, opts, false, NN, n_fields, 1, &full, &comp, &d_tiles))) return rc;
+    CK(cudaMemcpyAsync(d_ys, ys, sizeof(double) * nys, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_xs, xs, sizeof(double) * (size_t)nx, cudaMemcpyHostToDevice, st));
+    rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, nullptr, 1, opts, full, nullptr, d_stats,
+                      d_partials, nullptr, gx, st);
+    if (rc) return rc;
+    ort_wave_sets S;
+    memset(&S, 0, sizeof S);
+    S.n_sets = n_fields; S.stride = NN;
+    S.opd = full.opd; S.r = full.r; S.theta = full.theta; S.mask = full.mask; S.stats = d_stats;
+    if ((rc = zernike_enqueue(ctx, S, req, d_coef, d_resid, d_status, st))) return rc;
+    if (stats) CK(cudaMemcpyAsync(stats, d_stats, sizeof(ort_stats) * nf, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(coef, d_coef, sizeof(double) * nf * J, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(resid, d_resid, sizeof(double) * nf * 2, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(status, d_status, sizeof(int32_t) * nf, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return ORT_OK;
+}
+
 // ------------------------------------------------------------------------------------------
 // arbitrary rays / 2-D / paraxial / transfer / candidates: host wrappers stage through scratch
 // ------------------------------------------------------------------------------------------

@@ -14,6 +14,7 @@ enum Slot {
     SL_IN0, SL_IN1, SL_IN2, SL_IN3, SL_OUT0, SL_OUT1, SL_OUT2, SL_OUT3, SL_OUT4, SL_SINK, SL_POLY,
     SL_GATHER, SL_MERGED, SL_AIM, SL_TABLE, SL_CLIST,                                  // communicator: gathered records, merged records, prelude records, merit table
     SL_EN_STATE, SL_EN_HIST, SL_EN_BINS, SL_EN_CAND0, SL_EN_CAND1, SL_EN_COUNTS, SL_EN_RADIUS,   // encircled energy
+    SL_ZN_GPART, SL_ZN_RPART, SL_ZN_CSYM, SL_ZN_COEF, SL_ZN_RESID, SL_ZN_STATUS,              // Zernike fit
     SL_COUNT
 };
 

@@ -934,10 +934,35 @@ def wavefront(surfaces, system, Hs, k_rays=SPOT_RAYS, focus=None, lam=LAMBDA, vi
     of the on-axis map reproduces its W040 -- with the OPL accumulated surface by surface inside the grid
     kernel and closed on the reference sphere."""
     be = _be(backend)
+    p, xs, ys, flds, ext = _wavefront_setup(surfaces, system, Hs, k_rays, focus, vignette, backend, "wavefront")
+    nf = len(flds)
+    out = []
+    for j0 in range(0, nf, _lib.MAX_FIELDS):
+        sl = slice(j0, j0 + _lib.MAX_FIELDS)
+        r = be.trace3d_grid(flds[sl], ys[sl], xs, p["stop"], p["a_stop"], arith=arith, compact=True,
+                            want=("ex", "ey", "opd", "mask", "stats"), ext=ext, opd_scale=-1.0 / lam)
+        for j, H in enumerate(p["Hs"][sl]):
+            st = r["stats"][j]
+            n = int(st["n_kept"])
+            o = r["opd"][j][:n]
+            ex, ey = r["ex"][j][:n], r["ey"][j][:n]
+            out.append(Wavefront(np.concatenate([o, o]), np.concatenate([ex, -ex]), np.concatenate([ey, ey]), float(H),
+                                 math.sqrt(st["m2_opd"] / n) if n else float("nan"), float(st["mean_opd"]),
+                                 float(o.max() - o.min()) if n else float("nan"), stats=r["stats"][j:j + 1].copy()))
+    be.set_apertures(None)
+    return out
+
+
+def _wavefront_setup(surfaces, system, Hs, k_rays, focus, vignette, backend, caller):
+    """The OPD sweep of wavefront() and zernike(): full_trace's prelude, the chief ray of every field through the centre
+    of the stop, the reference sphere (centred on the chief ray's image point, radius = image plane - paraxial exit
+    pupil) and the field records that close the OPL on it.  Leaves the extended layout (image plane in the last medium),
+    polynomial terms and apertures (vignette) set on the backend -> (p, xs, ys, field records, opts.ext bits)."""
+    be = _be(backend)
     layout = _as_layout(surfaces)
     p = _full_trace_setup(layout, system, Hs, k_rays, focus, backend)
     if p["z0"] is not None:
-        raise NotImplementedError("wavefront: RayBasis (finite object) reference wavefront not implemented")
+        raise NotImplementedError(f"{caller}: RayBasis (finite object) reference wavefront not implemented")
     ext = p["ext"].copy()
     ext[-1, 2] = layout.n[-1]                     # the image plane sits in the last medium (no fake refraction)
     nf = len(p["Hs"])
@@ -958,20 +983,58 @@ def wavefront(surfaces, system, Hs, k_rays=SPOT_RAYS, focus=None, lam=LAMBDA, vi
     ys = np.stack([jl_range(p["y1"][j], p["y2"][j], k_rays) for j in range(nf)])
     flds = [dict(mode=0, u=float(p["u"][j]), v=0.0, h_prime=float(p["h_prime"][j]), opd_xc=0.0, opd_yc=float(yc[j]),
                  opd_radius=float(Rr), opl_ref=float(opl_ref[j])) for j in range(nf)]
+    return p, xs, ys, flds, _lib.EXT_OPD | (_lib.EXT_VIGNETTE if vignette else 0)
+
+
+@dataclass
+class ZernikeFit:
+    """EXTENSION (no reference type): Zernike decomposition of the wavefront of one field point -- the OPD map that
+    wavefront() returns, in waves -- over ANSI Z80.28 / OSA terms j = (n(n+2) + m)/2, n <= n_max, each of unit RMS over
+    the unit disk (include/ort_b200.h, ort_wavefront_zernike_dev).  coef[j] multiplies Z_j with index n[j], m[j];
+    the fit is that of the mirrored map, so the terms antisymmetric in x (sin m theta for even m, cos m theta for odd m)
+    are exactly 0.  rms_resid / pv_resid: RMS and PV of the map minus the fit.  status 0 ok, 1 fewer kept rays than
+    fitted terms, 2 singular normal matrix, 3 a non-finite OPD (coef and residuals NaN for status != 0)."""
+    H: float
+    n_max: int
+    n: np.ndarray
+    m: np.ndarray
+    coef: np.ndarray
+    rms_resid: float
+    pv_resid: float
+    status: int
+    n_kept: int
+    stats: np.ndarray = field(repr=False)
+
+
+def zernike_indices(n_max):
+    """(n, m) of the ANSI single index j = 0 .. (n_max + 1)(n_max + 2)/2 - 1"""
+    nm = [(n, m) for n in range(n_max + 1) for m in range(-n, n + 1, 2)]
+    return np.array([a for a, _ in nm], dtype=np.int64), np.array([b for _, b in nm], dtype=np.int64)
+
+
+def zernike(surfaces, system, Hs, n_max=8, k_rays=SPOT_RAYS, focus=None, lam=LAMBDA, vignette=False, norm="stop",
+            backend=None, arith=_lib.FAST):
+    """EXTENSION: Zernike coefficients (waves) of the wavefront of every field point of Hs -> list of ZernikeFit.  The
+    OPD sweep of wavefront() runs full grid on the device and the least-squares fit is made there
+    (ort_trace3d_zernike); only n_max-many coefficients per field cross PCIe.  norm "stop": rho = r / a_stop, the stop
+    rim is the unit circle; "rmax": rho = r / max(r) of the field's kept rays, the reference's RealRayError.r."""
+    if not (isinstance(n_max, (int, np.integer)) and 0 <= n_max <= _lib.ZERN_MAX_ORDER):
+        raise ValueError(f"zernike: n_max must be an integer in [0, {_lib.ZERN_MAX_ORDER}]")
+    if norm not in ("stop", "rmax"):
+        raise ValueError("zernike: norm is 'stop' or 'rmax'")
+    be = _be(backend)
+    p, xs, ys, flds, ext = _wavefront_setup(surfaces, system, Hs, k_rays, focus, vignette, backend, "zernike")
+    r_norm = p["a_stop"] if norm == "stop" else 0.0
+    ni, mi = zernike_indices(int(n_max))
     out = []
-    for j0 in range(0, nf, _lib.MAX_FIELDS):
+    for j0 in range(0, len(flds), _lib.MAX_FIELDS):
         sl = slice(j0, j0 + _lib.MAX_FIELDS)
-        r = be.trace3d_grid(flds[sl], ys[sl], xs, p["stop"], p["a_stop"], arith=arith, compact=True,
-                            want=("ex", "ey", "opd", "mask", "stats"), ext=_lib.EXT_OPD | (_lib.EXT_VIGNETTE if vignette else 0),
-                            opd_scale=-1.0 / lam)
+        z = be.trace3d_zernike(flds[sl], ys[sl], xs, p["stop"], p["a_stop"], int(n_max), r_norm, arith=arith, ext=ext,
+                               opd_scale=-1.0 / lam)
         for j, H in enumerate(p["Hs"][sl]):
-            st = r["stats"][j]
-            n = int(st["n_kept"])
-            o = r["opd"][j][:n]
-            ex, ey = r["ex"][j][:n], r["ey"][j][:n]
-            out.append(Wavefront(np.concatenate([o, o]), np.concatenate([ex, -ex]), np.concatenate([ey, ey]), float(H),
-                                 math.sqrt(st["m2_opd"] / n) if n else float("nan"), float(st["mean_opd"]),
-                                 float(o.max() - o.min()) if n else float("nan"), stats=r["stats"][j:j + 1].copy()))
+            out.append(ZernikeFit(float(H), int(n_max), ni.copy(), mi.copy(), z["coef"][j].copy(), float(z["resid"][j][0]),
+                                  float(z["resid"][j][1]), int(z["status"][j]), int(z["stats"][j]["n_kept"]),
+                                  z["stats"][j:j + 1].copy()))
     be.set_apertures(None)
     return out
 
