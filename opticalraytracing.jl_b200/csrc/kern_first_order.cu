@@ -10,7 +10,11 @@
 // asin / sin / atan are CUDA's double-precision libm (<= 2 ulp; Julia's own libm differs in the
 // last ulp too), so parity here is 1e-12 relative, not bit-exact.
 // ------------------------------------------------------------------------------------------
-// one iteration of the surface loop of src/RayTracing.jl:151-167; returns ts[i] (:160)
+// one iteration of the surface loop of src/RayTracing.jl:151-167; returns ts[i] (:160).
+// `aspheric` selects the method: 0 = AbstractMatrix / Layout{Spherical} (K forced to 0, asin(tilt(y, R)) :162, :101),
+// 1 = Layout{Aspheric} (K from the layout, atan(tilt(y, R, K, p)) on EVERY surface, :98, :171-173).  The reference tests
+// iszero(Ks) && ps === zero, and a Layout{Aspheric} holds Polynomial(zero) in p, which is not === zero (src/Types.jl:27,
+// 91), so the branch is chosen per layout, never per surface.  `pc` is non-null only with aspheric = 1.
 template <class SurfT>
 __device__ __forceinline__ double trace2d_step(const SurfT& S, int aspheric, double& y, double& U, double& sprev,
                                                unsigned& flags, const double* pc = nullptr, int npoly = 0)
@@ -31,7 +35,7 @@ __device__ __forceinline__ double trace2d_step(const SurfT& S, int aspheric, dou
     y = SA(y, SM(sg, tU));                                   // :158
     sprev = sg;                                              // ts[i+1] -= s :161
     double theta;
-    if (Ks == 0.0 && !pc) {                                  // iszero(Ks) && p === zero, per surface: asin(tilt(y, R))  :162, :101
+    if (!aspheric) {                                         // asin(tilt(y, R))  :162, :101
         double q = SD(y, S.R);
         if (fabs(q) > 1.0) flags |= ORT_FLAG_DOMAIN;
         theta = asin(q);
@@ -59,7 +63,7 @@ k_trace2d(const __grid_constant__ Presc P, Trace2dArgs A)
     if (A.U_out) A.U_out[i] = U;
     const int nsurf = P.nsurf;
     for (int s = 0; s < nsurf; s++) {
-        const double ts = trace2d_step(P.s[s], A.aspheric, y, U, sprev, flags,
+        const double ts = trace2d_step(P.s[s], A.aspheric, y, U, sprev, flags,     // the caller's layout type
                                        (A.aspheric && P.poly) ? P.poly + (size_t)s * P.npoly : nullptr, P.npoly);
         if (A.ts_out) A.ts_out[(size_t)s * N + i] = ts;
         if (A.y_out) A.y_out[(size_t)(s + 1) * N + i] = y;
@@ -180,7 +184,7 @@ __device__ __forceinline__ double aim_eval(const Presc& P, const AimArgs& A, dou
 {
     double y = A.vary_u ? other : x, U = A.vary_u ? x : other, sprev = 0.0;
     unsigned flags = 0;
-    for (int s = 0; s < A.stop; s++)
+    for (int s = 0; s < A.stop; s++)                       // aspheric: the layout type of the system being aimed
         trace2d_step(P.s[s], A.aspheric, y, U, sprev, flags, (A.aspheric && P.poly) ? P.poly + (size_t)s * P.npoly : nullptr, P.npoly);
     return y;
 }
@@ -789,7 +793,7 @@ template <bool REV>
 __device__ __noinline__ double cand_height(const CandView& V, int upto, int aspheric, double y, double U)
 {
     double sprev = 0.0; unsigned fl = 0;
-    for (int j = 0; j < upto; j++) { const Surf2 S = cand_surf<REV>(V, j); trace2d_step(S, aspheric, y, U, sprev, fl); }
+    for (int j = 0; j < upto; j++) { const Surf2 S = cand_surf<REV>(V, j); trace2d_step(S, aspheric, y, U, sprev, fl); }   // caller's flag
     return y;
 }
 
@@ -841,7 +845,8 @@ __global__ void __launch_bounds__((PAIR ? 4 : 2) * AIM_CPB) k_aim_candidates(con
     int status = 0;
     bool fin = true;
     if (role == 0) {
-        // ---- real chief ray, backwards (:265-296)
+        // ---- real chief ray, backwards (:265-296).  aspheric = 1 whatever A.aspheric: full_trace reaches trace_chief_ray with
+        // a Layout (src/PupilSampling.jl:85), so the reversed system is always built as a Layout{Aspheric} (:272-277)
         const double ybp = A.h_prime;
         double ubp = -SD(nuck, nlast);
         const int rstop = rows - stop_c;
@@ -850,7 +855,7 @@ __global__ void __launch_bounds__((PAIR ? 4 : 2) * AIM_CPB) k_aim_candidates(con
         double y = ybp, U = ubp, sprev = 0.0, csum = 0.0; unsigned fl = 0;
         for (int j = 0; j < k; j++) {
             const Surf2 S = cand_surf<true>(V, j);
-            const double ts = trace2d_step(S, 1, y, U, sprev, fl);
+            const double ts = trace2d_step(S, 1, y, U, sprev, fl);     // reversed Layout{Aspheric}, as above
             csum = (j == 0) ? ts : SA(csum, ts);                       // z = cumsum(ts)  (Types.jl:61-63)
         }
         const double ts_last = SS(V.t[0], sprev);
@@ -861,7 +866,7 @@ __global__ void __launch_bounds__((PAIR ? 4 : 2) * AIM_CPB) k_aim_candidates(con
     } else {
         // ---- real marginal ray (:223-240)
         double ym = SM(1.0, s);
-        auto fm = [&](double yy) { return cand_height<false>(V, stop_c, A.aspheric, yy, 0.0); };
+        auto fm = [&](double yy) { return cand_height<false>(V, stop_c, A.aspheric, yy, 0.0); };   // the system's layout type
         if ((PAIR ? secant_reference_pair(fm, ym, a_stop_signed, tol, &fin, odd) : secant_reference(fm, ym, a_stop_signed, tol, &fin)) < 0 || !fin) status |= 2;
         s_x[2][lane] = ym;
     }
@@ -873,7 +878,7 @@ __global__ void __launch_bounds__((PAIR ? 4 : 2) * AIM_CPB) k_aim_candidates(con
     const double U = SM(fabs(Hrel), Ubar);
     const double u = tan(U);
     double e = role == 0 ? SS(y_EP, SM(u, EP_t)) : SS(-y_EP, SM(u, EP_t));
-    auto edge = [&](double yy) { return cand_height<false>(V, stop_c, A.aspheric, yy, U); };
+    auto edge = [&](double yy) { return cand_height<false>(V, stop_c, A.aspheric, yy, U); };    // the system's layout type
     int st2 = 0;
     if ((PAIR ? secant_polish_pair(edge, e, role == 0 ? a_stop : -a_stop, a_stop, odd) : secant_polish(edge, e, role == 0 ? a_stop : -a_stop, a_stop)) < 0) st2 = 4;
     if (role == 1) { s_e2[lane] = e; s_st[1][lane] |= st2; }

@@ -653,7 +653,8 @@ def _full_trace_setup(surfaces, system, H, k_rays, focus, backend):
     EP_t = real_chief.z[0]
     Ubar = real_chief.u[0]
     U = Hs * Ubar
-    u = np.tan(U)
+    u = np.array([math.tan(x) for x in U])         # the C library's tan, as everywhere else here: numpy's vectorised
+                                                   # tan can round differently in the last bit
     y_EP = abs(real_marginal.y[0])
     y1, y2 = y_EP - u * EP_t, -y_EP - u * EP_t                                   # :99
     y1, y2 = trace_edge_rays(layout, y1, y2, U, stop, a_stop, backend=backend)   # :100

@@ -43,6 +43,14 @@ SINGLET = dict(
     a=np.array([20.0, 20.0]), h=17.787,
 )
 
+# The Cooke triplet as a Layout{Aspheric}, rows [R t n K]: the second element's rear surface a conic, every other curved
+# surface a K = 0 sphere.  A Layout{Aspheric} traces each of those spheres with atan(tilt(y, R, K, p)) (src/Types.jl:27,
+# src/RayTracing.jl:162), the fixture that tells that branch from asin(tilt(y, R)).
+COOKE_ASPHERIC = dict(
+    surfaces=np.column_stack([COOKE["surfaces"], [0.0, 0.0, 0.0, 0.0, -0.6, 0.0, 0.0, 0.0]]),
+    a=COOKE["a"], h=COOKE["h"],
+)
+
 # Parabolic reflector, Layout{Aspheric} rows [R t n K] (test/runtests.jl:335-340)
 PARABOLA = dict(
     surfaces=np.array([[inf, 0.0, 1.0, 0.0], [-100.0, 0.0, -1.0, -1.0]]),
@@ -53,6 +61,7 @@ PARABOLA = dict(
 REFLECTIVE = dict(
     surfaces=np.array([[inf, 0.0, 1.0], [-100.0, -24.0, -1.0], [50.0, -3.0, -1.5], [-50.0, 0.0, -1.0]]),
     a=np.array([15.0, 11.0, 11.0]), h=10.0,
+    K=np.array([0.0, 0.0, -0.5, 0.0]),     # as a Layout{Aspheric}: a K = 0 mirror first, one conic behind it
 )
 
 # 10-glass-surface double-Gauss, f/3-class (BASELINE config 2/3; NOT in the reference -- synthetic,
@@ -107,3 +116,15 @@ def perturbed_triplets(C, seed=7):
     out[:, 2, :] = S[:, 2]
     out[:, 3, :] = 0.0
     return out
+
+
+def reversed_chief_layout(surfaces, bfd, K=None):
+    """The reversed system trace_chief_ray traces for a Layout (src/RayTracing.jl:267-277): rev_R = -[Inf; R[end:-1:2]],
+    rev_t = t[end:-1:1] with rev_t[1] = BFD, rev_n = n[end:-1:1] and K = reverse(K) -- one row off against rev_R, as
+    the reference builds it.  Returns ([R t n] rows, K); the reversed system is always a Layout{Aspheric}."""
+    S = np.asarray(surfaces, dtype=np.float64)
+    rev_t = S[::-1, 1].copy()
+    rev_t[0] = bfd
+    rev = np.column_stack([-np.concatenate([[inf], S[:0:-1, 0]]), rev_t, S[::-1, 2]])
+    Kr = (np.zeros(S.shape[0]) if K is None else np.asarray(K, dtype=np.float64))[::-1].copy()
+    return rev, Kr

@@ -27,9 +27,10 @@ def _dec(x):
     return D(repr(float(x))) if not isinstance(x, Decimal) else x          # exact: repr(float) round-trips
 
 
-def trace(surfaces, y, x, u, v, K=None):
+def trace(surfaces, y, x, u, v, K=None, dirs=None):
     """surfaces: rows x 3 [R t n] (row 0 = object space, as the reference's Layout); slopes u = tan U, v = tan V.
-    -> (xs, ys, d, status): hit coordinates at surfaces 1 .. rows-1, final direction, "ok" | "miss" | "tir"."""
+    -> (xs, ys, d, status): hit coordinates at surfaces 1 .. rows-1, final direction, "ok" | "miss" | "tir".
+    dirs, if a list, receives the unit direction after every surface traced."""
     rows = len(surfaces)
     R = [float(r[0]) for r in surfaces]
     t = [float(r[1]) for r in surfaces]
@@ -87,4 +88,6 @@ def trace(surfaces, y, x, u, v, K=None):
             d = [mu * d[j] + gco * N[j] for j in range(3)]
         l = (d[0] * d[0] + d[1] * d[1] + d[2] * d[2]).sqrt()
         d = [a / l for a in d]
+        if dirs is not None:
+            dirs.append(d)
     return xs, ys, d, "ok"

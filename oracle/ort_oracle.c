@@ -313,7 +313,10 @@ ORC_API unsigned orc_trace2d(int rows, const double *R, const double *t, const d
         y += s * tan(U);                                       /* :158 */
         ts[i] += s; ts[i + 1] -= s;                            /* :160-161 */
         double theta;
-        if (Ks == 0.0 && !poly_on(i + 1)) {                    /* iszero(Ks) && ps === zero, per surface  :162 */
+        /* iszero(Ks) && ps === zero  :162.  A Layout{Aspheric} fills p with Polynomial(zero), which is not === zero
+         * (src/Types.jl:27, 91), so the choice is per layout: every surface of it takes atan, K = 0 spheres and
+         * planes included. */
+        if (!aspheric) {
             double q = y / Rs;                                 /* tilt(y,R) :101 */
             if (fabs(q) > 1.0) flags |= F_DOMAIN;              /* Julia asin throws */
             theta = asin(q);

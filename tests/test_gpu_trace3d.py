@@ -278,7 +278,7 @@ class _NoAimFields:
         return getattr(self._c, name)
 
 
-@pytest.mark.parametrize("name", ["COOKE", "DOUBLE_GAUSS", "TESSAR", "SINGLET"])
+@pytest.mark.parametrize("name", ["COOKE", "DOUBLE_GAUSS", "TESSAR", "SINGLET", "COOKE_ASPHERIC"])
 def test_one_call_prelude_equals_host_prelude(ctx, ort, name):
     """ort_aim_fields (the whole full_trace prelude of a field sweep in one call) against the host prelude that drives
     k_paraxial / k_aim2d / k_trace2d step by step: the same device arithmetic, so the aimed quantities agree to the last
@@ -295,9 +295,37 @@ def test_one_call_prelude_equals_host_prelude(ctx, ort, name):
     assert pa["stop"] == pb["stop"] and np.array_equal(pa["ext"], pb["ext"])
     ea = ort.full_trace_fields(system.layout, system, Hs, 64, backend=ctx)
     eb = ort.full_trace_fields(system.layout, system, Hs, 64, backend=_NoAimFields(ctx))
-    for a, b in zip(ea, eb):
-        assert abs(len(a.x) - len(b.x)) <= 4                      # the two rim rays of a field may flip with the last bit
-        assert abs(a.RMS / b.RMS - 1) < 1e-3
+    scale = max(np.max(np.abs(pb["h_prime"])), pb["y_EP"])
+    for j, (a, b) in enumerate(zip(ea, eb)):
+        ya, yb = ort.host.jl_range(pa["y1"][j], pa["y2"][j], 64), ort.host.jl_range(pb["y1"][j], pb["y2"][j], 64)
+        ka, kb = _kept_mask(ctx, ort, pa, j, ya), _kept_mask(ctx, ort, pb, j, yb)
+        rim = np.zeros_like(ka)
+        rim[[0, 63], :] = True                                       # the two rim rays (y1, y2) of every x column
+        assert not np.any((ka != kb) & ~rim)                          # masks differ at most on the rim rays
+        common = (ka & kb).reshape(-1)
+        sa, sb = _spot(ctx, ort, pa, j, ya), _spot(ctx, ort, pb, j, yb)
+        for q in range(2):
+            assert np.max(np.abs(sa[q][common] - sb[q][common])) <= 1e-12 * scale
+        ra, rb = (np.sqrt(np.mean(sa[0][common] ** 2 + (sa[1][common] - sa[1][common].mean()) ** 2)),
+                  np.sqrt(np.mean(sb[0][common] ** 2 + (sb[1][common] - sb[1][common].mean()) ** 2)))
+        assert abs(ra / rb - 1) <= 1e-12
+        assert abs(len(a.x) - len(b.x)) <= 4 and np.all(np.isfinite([a.RMS, b.RMS]))
+
+
+def _grid(ctx, ort, p, j, ys, want):
+    ctx.set_layout(p["ext"], p["K"])
+    xs = ort.host.jl_range(0.0, p["y_EP"], 32)
+    return ctx.trace3d_grid([dict(u=p["u"][j], v=0.0, h_prime=p["h_prime"][j])], ys, xs, p["stop"], p["a_stop"],
+                            arith=ort.STRICT, want=want)
+
+
+def _kept_mask(ctx, ort, p, j, ys):
+    return _grid(ctx, ort, p, j, ys, ("mask",))["mask"][0].reshape(64, 32).astype(bool)
+
+
+def _spot(ctx, ort, p, j, ys):
+    r = _grid(ctx, ort, p, j, ys, ("ex", "ey"))
+    return r["ex"][0], r["ey"][0]
 
 
 def test_rays_device_pointer_form(ctx, ort):
@@ -404,6 +432,7 @@ def test_candidates_aimed_other_systems(ctx, orc, pre, ort, name, H, conic):
         if conic:
             RtnK[c, 3] = np.where(np.isfinite(S[:, 0]), rng.uniform(-0.6, 0.3, rows), 0.0)
             RtnK[c, 3, 0] = 0.0
+            RtnK[c, 3, 1 + (c % 2)::2] = 0.0        # K exactly 0 on every other surface: the atan branch on spheres
     aim = ctx.aim_candidates(RtnK, P["a"], P["h"], H, aspheric=conic)
     assert np.all(aim[:, 11] == 0.0)
     for c in range(C):
