@@ -41,8 +41,9 @@ extern "C" {
 
 #define ORT_VERSION 200 /* 0.2.0: communicator inside the library, ort_opts.gather_stats, ort_grid_out.stats_local;
                            ort_trace3d_focus / ort_trace3d_focus_dev (through-focus sweep) and ort_spot_energy_dev /
-                           ort_trace3d_energy (encircled energy) and ort_wavefront_zernike_dev / ort_trace3d_zernike
-                           (Zernike fit of the wavefront) added without a version change */
+                           ort_trace3d_energy (encircled energy), ort_wavefront_zernike_dev / ort_trace3d_zernike
+                           (Zernike fit of the wavefront) and ort_wavefront_psf_dev / ort_trace3d_psf (diffraction PSF)
+                           added without a version change */
 
 /* status codes */
 #define ORT_OK            0
@@ -343,6 +344,57 @@ int ort_wavefront_zernike_dev(ort_ctx *ctx, const ort_wave_sets *sets /* host st
 int ort_trace3d_zernike(ort_ctx *ctx, const ort_field *fields, int n_fields, const double *ys, int ny, const double *xs,
                         int nx, int stop, double a_stop, const ort_opts *opts, const ort_zernike_req *req,
                         ort_stats *stats, double *coef, double *resid, int32_t *status);
+
+/* ---- EXTENSION (no reference method): diffraction point-spread function and Strehl ratio of the ray-traced wavefront,
+ *      computed on the device from the outputs of a grid sweep with ORT_EXT_OPD in full-grid form (opts.compact = 0).
+ *      A SET is one field of such a sweep; its kept rays are those with mask == 1, n = stats[s].n_kept.  W_i = opd of ray
+ *        i (the Python host sweeps with opd_scale = -1/lambda: W in waves, the map Wavefront.opd holds);
+ *        (x_i, y_i) = (xs[ix], ys[s][iy]) its launch coordinates on the pupil grid, i = iy*nx + ix.
+ *      The PSF is that of the MIRRORED 2n-point set that RealRayError, Wavefront, the encircled energy and the Zernike fit
+ *        describe: every traced ray stands for (+-x_i, y_i) with the same W_i (the x = 0 column counts twice):
+ *          E(xi, eta)   = sum_{kept i} sum_{sigma = +-1} exp(2 pi i (W_i + s (sigma x_i xi + y_i eta)))
+ *                       = sum_i 2 cos(2 pi s x_i xi) exp(2 pi i (W_i + s y_i eta))
+ *          psf(xi, eta) = |E|^2 / (2n)^2        (1 = the diffraction-limited peak of the same, possibly vignetted, pupil)
+ *          strehl_ref   = |sum_i exp(2 pi i W_i)|^2 / n^2     (psf at xi = eta = 0)
+ *      Pixel (iu, iv) sits at xi = (iu - (n_u-1)/2) du, eta = (iv - (n_v-1)/2) dv, relative to the centre of the
+ *        reference sphere (opd_xc, opd_yc), the chief ray's image point; xi runs along x (sagittal), eta along y.
+ *      s = req.scale > 0, in cycles per (pupil unit x image unit).  The Python host passes s = 1/(lambda f), f = system.f:
+ *        the sine-condition mapping of an entrance-pupil height h to the image-space direction sine h/f, i.e. the scalar
+ *        Fraunhofer ("FFT PSF") model.  Obliquity, amplitude apodisation and pupil distortion are neglected.
+ *      The grid wraps (aliases) with period 1/(s dx) in xi and 1/(s dy) in eta for uniform pupil steps dx, dy.
+ *      Outputs per set s:
+ *        psf[s][n_v][n_u];
+ *        strehl[s][2]   (strehl_ref, the maximum of psf over the pixel grid);
+ *        peak[s]        iv*n_u + iu of that maximum, the lowest index on a tie;
+ *        status[s]      0 ok; 1 n = 0; 3 a kept ray has a non-finite opd (the codes of the Zernike fit; 2 is unused).
+ *                       For status != 0 psf and strehl are NaN and peak is -1.
+ *      The device may use y - ybar_s for phase accuracy (|E|^2 does not change).  Determinism: no floating-point atomics,
+ *      partial sums folded in a fixed order: bit-identical run to run on one device, not bit-equal to numpy. */
+#define ORT_PSF_MAX_SIDE 1024
+typedef struct ort_psf_req {
+    int32_t n_u, n_v;               /* pixels along xi and eta, 1 .. ORT_PSF_MAX_SIDE */
+    double  du, dv;                 /* pixel pitch in image units, finite and > 0 */
+    double  scale;                  /* s, finite and > 0 */
+} ort_psf_req;
+/* Device form (enqueue only on `stream`): the sets already in HBM in full-grid form (sets->mask required; r and theta are
+ * not read), d_ys [ys_per_set ? n_sets : 1][ny] and d_xs [nx] the grid coordinates on the device.  d_psf
+ * [n_sets][n_v][n_u], d_strehl [n_sets][2], d_peak and d_status [n_sets].  ORT_EINVAL before anything is enqueued for:
+ * a NULL array, stride != ny*nx, ny or nx < 1, n_sets outside [1, ORT_MAX_FIELDS], n_u or n_v outside
+ * [1, ORT_PSF_MAX_SIDE], du, dv or scale not finite or <= 0.  Launches five kernels whatever the sizes.  Scratch: the
+ * stage-A products take 16 n_sets kx ny nup bytes (nup = ceil(n_u / 2) rounded up to 64 or 128, kx <= 4 chunks of nx),
+ * about 2 kx nup / nx times the OPD input: small on wide grids, large on tall narrow ones (nx = 1 at n_u 1024 is 8 KB
+ * per pupil row per set); the stage-B partials take 16 n_sets ky n_v ceil(n_u / 2) bytes (ky > 1 only while the pixel
+ * tiles alone leave SMs idle).  A scratch that cannot grow is ORT_ENOMEM. */
+int ort_wavefront_psf_dev(ort_ctx *ctx, const ort_wave_sets *sets /* host struct */, const double *d_ys, int ys_per_set,
+                          int ny, const double *d_xs, int nx, const ort_psf_req *req, double *d_psf, double *d_strehl,
+                          int32_t *d_peak, int32_t *d_status, void *stream);
+/* Host form: the grid sweep of the layout (polynomial terms and vignetting accepted as by ort_trace3d_grid) full grid
+ * into the context's scratch with opd, mask and stats, then the PSF on it; only stats [n_fields] (may be NULL),
+ * psf [n_fields][n_v][n_u], strehl [n_fields][2], peak and status [n_fields] cross PCIe.  opts.ext must hold ORT_EXT_OPD
+ * and opts.compact must be 0 (ORT_EINVAL); opts.gather_stats is ORT_EUNSUPPORTED. */
+int ort_trace3d_psf(ort_ctx *ctx, const ort_field *fields, int n_fields, const double *ys, int ny, const double *xs, int nx,
+                    int stop, double a_stop, const ort_opts *opts, const ort_psf_req *req, ort_stats *stats, double *psf,
+                    double *strehl, int32_t *peak, int32_t *status);
 
 /* ---- 3-D skew trace of N arbitrary rays, all surfaces recorded: replaces
  *      raytrace(surfaces, y, x, U, V, Vector{RealRay}) src/PupilSampling.jl:34-65 for a batch.

@@ -340,11 +340,10 @@ struct OrtZernikeReq
 end
 const ORT_EXT_OPD, ORT_EXT_VIGNETTE = Int32(1), Int32(2)
 
-function zernike(::B200, surfaces::Layout, system::System, H::Float64; n_max::Int = 8, k_rays::Int = spot_rays,
-                 focus = nothing, λ = 587.5618e-6, vignette::Bool = false, norm::Symbol = :stop, arith = ORT_ARITH_FAST)
-    require_conic(surfaces)
-    0 ≤ n_max ≤ 12 || throw(DomainError(n_max, "0 ≤ n_max ≤ 12"))
-    norm ∈ (:stop, :rmax) || throw(ArgumentError("norm is :stop or :rmax"))
+# The OPD sweep of the Python host's wavefront() for one field point: full_trace's prelude, the chief ray through the
+# centre of the stop, the reference sphere centred on its image point with radius image plane - paraxial exit pupil.
+# Leaves the extended layout (image plane in the last medium) and the apertures (vignette) set.
+function opd_sweep_setup(surfaces::Layout, system::System, H::Float64, k_rays::Int, focus, vignette::Bool)
     H = abs(H)
     H ≤ 1.0 || throw(DomainError(H, "Domain: |H| ≤ 1.0"))
     focus === nothing && (focus = system.marginal.z[end] - system.marginal.z[end-1])   # :87
@@ -381,6 +380,15 @@ function zernike(::B200, surfaces::Layout, system::System, H::Float64; n_max::In
     field = OrtField(0, 0, u, 0.0, 0.0, 0.0, u * system.f, 0.0, yv[end], Rr, opl_ref)
     ys = collect(range(y1, y2, k_rays))              # :121
     xs = collect(range(0.0, y_EP, div(k_rays, 2)))   # :122
+    return field, ys, xs, stop, a_stop, y_EP
+end
+
+function zernike(::B200, surfaces::Layout, system::System, H::Float64; n_max::Int = 8, k_rays::Int = spot_rays,
+                 focus = nothing, λ = 587.5618e-6, vignette::Bool = false, norm::Symbol = :stop, arith = ORT_ARITH_FAST)
+    require_conic(surfaces)
+    0 ≤ n_max ≤ 12 || throw(DomainError(n_max, "0 ≤ n_max ≤ 12"))
+    norm ∈ (:stop, :rmax) || throw(ArgumentError("norm is :stop or :rmax"))
+    field, ys, xs, stop, a_stop, _ = opd_sweep_setup(surfaces, system, H, k_rays, focus, vignette)
     J = (n_max + 1) * (n_max + 2) ÷ 2
     stats = [OrtStats(0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0)]
     coef = zeros(J); resid = zeros(2); status = zeros(Int32, 1)
@@ -394,6 +402,47 @@ function zernike(::B200, surfaces::Layout, system::System, H::Float64; n_max::In
     check(ccall((:ort_set_apertures, LIB), Cint, (Ptr{Cvoid}, Cint, Ptr{Float64}), ctx(), 0, C_NULL))
     nm = [(nn, m) for nn in 0:n_max for m in -nn:2:nn]
     return (n = first.(nm), m = last.(nm), coef = coef, rms_resid = resid[1], pv_resid = resid[2],
+            status = Int(status[1]), n_kept = stats[1].n_kept)
+end
+
+# --- Diffraction PSF and Strehl ratio of the wavefront (EXTENSION, no reference method) ---------------------------
+# The OPD sweep of zernike, then ONE ccall (ort_trace3d_psf) that sweeps the pupil grid with ORT_EXT_OPD on the device
+# and computes the scalar Fraunhofer PSF of the mirrored pupil there, s = 1/(λ f): pupil height h maps to the image-space
+# direction sine h/f (obliquity, apodisation and pupil distortion neglected).  psf is n_u × n_v: psf[iu, iv] is pixel
+# (iu, iv) of the C layout [iv][iu]; u, v are the pixel centres in mm from the chief ray's image point.
+# strehl: psf at that point; peak: the maximum over the grid.  Only the pixel grid crosses PCIe.  Not runnable here (no
+# Julia); the Python host's psf is the tested form of the same calls.
+struct OrtPsfReq
+    n_u::Int32; n_v::Int32; du::Float64; dv::Float64; scale::Float64
+end
+
+function psf(::B200, surfaces::Layout, system::System, H::Float64; n_pix = nothing, pixel = nothing,
+             k_rays::Int = spot_rays, focus = nothing, λ = 587.5618e-6, vignette::Bool = false, arith = ORT_ARITH_FAST)
+    require_conic(surfaces)
+    n_u, n_v = n_pix === nothing ? (k_rays - 1, k_rays - 1) : n_pix isa Integer ? (n_pix, n_pix) : Tuple(n_pix)
+    (1 ≤ n_u ≤ 1024 && 1 ≤ n_v ≤ 1024) || throw(DomainError(n_pix, "1 ≤ n_pix ≤ 1024"))
+    s = 1.0 / (λ * system.f)
+    field, ys, xs, stop, a_stop, y_EP = opd_sweep_setup(surfaces, system, H, k_rays, focus, vignette)
+    du, dv = pixel === nothing ? (1 / (4 * s * y_EP), 1 / (4 * s * y_EP)) : pixel isa Real ? (pixel, pixel) : Tuple(pixel)
+    dx, dy = length(xs) > 1 ? xs[2] - xs[1] : 0.0, length(ys) > 1 ? abs(ys[2] - ys[1]) : 0.0
+    if !(n_u * du * s * dx ≤ 1 + 1e-9 && n_v * dv * s * dy ≤ 1 + 1e-9)
+        check(ccall((:ort_set_apertures, LIB), Cint, (Ptr{Cvoid}, Cint, Ptr{Float64}), ctx(), 0, C_NULL))
+        throw(ArgumentError("the pixel grid exceeds the alias period of the pupil grid: raise k_rays"))
+    end
+    stats = [OrtStats(0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0)]
+    img = zeros(n_u, n_v); strehl = zeros(2); peak = zeros(Int32, 1); status = zeros(Int32, 1)
+    opts = Ref(OrtOpts(arith, 0, 0, ORT_EXT_OPD | (vignette ? ORT_EXT_VIGNETTE : Int32(0)), 0.0, 1.0, -1.0 / λ, 0, 0))
+    req = Ref(OrtPsfReq(n_u, n_v, du, dv, s))
+    check(ccall((:ort_trace3d_psf, LIB), Cint,
+                (Ptr{Cvoid}, Ref{OrtField}, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint, Float64, Ref{OrtOpts},
+                 Ref{OrtPsfReq}, Ptr{OrtStats}, Ptr{Float64}, Ptr{Float64}, Ptr{Int32}, Ptr{Int32}),
+                ctx(), Ref(field), 1, ys, length(ys), xs, length(xs), stop, a_stop, opts, req, stats, img, strehl,
+                peak, status))
+    check(ccall((:ort_set_apertures, LIB), Cint, (Ptr{Cvoid}, Cint, Ptr{Float64}), ctx(), 0, C_NULL))
+    u = ((0:n_u-1) .- (n_u - 1) / 2) .* du
+    v = ((0:n_v-1) .- (n_v - 1) / 2) .* dv
+    return (u = collect(u), v = collect(v), psf = img, strehl = strehl[1], peak = strehl[2],
+            peak_uv = peak[1] < 0 ? (NaN, NaN) : (u[peak[1] % n_u + 1], v[peak[1] ÷ n_u + 1]),
             status = Int(status[1]), n_kept = stats[1].n_kept)
 end
 

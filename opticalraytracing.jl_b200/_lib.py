@@ -23,6 +23,7 @@ MAX_RADII, MAX_FRACS = 1024, 8
 ENERGY_CIRCLE, ENERGY_SQUARE = 0, 1
 CENTER_CENTROID, CENTER_PARAXIAL = 0, 1
 ZERN_MAX_ORDER = 12
+PSF_MAX_SIDE = 1024
 
 # every symbol include/ort_b200.h declares (tests check the .so exports exactly these)
 SYMBOLS = [
@@ -31,6 +32,7 @@ SYMBOLS = [
     "ort_set_layout", "ort_set_apertures", "ort_set_polynomials",
     "ort_trace3d_grid", "ort_trace3d_grid_dev", "ort_trace3d_focus", "ort_trace3d_focus_dev",
     "ort_spot_energy_dev", "ort_trace3d_energy", "ort_wavefront_zernike_dev", "ort_trace3d_zernike",
+    "ort_wavefront_psf_dev", "ort_trace3d_psf",
     "ort_trace3d_rays", "ort_trace3d_rays_opl", "ort_trace3d_rays_dev", "ort_trace2d_batch", "ort_aim2d",
     "ort_paraxial_batch", "ort_paraxial_batch_dev", "ort_transfer_batch", "ort_transfer_batch_dev",
     "ort_trace3d_candidates", "ort_trace3d_candidates_dev", "ort_aim_candidates", "ort_aim_candidates_dev", "ort_aim_fields",
@@ -114,6 +116,10 @@ class WaveSets(C.Structure):
 WAVE_SETS_NAMES = tuple(name for name, _ in WaveSets._fields_)
 
 
+class PsfReq(C.Structure):
+    _fields_ = [("n_u", C.c_int32), ("n_v", C.c_int32), ("du", C.c_double), ("dv", C.c_double), ("scale", C.c_double)]
+
+
 def zernike_terms(n_max):
     """J = (n_max + 1)(n_max + 2) / 2 coefficients per set, in ANSI order"""
     return (int(n_max) + 1) * (int(n_max) + 2) // 2
@@ -168,6 +174,9 @@ def load():
                                             C.c_void_p, C.c_void_p, C.c_void_p]
     L.ort_trace3d_zernike.argtypes = grid_args[:9] + [C.POINTER(Opts), C.POINTER(ZernikeReq), C.c_void_p, C.c_void_p,
                                                       C.c_void_p, C.c_void_p]
+    L.ort_wavefront_psf_dev.argtypes = [C.c_void_p, C.POINTER(WaveSets), C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                        C.c_int, C.POINTER(PsfReq)] + [C.c_void_p] * 5
+    L.ort_trace3d_psf.argtypes = grid_args[:9] + [C.POINTER(Opts), C.POINTER(PsfReq)] + [C.c_void_p] * 5
     L.ort_trace3d_rays.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p]
     L.ort_trace3d_rays_opl.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p, _dp]
     L.ort_trace3d_rays_dev.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 6
@@ -654,6 +663,42 @@ class Context:
                                             float(a_stop), C.byref(op), C.byref(req), stats.ctypes.data,
                                             coef.ctypes.data, resid.ctypes.data, status.ctypes.data))
         return dict(stats=stats, coef=coef, resid=resid, status=status)
+
+    # ---- diffraction PSF of the wavefront ---------------------------------------------------
+    def wavefront_psf_dev(self, sets, d_ys, ys_per_set, ny, d_xs, nx, n_u, n_v, du, dv, scale, d_psf=0, d_strehl=0,
+                          d_peak=0, d_status=0, stream=0):
+        """Diffraction PSF of full-grid wavefront sets already in HBM (ort_wavefront_psf_dev, enqueue only).  sets: dict with
+        n_sets, stride = ny * nx and the device addresses opd, mask, stats (r and theta are not read); d_ys
+        [ys_per_set ? n_sets : 1][ny], d_xs [nx] device addresses.  d_psf: float64 [n_sets][n_v][n_u], d_strehl: float64
+        [n_sets][2], d_peak, d_status: int32 [n_sets] (device addresses)."""
+        ws = WaveSets(*[sets.get(k) or 0 for k in WAVE_SETS_NAMES])
+        req = PsfReq(int(n_u), int(n_v), float(du), float(dv), float(scale))
+        self._ck(self.L.ort_wavefront_psf_dev(self.h, C.byref(ws), C.c_void_p(d_ys or 0), int(ys_per_set), int(ny),
+                                              C.c_void_p(d_xs or 0), int(nx), C.byref(req), C.c_void_p(d_psf or 0),
+                                              C.c_void_p(d_strehl or 0), C.c_void_p(d_peak or 0),
+                                              C.c_void_p(d_status or 0), C.c_void_p(stream)))
+
+    def trace3d_psf(self, fields, ys, xs, stop, a_stop, n_u, n_v, du, dv, scale, arith=FAST, ext=EXT_OPD, opd_scale=1.0):
+        """The grid sweep with ORT_EXT_OPD full grid on the device and the diffraction PSF of every field on it
+        (ort_trace3d_psf); no ray crosses PCIe.  Returns dict(stats (n_fields,), psf (n_fields, n_v, n_u) float64,
+        strehl (n_fields, 2) float64 = strehl_ref, maximum, peak (n_fields,) int32 = iv * n_u + iu, status (n_fields,)
+        int32)."""
+        farr, nf = make_fields(fields)
+        ys, xs = _d(ys), _d(xs)
+        per_field = ys.ndim == 2
+        if per_field and ys.shape[0] != nf:
+            raise ValueError("ys must be (ny,) or (n_fields, ny)")
+        stats = np.zeros(nf, dtype=STATS_DTYPE)
+        psf = np.zeros((nf, max(int(n_v), 0), max(int(n_u), 0)), dtype=np.float64)
+        strehl = np.zeros((nf, 2), dtype=np.float64)
+        peak = np.zeros(nf, dtype=np.int32)
+        status = np.zeros(nf, dtype=np.int32)
+        req = PsfReq(int(n_u), int(n_v), float(du), float(dv), float(scale))
+        op = _opts(arith, False, per_field, ext, opd_scale=opd_scale)
+        self._ck(self.L.ort_trace3d_psf(self.h, farr, nf, _vp(ys), ys.shape[-1], _vp(xs), len(xs), int(stop),
+                                        float(a_stop), C.byref(op), C.byref(req), stats.ctypes.data, psf.ctypes.data,
+                                        strehl.ctypes.data, peak.ctypes.data, status.ctypes.data))
+        return dict(stats=stats, psf=psf, strehl=strehl, peak=peak, status=status)
 
     # ---- arbitrary rays ------------------------------------------------------------------
     def trace3d_rays(self, y0, x0, u0, v0, arith=STRICT, opl=False):

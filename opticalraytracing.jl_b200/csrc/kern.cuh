@@ -80,6 +80,30 @@ struct ZernArgs {
     int* status;                                // [n_sets]
 };
 
+// Diffraction PSF of the wavefront (kern_psf.cu)
+struct PsfArgs {
+    int n_sets, ny, nx;
+    long long stride;
+    const double* opd; const uint8_t* mask; const ort_stats* stats;
+    const double *ys, *xs;                      // ys + s * ys_stride: the iy coordinates of set s
+    long long ys_stride;                        // 0 or ny
+    int n_u, n_v;
+    double du, dv, scale;
+    int nuh, nup;                               // computed columns (xi >= 0) = ceil(n_u / 2); nuh padded to k_psf_x's tile
+    int tx;                                     // k_psf_x threads along the columns: 8 or 16
+    int rt, kx, kx_len;                         // k_psf_x row tiles, ix chunks, ix per chunk
+    int vt, jt, ky, ky_len;                     // k_psf_y iv tiles, j tiles, iy chunks, iy per chunk
+    int fb;                                     // k_psf_fold CTAs per set
+    double* ctab;                               // [nx][nup]: 2 cos(2 pi s x xi)
+    double2* T;                                 // [n_sets][kx][ny][nup]: stage A, one partial per ix chunk
+    double* rsum;                               // [n_sets][rt][kx][3]: sum P (re, im), 1.0 if a kept opd is not finite
+    double2* E;                                 // [n_sets][ky][n_v][nuh]: stage B, one partial per iy chunk
+    double* bval; int* bidx;                    // [n_sets][fb]: per-CTA maximum of the PSF and its grid index
+    double* psf;                                // [n_sets][n_v][n_u]
+    double* strehl;                             // [n_sets][2]
+    int *peak, *status;                         // [n_sets]
+};
+
 struct CompactArgs {
     unsigned NN;
     const uint8_t* mask;
@@ -242,6 +266,10 @@ int zern_fitted_terms(int n_max);
 cudaError_t zern_dims(ZernArgs& A, int sm_count);
 size_t zern_gram_record(const ZernArgs& A);
 cudaError_t launch_zernike(const ZernArgs& A, cudaStream_t st, int* launches);
+// diffraction PSF: psf_dims fills nuh .. fb from n_sets, ny, nx, n_u and n_v (the scratch sizes follow from them);
+// launch_psf enqueues the five kernels
+cudaError_t psf_dims(PsfArgs& A, int sm_count);
+cudaError_t launch_psf(const PsfArgs& A, cudaStream_t st, int* launches);
 cudaError_t launch_rays(const Presc& P, const RaysArgs& A, int arith, cudaStream_t st);
 cudaError_t launch_candidates(const CandArgs& A, int arith, cudaStream_t st, int sm_count);
 cudaError_t launch_trace2d(const Presc& P, const Trace2dArgs& A, cudaStream_t st);

@@ -992,6 +992,132 @@ int ort_trace3d_zernike(ort_ctx* ctx, const ort_field* fields, int n_fields, con
     return ORT_OK;
 }
 
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------
+// Diffraction PSF of the wavefront (kern_psf.cu)
+// ------------------------------------------------------------------------------------------
+static int psf_req_check(ort_ctx* ctx, const ort_psf_req* req, const void* psf, const void* strehl, const void* peak,
+                         const void* status)
+{
+    if (!req) return fail(ctx, ORT_EINVAL, "psf: req is NULL");
+    if (req->n_u < 1 || req->n_u > ORT_PSF_MAX_SIDE || req->n_v < 1 || req->n_v > ORT_PSF_MAX_SIDE)
+        return fail(ctx, ORT_EINVAL, "psf: n_u = %d, n_v = %d not in [1, %d]", req->n_u, req->n_v, ORT_PSF_MAX_SIDE);
+    if (!(isfinite(req->du) && req->du > 0.0) || !(isfinite(req->dv) && req->dv > 0.0) ||
+        !(isfinite(req->scale) && req->scale > 0.0))
+        return fail(ctx, ORT_EINVAL, "psf: du = %g, dv = %g, scale = %g must be finite and > 0", req->du, req->dv,
+                    req->scale);
+    if (!psf || !strehl || !peak || !status) return fail(ctx, ORT_EINVAL, "psf: psf, strehl, peak or status is NULL");
+    return ORT_OK;
+}
+
+// Enqueue the five PSF kernels over `sets` on st (inside the entry point's ScratchScope); one ProfScope around them
+static int psf_enqueue(ort_ctx* ctx, const ort_wave_sets& S, const double* d_ys, int ys_per_set, int ny,
+                       const double* d_xs, int nx, const ort_psf_req* req, double* d_psf, double* d_strehl,
+                       int32_t* d_peak, int32_t* d_status, cudaStream_t st)
+{
+    PsfArgs A;
+    memset(&A, 0, sizeof A);
+    A.n_sets = S.n_sets; A.ny = ny; A.nx = nx; A.stride = S.stride;
+    A.opd = S.opd; A.mask = S.mask; A.stats = S.stats;
+    A.ys = d_ys; A.ys_stride = ys_per_set ? ny : 0; A.xs = d_xs;
+    A.n_u = req->n_u; A.n_v = req->n_v; A.du = req->du; A.dv = req->dv; A.scale = req->scale;
+    CK(psf_dims(A, ctx->sm_count));
+    const size_t ns = (size_t)S.n_sets;
+    ENSURE(SL_PSF_CTAB, sizeof(double) * (size_t)nx * A.nup, A.ctab);
+    ENSURE(SL_PSF_T, sizeof(double2) * ns * A.kx * (size_t)ny * A.nup, A.T);
+    ENSURE(SL_PSF_RSUM, sizeof(double) * 3 * ns * A.rt * A.kx, A.rsum);
+    ENSURE(SL_PSF_E, sizeof(double2) * ns * A.ky * A.n_v * A.nuh, A.E);
+    ENSURE(SL_PSF_BVAL, sizeof(double) * ns * A.fb, A.bval);
+    ENSURE(SL_PSF_BIDX, sizeof(int) * ns * A.fb, A.bidx);
+    A.psf = d_psf; A.strehl = d_strehl; A.peak = (int*)d_peak; A.status = (int*)d_status;
+    int n = 0;
+    {
+        ProfScope prof(ctx, st);
+        CK(launch_psf(A, st, &n));
+    }
+    ctx->launches += n;
+    return ORT_OK;
+}
+
+extern "C" {
+
+int ort_wavefront_psf_dev(ort_ctx* ctx, const ort_wave_sets* sets, const double* d_ys, int ys_per_set, int ny,
+                          const double* d_xs, int nx, const ort_psf_req* req, double* d_psf, double* d_strehl,
+                          int32_t* d_peak, int32_t* d_status, void* stream)
+{
+    if (!ctx) return ORT_EINVAL;
+    if (!sets) return fail(ctx, ORT_EINVAL, "wavefront_psf: sets is NULL");
+    if (sets->n_sets < 1 || sets->n_sets > ORT_MAX_FIELDS)
+        return fail(ctx, ORT_EINVAL, "wavefront_psf: n_sets = %d not in [1, %d]", sets->n_sets, ORT_MAX_FIELDS);
+    if (ny < 1 || nx < 1 || sets->stride != (long long)ny * nx || sets->stride >= (1LL << 31))
+        return fail(ctx, ORT_EINVAL, "wavefront_psf: stride = %lld is not ny*nx = %d*%d >= 1 (< 2^31)",
+                    (long long)sets->stride, ny, nx);
+    if (!sets->opd || !sets->mask || !sets->stats || !d_ys || !d_xs)
+        return fail(ctx, ORT_EINVAL, "wavefront_psf: opd, mask, stats, ys or xs is NULL");
+    int rc = psf_req_check(ctx, req, d_psf, d_strehl, d_peak, d_status);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    ScratchScope scratch(ctx, st);
+    return psf_enqueue(ctx, *sets, d_ys, ys_per_set, ny, d_xs, nx, req, d_psf, d_strehl, d_peak, d_status, st);
+}
+
+int ort_trace3d_psf(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* ys, int ny, const double* xs, int nx,
+                    int stop, double a_stop, const ort_opts* opts, const ort_psf_req* req, ort_stats* stats, double* psf,
+                    double* strehl, int32_t* peak, int32_t* status)
+{
+    if (!ctx) return ORT_EINVAL;
+    if (!opts) return fail(ctx, ORT_EINVAL, "trace3d_psf: opts is NULL");
+    if (opts->gather_stats) return fail(ctx, ORT_EUNSUPPORTED, "trace3d_psf: opts.gather_stats is not supported");
+    if (opts->compact) return fail(ctx, ORT_EINVAL, "trace3d_psf: opts.compact must be 0");
+    if (!(opts->ext & ORT_EXT_OPD)) return fail(ctx, ORT_EINVAL, "trace3d_psf: opts.ext must hold ORT_EXT_OPD");
+    // the members the PSF reads; ort_sweep_scratch traces each one a host call wants into its scratch slot
+    static double tag; static uint8_t mtag;
+    ort_grid_out want;
+    memset(&want, 0, sizeof want);
+    want.opd = &tag; want.mask = &mtag;
+    int rc = grid_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, opts, &want);
+    if (rc || (rc = psf_req_check(ctx, req, psf, strehl, peak, status))) return rc;
+    if (ny < 1 || nx < 1) return fail(ctx, ORT_EINVAL, "trace3d_psf: empty grid");
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    ScratchScope scratch(ctx, st);
+    const unsigned NN = (unsigned)((long long)ny * nx);
+    const size_t nf = (size_t)n_fields, npix = (size_t)req->n_u * req->n_v;
+    const int gx = grid_dims(ctx, ctx->bps, ort_grid_waves(), opts, n_fields, NN);
+    const size_t nys = (size_t)ny * (opts->ys_per_field ? n_fields : 1);
+    double *d_ys, *d_xs;
+    ENSURE(SL_YS, sizeof(double) * nys, d_ys);
+    ENSURE(SL_XS, sizeof(double) * (size_t)nx, d_xs);
+    RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * nf, d_partials);
+    ort_stats* d_stats; ENSURE(SL_STATS, sizeof(ort_stats) * nf, d_stats);
+    double* d_psf; ENSURE(SL_PSF_OUT, sizeof(double) * nf * npix, d_psf);
+    double* d_strehl; ENSURE(SL_PSF_STREHL, sizeof(double) * nf * 2, d_strehl);
+    int32_t* d_peak; ENSURE(SL_PSF_PEAK, sizeof(int32_t) * nf, d_peak);
+    int32_t* d_status; ENSURE(SL_PSF_STATUS, sizeof(int32_t) * nf, d_status);
+    ort_grid_out full, comp; int* d_tiles;
+    if ((rc = ort_sweep_scratch(ctx, &want, opts, false, NN, n_fields, 1, &full, &comp, &d_tiles))) return rc;
+    CK(cudaMemcpyAsync(d_ys, ys, sizeof(double) * nys, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_xs, xs, sizeof(double) * (size_t)nx, cudaMemcpyHostToDevice, st));
+    rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, nullptr, 1, opts, full, nullptr, d_stats,
+                      d_partials, nullptr, gx, st);
+    if (rc) return rc;
+    ort_wave_sets S;
+    memset(&S, 0, sizeof S);
+    S.n_sets = n_fields; S.stride = NN;
+    S.opd = full.opd; S.mask = full.mask; S.stats = d_stats;
+    if ((rc = psf_enqueue(ctx, S, d_ys, opts->ys_per_field, ny, d_xs, nx, req, d_psf, d_strehl, d_peak, d_status, st)))
+        return rc;
+    if (stats) CK(cudaMemcpyAsync(stats, d_stats, sizeof(ort_stats) * nf, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(psf, d_psf, sizeof(double) * nf * npix, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(strehl, d_strehl, sizeof(double) * nf * 2, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(peak, d_peak, sizeof(int32_t) * nf, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(status, d_status, sizeof(int32_t) * nf, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return ORT_OK;
+}
+
 // ------------------------------------------------------------------------------------------
 // arbitrary rays / 2-D / paraxial / transfer / candidates: host wrappers stage through scratch
 // ------------------------------------------------------------------------------------------

@@ -15,6 +15,8 @@ enum Slot {
     SL_GATHER, SL_MERGED, SL_AIM, SL_TABLE, SL_CLIST,                                  // communicator: gathered records, merged records, prelude records, merit table
     SL_EN_STATE, SL_EN_HIST, SL_EN_BINS, SL_EN_CAND0, SL_EN_CAND1, SL_EN_COUNTS, SL_EN_RADIUS,   // encircled energy
     SL_ZN_GPART, SL_ZN_RPART, SL_ZN_CSYM, SL_ZN_COEF, SL_ZN_RESID, SL_ZN_STATUS,              // Zernike fit
+    SL_PSF_CTAB, SL_PSF_T, SL_PSF_RSUM, SL_PSF_E, SL_PSF_BVAL, SL_PSF_BIDX,                  // diffraction PSF: work
+    SL_PSF_OUT, SL_PSF_STREHL, SL_PSF_PEAK, SL_PSF_STATUS,                                  // ... and the host form's results
     SL_COUNT
 };
 

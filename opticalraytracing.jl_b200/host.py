@@ -1040,6 +1040,84 @@ def zernike(surfaces, system, Hs, n_max=8, k_rays=SPOT_RAYS, focus=None, lam=LAM
     return out
 
 
+@dataclass
+class PSF:
+    """EXTENSION (no reference type): diffraction point-spread function of one field point -- the scalar Fraunhofer PSF of
+    the mirrored pupil that wavefront() returns, pupil height h mapped to the image-space direction sine h / f
+    (include/ort_b200.h, ort_wavefront_psf_dev).  u, v: pixel centres in mm from the chief ray's image point, u along x
+    (sagittal), v along y; psf[iv, iu], 1 = the diffraction-limited peak of the same (possibly vignetted) pupil.
+    strehl: psf at the chief ray's image point, |mean(exp(2 pi i W))|^2; peak: the maximum of psf over the grid, at
+    peak_uv.  status 0 ok, 1 no kept ray, 3 a non-finite OPD (psf, strehl and peak NaN for status != 0)."""
+    H: float
+    u: np.ndarray
+    v: np.ndarray
+    psf: np.ndarray
+    strehl: float
+    peak: float
+    peak_uv: tuple
+    status: int
+    n_kept: int
+    stats: np.ndarray = field(repr=False)
+
+
+def _pair(x, name, kind):
+    t = tuple(x) if isinstance(x, (tuple, list, np.ndarray)) else (x, x)
+    if len(t) != 2:
+        raise ValueError(f"psf: {name} is one value or a pair (along x, along y)")
+    return tuple(kind(a) for a in t)
+
+
+def psf(surfaces, system, Hs, n_pix=None, pixel=None, k_rays=SPOT_RAYS, focus=None, lam=LAMBDA, vignette=False,
+        backend=None, arith=_lib.FAST):
+    """EXTENSION: diffraction PSF and Strehl ratio of every field point of Hs -> list of PSF.  The OPD sweep of
+    wavefront() runs full grid on the device and the PSF is computed there (ort_trace3d_psf): a matrix Fourier transform
+    of exp(2 pi i W) over the traced pupil grid with s = 1 / (lam f).  Only the pixel grid crosses PCIe.
+    n_pix: pixels per side, an int or (n_u, n_v), default k_rays - 1 (odd: the chief ray's image point is a pixel);
+    pixel: pitch in mm, a value or (du, dv), default lam F# / 2 = 1 / (4 s y_EP).  Raises ValueError when the pixel grid
+    is longer than the alias period 1 / (s dx) or 1 / (s dy) of the pupil grid."""
+    if not (isinstance(k_rays, (int, np.integer)) and k_rays >= 2):
+        raise ValueError("psf: k_rays must be an integer >= 2")
+    n_u, n_v = _pair(k_rays - 1 if n_pix is None else n_pix, "n_pix", int)
+    if not (1 <= n_u <= _lib.PSF_MAX_SIDE and 1 <= n_v <= _lib.PSF_MAX_SIDE):
+        raise ValueError(f"psf: n_pix must lie in [1, {_lib.PSF_MAX_SIDE}]")
+    if pixel is not None:
+        du, dv = _pair(pixel, "pixel", float)
+        if not (math.isfinite(du) and math.isfinite(dv) and du > 0 and dv > 0):
+            raise ValueError("psf: pixel must be finite and > 0")
+    be = _be(backend)
+    p, xs, ys, flds, ext = _wavefront_setup(surfaces, system, Hs, k_rays, focus, vignette, backend, "psf")
+    try:
+        scale = 1.0 / (lam * system.f)
+        if not (math.isfinite(scale) and scale > 0):
+            raise ValueError("psf: 1 / (lam f) must be finite and > 0")
+        if pixel is None:
+            du = dv = 1.0 / (4.0 * scale * p["y_EP"])
+        # the grid must not wrap: n du <= 1 / (s dx), the alias period of the pupil step dx (1e-9: equality is allowed)
+        dx = abs(xs[1] - xs[0]) if len(xs) > 1 else 0.0
+        dy = float(np.max(np.abs(ys[:, 1] - ys[:, 0]))) if ys.shape[1] > 1 else 0.0
+        if n_u * du * scale * dx > 1 + 1e-9 or n_v * dv * scale * dy > 1 + 1e-9:
+            span = float(np.max(np.abs(ys[:, -1] - ys[:, 0])))
+            k_fit = max(2 * (math.ceil(n_u * du * scale * p["y_EP"]) + 1), math.ceil(n_v * dv * scale * span) + 1)
+            raise ValueError(f"psf: {n_u} x {n_v} pixels of {du:.4g} x {dv:.4g} mm exceed the alias period "
+                             f"{1 / (scale * dx) if dx else math.inf:.4g} x {1 / (scale * dy) if dy else math.inf:.4g} mm "
+                             f"of k_rays = {k_rays}; k_rays >= {k_fit + (k_fit & 1)} would fit")
+        u, v = (np.arange(n_u) - (n_u - 1) / 2) * du, (np.arange(n_v) - (n_v - 1) / 2) * dv
+        out = []
+        for j0 in range(0, len(flds), _lib.MAX_FIELDS):
+            sl = slice(j0, j0 + _lib.MAX_FIELDS)
+            r = be.trace3d_psf(flds[sl], ys[sl], xs, p["stop"], p["a_stop"], n_u, n_v, du, dv, scale, arith=arith,
+                               ext=ext, opd_scale=-1.0 / lam)
+            for j, H in enumerate(p["Hs"][sl]):
+                pk = int(r["peak"][j])
+                uv = (float(u[pk % n_u]), float(v[pk // n_u])) if pk >= 0 else (math.nan, math.nan)
+                out.append(PSF(float(H), u.copy(), v.copy(), r["psf"][j].copy(), float(r["strehl"][j][0]),
+                               float(r["strehl"][j][1]), uv, int(r["status"][j]), int(r["stats"][j]["n_kept"]),
+                               r["stats"][j:j + 1].copy()))
+    finally:
+        be.set_apertures(None)
+    return out
+
+
 # ------------------------------------------------------------------------------------------------
 # Seidel aberrations (SURVEY.md section 8 f2): the per-candidate objective of the reference's optimize()
 # ------------------------------------------------------------------------------------------------
