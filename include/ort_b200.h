@@ -42,8 +42,9 @@ extern "C" {
 #define ORT_VERSION 200 /* 0.2.0: communicator inside the library, ort_opts.gather_stats, ort_grid_out.stats_local;
                            ort_trace3d_focus / ort_trace3d_focus_dev (through-focus sweep) and ort_spot_energy_dev /
                            ort_trace3d_energy (encircled energy), ort_wavefront_zernike_dev / ort_trace3d_zernike
-                           (Zernike fit of the wavefront) and ort_wavefront_psf_dev / ort_trace3d_psf (diffraction PSF)
-                           added without a version change */
+                           (Zernike fit of the wavefront), ort_wavefront_psf_dev / ort_trace3d_psf (diffraction PSF)
+                           and ort_wavefront_mtf_dev / ort_trace3d_mtf (diffraction MTF) added without a version
+                           change */
 
 /* status codes */
 #define ORT_OK            0
@@ -395,6 +396,60 @@ int ort_wavefront_psf_dev(ort_ctx *ctx, const ort_wave_sets *sets /* host struct
 int ort_trace3d_psf(ort_ctx *ctx, const ort_field *fields, int n_fields, const double *ys, int ny, const double *xs, int nx,
                     int stop, double a_stop, const ort_opts *opts, const ort_psf_req *req, ort_stats *stats, double *psf,
                     double *strehl, int32_t *peak, int32_t *status);
+
+/* ---- EXTENSION (no reference method): diffraction modulation transfer function of the ray-traced wavefront, computed on
+ *      the device from the outputs of a grid sweep with ORT_EXT_OPD in full-grid form (opts.compact = 0): the optical
+ *      transfer function of the PSF that ort_wavefront_psf_dev defines (same sets, same scale s, same mirrored pupil),
+ *      along two azimuths.
+ *      A SET is as for the PSF: W_i = opd (waves when the Python host sweeps with opd_scale = -1/lambda), P[iy][ix] =
+ *        exp(2 pi i W) for kept rays (mask == 1) and 0 otherwise, n = stats[s].n_kept.
+ *      The pupil must be a MIRRORED LATTICE, defined by index, not by value: xs[0] == 0, dx = xs[nx-1]/(nx-1) finite and
+ *        > 0, dy_s = (ys_s[ny-1] - ys_s[0])/(ny-1) finite and != 0 (the host's ys run downwards from y1 > y2: dy_s < 0).
+ *        The host's grids (xs = range(0, y_EP, k/2), ys = range(y1, y2, k)) have this form to within an ulp per element.
+ *      Mirrored amplitude, jx in [-(nx-1), nx-1]: A[iy][jx] = P[iy][|jx|] for jx != 0, A[iy][0] = 2 P[iy][0].
+ *          C_sag(k) = sum_iy sum_jx A[iy][jx+k] conj A[iy][jx]        k = 0 .. 2(nx-1)   (real: the mirror)
+ *          C_tan(k) = sum_jx sum_iy A[iy+k][jx] conj A[iy][jx]        k = 0 .. ny-1
+ *                   = sum_ix w_ix sum_iy P[iy+k][ix] conj P[iy][ix],  w_0 = 4, w_ix = 2 otherwise
+ *          OTF(k)   = C(k) / C(0)     (C(0) = 2n + 2n0 for both, n0 = kept rays in the x = 0 column; OTF(0) = 1 exactly)
+ *        i.e. OTF(nu) = int psf exp(-2 pi i nu . (xi, eta)) / int psf of that PSF: sagittal = nu along xi (x) at
+ *        nu = k s dx, tangential = nu along eta (y) at nu = k s |dy_s|.  For dy_s < 0 a frequency nu > 0 pairs rows iy + k
+ *        with iy the other way round, and the tangential OTF is conj C_tan(k) / C(0).
+ *      Requested frequencies req.freqs[0 .. n_freq), cycles per image unit, finite and >= 0, in any order.  Per azimuth,
+ *        q = nu / (s d) with d = dx or |dy_s|, k0 = floor(q), f = q - k0:
+ *          OTF(nu) = (1 - f) OTF(k0) + f OTF(k0 + 1),   OTF(k) = 0 past the last lag.
+ *        The diffraction cutoffs of the sampled pupil are 2 (nx-1) dx s (= 2 y_EP s = 1/(lambda F#) on the host's grids)
+ *        and (ny-1) |dy_s| s.
+ *      Outputs per set s:
+ *        otf[s][2][n_freq][2]  [0] sagittal, [1] tangential; (re, im).  The sagittal imaginary part is exactly 0.
+ *        status[s]             0 ok; 1 n = 0; 3 a kept ray has a non-finite opd (the PSF's codes); 4 the grid is not a
+ *                              mirrored lattice (read from d_xs and d_ys).  The lowest code that applies.  For
+ *                              status != 0 otf is NaN.
+ *      Determinism: no floating-point atomics, partial sums folded in a fixed order: bit-identical run to run on one
+ *      device, not bit-equal to numpy. */
+#define ORT_MTF_MAX_FREQS 1024
+typedef struct ort_mtf_req {
+    int32_t n_freq, reserved;       /* 1 .. ORT_MTF_MAX_FREQS */
+    const double *freqs;            /* host array [n_freq] */
+    double  scale;                  /* s, as ort_psf_req.scale: finite and > 0 */
+} ort_mtf_req;                      /* 24 bytes */
+/* Device form (enqueue only on `stream`): the sets already in HBM in full-grid form (sets->mask required; r and theta are
+ * not read), d_ys [ys_per_set ? n_sets : 1][ny] and d_xs [nx] the grid coordinates on the device.  d_otf
+ * [n_sets][2][n_freq][2], d_status [n_sets].  ORT_EINVAL before anything is enqueued for: a NULL array, stride != ny*nx,
+ * stride >= 2^31, nx < 2 or ny < 2, n_sets outside [1, ORT_MAX_FIELDS], n_freq outside [1, ORT_MTF_MAX_FREQS], a frequency negative or
+ * not finite, scale not finite or <= 0.  Launches four kernels whatever the sizes.  Scratch: the pupil amplitude, once
+ * row-major and once transposed, takes 32 n_sets ny nx bytes (2.7 GB for 5 fields of 5792 x 2896 rays, four times the
+ * OPD input); the lag partials take 24 n_sets (2 n_freq + 1) g bytes with g <= a few thousand row groups.  A scratch
+ * that cannot grow is ORT_ENOMEM. */
+int ort_wavefront_mtf_dev(ort_ctx *ctx, const ort_wave_sets *sets /* host struct */, const double *d_ys, int ys_per_set,
+                          int ny, const double *d_xs, int nx, const ort_mtf_req *req, double *d_otf, int32_t *d_status,
+                          void *stream);
+/* Host form: the grid sweep of the layout (polynomial terms and vignetting accepted as by ort_trace3d_grid) full grid
+ * into the context's scratch with opd, mask and stats, then the MTF on it; only stats [n_fields] (may be NULL),
+ * otf [n_fields][2][n_freq][2] and status [n_fields] cross PCIe.  opts.ext must hold ORT_EXT_OPD and opts.compact must
+ * be 0 (ORT_EINVAL); opts.gather_stats is ORT_EUNSUPPORTED. */
+int ort_trace3d_mtf(ort_ctx *ctx, const ort_field *fields, int n_fields, const double *ys, int ny, const double *xs, int nx,
+                    int stop, double a_stop, const ort_opts *opts, const ort_mtf_req *req, ort_stats *stats, double *otf,
+                    int32_t *status);
 
 /* ---- 3-D skew trace of N arbitrary rays, all surfaces recorded: replaces
  *      raytrace(surfaces, y, x, U, V, Vector{RealRay}) src/PupilSampling.jl:34-65 for a batch.

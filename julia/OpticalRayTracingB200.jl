@@ -446,6 +446,46 @@ function psf(::B200, surfaces::Layout, system::System, H::Float64; n_pix = nothi
             status = Int(status[1]), n_kept = stats[1].n_kept)
 end
 
+# --- Diffraction MTF of the wavefront (EXTENSION, no reference method) -------------------------------------------------
+# The OPD sweep of psf, then ONE ccall (ort_trace3d_mtf) that sweeps the pupil grid with ORT_EXT_OPD on the device and
+# computes there the optical transfer function of the PSF that psf describes (s = 1/(λ f)): the normalised
+# autocorrelation of the mirrored pupil exp(2πi W), sagittal (frequency along x) and tangential (along y), interpolated
+# linearly between lattice lags.  freqs in cycles/mm, default 32 from 0 to 1/(λ F#) = 2 s y_EP; otf is 2 × n_freq
+# (row 1 sagittal, row 2 tangential), mtf = abs.(otf), ptf = angle.(otf).  Only the OTF values cross PCIe.  Not runnable
+# here (no Julia); the Python host's mtf is the tested form of the same calls.
+struct OrtMtfReq
+    n_freq::Int32; reserved::Int32; freqs::Ptr{Float64}; scale::Float64
+end
+
+function mtf(::B200, surfaces::Layout, system::System, H::Float64; freqs = nothing, k_rays::Int = spot_rays,
+             focus = nothing, λ = 587.5618e-6, vignette::Bool = false, arith = ORT_ARITH_FAST)
+    require_conic(surfaces)
+    k_rays ≥ 4 || throw(DomainError(k_rays, "k_rays ≥ 4"))
+    s = 1.0 / (λ * system.f)
+    field, ys, xs, stop, a_stop, y_EP = opd_sweep_setup(surfaces, system, H, k_rays, focus, vignette)
+    f = freqs === nothing ? collect(range(0.0, 2 * s * y_EP, length = 32)) : Vector{Float64}(freqs)
+    if !(1 ≤ length(f) ≤ 1024 && all(x -> isfinite(x) && x ≥ 0, f))
+        check(ccall((:ort_set_apertures, LIB), Cint, (Ptr{Cvoid}, Cint, Ptr{Float64}), ctx(), 0, C_NULL))
+        throw(DomainError(freqs, "1 to 1024 frequencies, finite and ≥ 0"))
+    end
+    stats = [OrtStats(0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0, 0)]
+    otf = zeros(2, length(f), 2); status = zeros(Int32, 1)          # otf[ri, j, a] is C otf[a][j][ri] ([az][f][2])
+    opts = Ref(OrtOpts(arith, 0, 0, ORT_EXT_OPD | (vignette ? ORT_EXT_VIGNETTE : Int32(0)), 0.0, 1.0, -1.0 / λ, 0, 0))
+    GC.@preserve f begin
+        req = Ref(OrtMtfReq(length(f), 0, pointer(f), s))
+        check(ccall((:ort_trace3d_mtf, LIB), Cint,
+                    (Ptr{Cvoid}, Ref{OrtField}, Cint, Ptr{Float64}, Cint, Ptr{Float64}, Cint, Cint, Float64, Ref{OrtOpts},
+                     Ref{OrtMtfReq}, Ptr{OrtStats}, Ptr{Float64}, Ptr{Int32}),
+                    ctx(), Ref(field), 1, ys, length(ys), xs, length(xs), stop, a_stop, opts, req, stats, otf, status))
+    end
+    check(ccall((:ort_set_apertures, LIB), Cint, (Ptr{Cvoid}, Cint, Ptr{Float64}), ctx(), 0, C_NULL))
+    o = [complex(otf[1, j, a], otf[2, j, a]) for a in 1:2, j in 1:length(f)]
+    nx, ny = length(xs), length(ys)
+    cutoff = (2 * (nx - 1) * (xs[end] / (nx - 1)) * s, (ny - 1) * abs((ys[end] - ys[1]) / (ny - 1)) * s)
+    return (freqs = f, otf = o, mtf = abs.(o), ptf = angle.(o), cutoff = cutoff, status = Int(status[1]),
+            n_kept = stats[1].n_kept)
+end
+
 # --- batched 2-D meridional real rays: src/RayTracing.jl:145-173 ------------------------------
 # Returns (y, U, ts), each rows × N, for N rays in one kernel launch.
 function raytrace(surfaces::Layout{T}, ys::Vector{Float64}, Us::Vector{Float64}, ::Type{RealRay}) where T

@@ -24,6 +24,7 @@ ENERGY_CIRCLE, ENERGY_SQUARE = 0, 1
 CENTER_CENTROID, CENTER_PARAXIAL = 0, 1
 ZERN_MAX_ORDER = 12
 PSF_MAX_SIDE = 1024
+MTF_MAX_FREQS = 1024
 
 # every symbol include/ort_b200.h declares (tests check the .so exports exactly these)
 SYMBOLS = [
@@ -32,7 +33,7 @@ SYMBOLS = [
     "ort_set_layout", "ort_set_apertures", "ort_set_polynomials",
     "ort_trace3d_grid", "ort_trace3d_grid_dev", "ort_trace3d_focus", "ort_trace3d_focus_dev",
     "ort_spot_energy_dev", "ort_trace3d_energy", "ort_wavefront_zernike_dev", "ort_trace3d_zernike",
-    "ort_wavefront_psf_dev", "ort_trace3d_psf",
+    "ort_wavefront_psf_dev", "ort_trace3d_psf", "ort_wavefront_mtf_dev", "ort_trace3d_mtf",
     "ort_trace3d_rays", "ort_trace3d_rays_opl", "ort_trace3d_rays_dev", "ort_trace2d_batch", "ort_aim2d",
     "ort_paraxial_batch", "ort_paraxial_batch_dev", "ort_transfer_batch", "ort_transfer_batch_dev",
     "ort_trace3d_candidates", "ort_trace3d_candidates_dev", "ort_aim_candidates", "ort_aim_candidates_dev", "ort_aim_fields",
@@ -120,6 +121,17 @@ class PsfReq(C.Structure):
     _fields_ = [("n_u", C.c_int32), ("n_v", C.c_int32), ("du", C.c_double), ("dv", C.c_double), ("scale", C.c_double)]
 
 
+class MtfReq(C.Structure):
+    _fields_ = [("n_freq", C.c_int32), ("reserved", C.c_int32), ("freqs", C.POINTER(C.c_double)),
+                ("scale", C.c_double)]
+
+
+def mtf_req(freqs, scale):
+    """-> (MtfReq, the float64 array it points into: keep it alive while the request is used)"""
+    f = np.ascontiguousarray(np.asarray(freqs, dtype=np.float64).ravel())
+    return MtfReq(len(f), 0, f.ctypes.data_as(C.POINTER(C.c_double)), float(scale)), f
+
+
 def zernike_terms(n_max):
     """J = (n_max + 1)(n_max + 2) / 2 coefficients per set, in ANSI order"""
     return (int(n_max) + 1) * (int(n_max) + 2) // 2
@@ -177,6 +189,9 @@ def load():
     L.ort_wavefront_psf_dev.argtypes = [C.c_void_p, C.POINTER(WaveSets), C.c_void_p, C.c_int, C.c_int, C.c_void_p,
                                         C.c_int, C.POINTER(PsfReq)] + [C.c_void_p] * 5
     L.ort_trace3d_psf.argtypes = grid_args[:9] + [C.POINTER(Opts), C.POINTER(PsfReq)] + [C.c_void_p] * 5
+    L.ort_wavefront_mtf_dev.argtypes = [C.c_void_p, C.POINTER(WaveSets), C.c_void_p, C.c_int, C.c_int, C.c_void_p,
+                                        C.c_int, C.POINTER(MtfReq)] + [C.c_void_p] * 3
+    L.ort_trace3d_mtf.argtypes = grid_args[:9] + [C.POINTER(Opts), C.POINTER(MtfReq)] + [C.c_void_p] * 3
     L.ort_trace3d_rays.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p]
     L.ort_trace3d_rays_opl.argtypes = [C.c_void_p, C.c_int64, _dp, _dp, _dp, _dp, C.c_int, _dp, _dp, _dp, _u8p, _dp]
     L.ort_trace3d_rays_dev.argtypes = [C.c_void_p, C.c_int64] + [C.c_void_p] * 4 + [C.c_int] + [C.c_void_p] * 6
@@ -699,6 +714,38 @@ class Context:
                                         float(a_stop), C.byref(op), C.byref(req), stats.ctypes.data, psf.ctypes.data,
                                         strehl.ctypes.data, peak.ctypes.data, status.ctypes.data))
         return dict(stats=stats, psf=psf, strehl=strehl, peak=peak, status=status)
+
+    # ---- diffraction MTF of the wavefront ---------------------------------------------------
+    def wavefront_mtf_dev(self, sets, d_ys, ys_per_set, ny, d_xs, nx, freqs, scale, d_otf=0, d_status=0, stream=0):
+        """Diffraction OTF of full-grid wavefront sets already in HBM (ort_wavefront_mtf_dev, enqueue only).  sets: dict with
+        n_sets, stride = ny * nx and the device addresses opd, mask, stats (r and theta are not read); d_ys
+        [ys_per_set ? n_sets : 1][ny], d_xs [nx] device addresses; freqs: host array, cycles per image unit.  d_otf:
+        float64 [n_sets][2][n_freq][2] (sagittal, tangential; re, im), d_status: int32 [n_sets] (device addresses)."""
+        ws = WaveSets(*[sets.get(k) or 0 for k in WAVE_SETS_NAMES])
+        req, keep = mtf_req(freqs, scale)
+        self._ck(self.L.ort_wavefront_mtf_dev(self.h, C.byref(ws), C.c_void_p(d_ys or 0), int(ys_per_set), int(ny),
+                                              C.c_void_p(d_xs or 0), int(nx), C.byref(req), C.c_void_p(d_otf or 0),
+                                              C.c_void_p(d_status or 0), C.c_void_p(stream)))
+        del keep
+
+    def trace3d_mtf(self, fields, ys, xs, stop, a_stop, freqs, scale, arith=FAST, ext=EXT_OPD, opd_scale=1.0):
+        """The grid sweep with ORT_EXT_OPD full grid on the device and the diffraction OTF of every field on it
+        (ort_trace3d_mtf); no ray crosses PCIe.  Returns dict(stats (n_fields,), otf (n_fields, 2, n_freq) complex128
+        (sagittal, tangential), status (n_fields,) int32)."""
+        farr, nf = make_fields(fields)
+        ys, xs = _d(ys), _d(xs)
+        per_field = ys.ndim == 2
+        if per_field and ys.shape[0] != nf:
+            raise ValueError("ys must be (ny,) or (n_fields, ny)")
+        req, keep = mtf_req(freqs, scale)
+        stats = np.zeros(nf, dtype=STATS_DTYPE)
+        otf = np.zeros((nf, 2, len(keep), 2), dtype=np.float64)
+        status = np.zeros(nf, dtype=np.int32)
+        op = _opts(arith, False, per_field, ext, opd_scale=opd_scale)
+        self._ck(self.L.ort_trace3d_mtf(self.h, farr, nf, _vp(ys), ys.shape[-1], _vp(xs), len(xs), int(stop),
+                                        float(a_stop), C.byref(op), C.byref(req), stats.ctypes.data, otf.ctypes.data,
+                                        status.ctypes.data))
+        return dict(stats=stats, otf=otf[..., 0] + 1j * otf[..., 1], status=status)
 
     # ---- arbitrary rays ------------------------------------------------------------------
     def trace3d_rays(self, y0, x0, u0, v0, arith=STRICT, opl=False):

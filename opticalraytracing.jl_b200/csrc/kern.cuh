@@ -104,6 +104,30 @@ struct PsfArgs {
     int *peak, *status;                         // [n_sets]
 };
 
+// Diffraction MTF of the wavefront (kern_mtf.cu)
+struct MtfArgs {
+    int n_sets, ny, nx;
+    long long stride;
+    const double* opd; const uint8_t* mask; const ort_stats* stats;
+    const double *ys, *xs;                      // ys + s * ys_stride: the iy coordinates of set s
+    long long ys_stride;                        // 0 or ny
+    int n_freq;
+    double scale;
+    int n_slot;                                 // lag slots per azimuth, 2 n_freq + 1: k0 and k0 + 1 of each frequency, 0
+    int lb, nlb;                                // lag slots per block of k_mtf_sag / k_mtf_tan, blocks
+    int tiles_x, tiles;                         // k_mtf_pupil 32 x 32 tiles along x, per set
+    int rg_s, rl_s;                             // k_mtf_sag row groups per set, rows per group
+    int rg_t, rl_t;                             // k_mtf_tan column groups per set, columns per group
+    double2* P;                                 // [n_sets][ny][nx]: mask exp(2 pi i W), column 0 doubled
+    double2* PT;                                // [n_sets][nx][ny]: its transpose
+    uint8_t* bad;                               // [n_sets][tiles]: 1 if a kept opd of the tile is not finite
+    double* psag;                               // [n_sets][rg_s][n_slot]: sagittal lag sums per row group
+    double2* ptan;                              // [n_sets][rg_t][n_slot]: tangential lag sums per column group
+    double* otf;                                // [n_sets][2][n_freq][2]
+    int* status;                                // [n_sets]
+    double freqs[ORT_MTF_MAX_FREQS];            // cycles per image unit
+};
+
 struct CompactArgs {
     unsigned NN;
     const uint8_t* mask;
@@ -270,6 +294,12 @@ cudaError_t launch_zernike(const ZernArgs& A, cudaStream_t st, int* launches);
 // launch_psf enqueues the five kernels
 cudaError_t psf_dims(PsfArgs& A, int sm_count);
 cudaError_t launch_psf(const PsfArgs& A, cudaStream_t st, int* launches);
+// diffraction MTF: mtf_occupancy sets the kernels' shared-memory limit and returns the resident CTAs/SM of the lag
+// kernels [sagittal, tangential][global, staged] (once per context); mtf_dims fills n_slot .. rl_t from n_sets, ny, nx
+// and n_freq (the scratch sizes follow from them); launch_mtf enqueues the four kernels
+cudaError_t mtf_occupancy(int (&occ)[2][2]);
+cudaError_t mtf_dims(MtfArgs& A, int sm_count, const int (&occ)[2][2]);
+cudaError_t launch_mtf(const MtfArgs& A, cudaStream_t st, int* launches);
 cudaError_t launch_rays(const Presc& P, const RaysArgs& A, int arith, cudaStream_t st);
 cudaError_t launch_candidates(const CandArgs& A, int arith, cudaStream_t st, int sm_count);
 cudaError_t launch_trace2d(const Presc& P, const Trace2dArgs& A, cudaStream_t st);

@@ -1118,6 +1118,129 @@ int ort_trace3d_psf(ort_ctx* ctx, const ort_field* fields, int n_fields, const d
     return ORT_OK;
 }
 
+}  // extern "C"
+
+// ------------------------------------------------------------------------------------------
+// Diffraction MTF of the wavefront (kern_mtf.cu)
+// ------------------------------------------------------------------------------------------
+static int mtf_req_check(ort_ctx* ctx, const ort_mtf_req* req, const void* otf, const void* status)
+{
+    if (!req) return fail(ctx, ORT_EINVAL, "mtf: req is NULL");
+    if (req->n_freq < 1 || req->n_freq > ORT_MTF_MAX_FREQS)
+        return fail(ctx, ORT_EINVAL, "mtf: n_freq = %d not in [1, %d]", req->n_freq, ORT_MTF_MAX_FREQS);
+    if (!req->freqs) return fail(ctx, ORT_EINVAL, "mtf: freqs is NULL");
+    for (int i = 0; i < req->n_freq; i++)
+        if (!(isfinite(req->freqs[i]) && req->freqs[i] >= 0.0))
+            return fail(ctx, ORT_EINVAL, "mtf: freqs[%d] = %g must be finite and >= 0", i, req->freqs[i]);
+    if (!(isfinite(req->scale) && req->scale > 0.0))
+        return fail(ctx, ORT_EINVAL, "mtf: scale = %g must be finite and > 0", req->scale);
+    if (!otf || !status) return fail(ctx, ORT_EINVAL, "mtf: otf or status is NULL");
+    return ORT_OK;
+}
+
+// Enqueue the four MTF kernels over `sets` on st (inside the entry point's ScratchScope); one ProfScope around them
+static int mtf_enqueue(ort_ctx* ctx, const ort_wave_sets& S, const double* d_ys, int ys_per_set, int ny,
+                       const double* d_xs, int nx, const ort_mtf_req* req, double* d_otf, int32_t* d_status,
+                       cudaStream_t st)
+{
+    MtfArgs A;
+    memset(&A, 0, sizeof A);
+    A.n_sets = S.n_sets; A.ny = ny; A.nx = nx; A.stride = S.stride;
+    A.opd = S.opd; A.mask = S.mask; A.stats = S.stats;
+    A.ys = d_ys; A.ys_stride = ys_per_set ? ny : 0; A.xs = d_xs;
+    A.n_freq = req->n_freq; A.scale = req->scale;
+    memcpy(A.freqs, req->freqs, sizeof(double) * (size_t)req->n_freq);
+    if (ctx->mtf_occ[0][0] == 0) CK(mtf_occupancy(ctx->mtf_occ));
+    CK(mtf_dims(A, ctx->sm_count, ctx->mtf_occ));
+    const size_t ns = (size_t)S.n_sets;
+    ENSURE(SL_MTF_P, sizeof(double2) * ns * (size_t)S.stride, A.P);
+    ENSURE(SL_MTF_PT, sizeof(double2) * ns * (size_t)S.stride, A.PT);
+    ENSURE(SL_MTF_BAD, sizeof(uint8_t) * ns * (size_t)A.tiles, A.bad);
+    ENSURE(SL_MTF_PSAG, sizeof(double) * ns * A.rg_s * A.n_slot, A.psag);
+    ENSURE(SL_MTF_PTAN, sizeof(double2) * ns * A.rg_t * A.n_slot, A.ptan);
+    A.otf = d_otf; A.status = (int*)d_status;
+    int n = 0;
+    {
+        ProfScope prof(ctx, st);
+        CK(launch_mtf(A, st, &n));
+    }
+    ctx->launches += n;
+    return ORT_OK;
+}
+
+extern "C" {
+
+int ort_wavefront_mtf_dev(ort_ctx* ctx, const ort_wave_sets* sets, const double* d_ys, int ys_per_set, int ny,
+                          const double* d_xs, int nx, const ort_mtf_req* req, double* d_otf, int32_t* d_status,
+                          void* stream)
+{
+    if (!ctx) return ORT_EINVAL;
+    if (!sets) return fail(ctx, ORT_EINVAL, "wavefront_mtf: sets is NULL");
+    if (sets->n_sets < 1 || sets->n_sets > ORT_MAX_FIELDS)
+        return fail(ctx, ORT_EINVAL, "wavefront_mtf: n_sets = %d not in [1, %d]", sets->n_sets, ORT_MAX_FIELDS);
+    if (ny < 2 || nx < 2 || sets->stride != (long long)ny * nx || sets->stride >= (1LL << 31))
+        return fail(ctx, ORT_EINVAL, "wavefront_mtf: stride = %lld is not ny*nx = %d*%d with ny, nx >= 2 (< 2^31)",
+                    (long long)sets->stride, ny, nx);
+    if (!sets->opd || !sets->mask || !sets->stats || !d_ys || !d_xs)
+        return fail(ctx, ORT_EINVAL, "wavefront_mtf: opd, mask, stats, ys or xs is NULL");
+    int rc = mtf_req_check(ctx, req, d_otf, d_status);
+    if (rc) return rc;
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = (cudaStream_t)stream;
+    ScratchScope scratch(ctx, st);
+    return mtf_enqueue(ctx, *sets, d_ys, ys_per_set, ny, d_xs, nx, req, d_otf, d_status, st);
+}
+
+int ort_trace3d_mtf(ort_ctx* ctx, const ort_field* fields, int n_fields, const double* ys, int ny, const double* xs, int nx,
+                    int stop, double a_stop, const ort_opts* opts, const ort_mtf_req* req, ort_stats* stats, double* otf,
+                    int32_t* status)
+{
+    if (!ctx) return ORT_EINVAL;
+    if (!opts) return fail(ctx, ORT_EINVAL, "trace3d_mtf: opts is NULL");
+    if (opts->gather_stats) return fail(ctx, ORT_EUNSUPPORTED, "trace3d_mtf: opts.gather_stats is not supported");
+    if (opts->compact) return fail(ctx, ORT_EINVAL, "trace3d_mtf: opts.compact must be 0");
+    if (!(opts->ext & ORT_EXT_OPD)) return fail(ctx, ORT_EINVAL, "trace3d_mtf: opts.ext must hold ORT_EXT_OPD");
+    // the members the MTF reads; ort_sweep_scratch traces each one a host call wants into its scratch slot
+    static double tag; static uint8_t mtag;
+    ort_grid_out want;
+    memset(&want, 0, sizeof want);
+    want.opd = &tag; want.mask = &mtag;
+    int rc = grid_check(ctx, fields, n_fields, ys, ny, xs, nx, stop, opts, &want);
+    if (rc || (rc = mtf_req_check(ctx, req, otf, status))) return rc;
+    if (ny < 2 || nx < 2) return fail(ctx, ORT_EINVAL, "trace3d_mtf: ny = %d, nx = %d must be >= 2", ny, nx);
+    CK(cudaSetDevice(ctx->device));
+    cudaStream_t st = ctx->stream;
+    ScratchScope scratch(ctx, st);
+    const unsigned NN = (unsigned)((long long)ny * nx);
+    const size_t nf = (size_t)n_fields, nout = 4 * (size_t)req->n_freq;
+    const int gx = grid_dims(ctx, ctx->bps, ort_grid_waves(), opts, n_fields, NN);
+    const size_t nys = (size_t)ny * (opts->ys_per_field ? n_fields : 1);
+    double *d_ys, *d_xs;
+    ENSURE(SL_YS, sizeof(double) * nys, d_ys);
+    ENSURE(SL_XS, sizeof(double) * (size_t)nx, d_xs);
+    RawPart* d_partials; ENSURE(SL_PARTIALS, sizeof(RawPart) * (size_t)gx * nf, d_partials);
+    ort_stats* d_stats; ENSURE(SL_STATS, sizeof(ort_stats) * nf, d_stats);
+    double* d_otf; ENSURE(SL_MTF_OTF, sizeof(double) * nf * nout, d_otf);
+    int32_t* d_status; ENSURE(SL_MTF_STATUS, sizeof(int32_t) * nf, d_status);
+    ort_grid_out full, comp; int* d_tiles;
+    if ((rc = ort_sweep_scratch(ctx, &want, opts, false, NN, n_fields, 1, &full, &comp, &d_tiles))) return rc;
+    CK(cudaMemcpyAsync(d_ys, ys, sizeof(double) * nys, cudaMemcpyHostToDevice, st));
+    CK(cudaMemcpyAsync(d_xs, xs, sizeof(double) * (size_t)nx, cudaMemcpyHostToDevice, st));
+    rc = grid_enqueue(ctx, fields, n_fields, d_ys, ny, d_xs, nx, stop, a_stop, nullptr, 1, opts, full, nullptr, d_stats,
+                      d_partials, nullptr, gx, st);
+    if (rc) return rc;
+    ort_wave_sets S;
+    memset(&S, 0, sizeof S);
+    S.n_sets = n_fields; S.stride = NN;
+    S.opd = full.opd; S.mask = full.mask; S.stats = d_stats;
+    if ((rc = mtf_enqueue(ctx, S, d_ys, opts->ys_per_field, ny, d_xs, nx, req, d_otf, d_status, st))) return rc;
+    if (stats) CK(cudaMemcpyAsync(stats, d_stats, sizeof(ort_stats) * nf, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(otf, d_otf, sizeof(double) * nf * nout, cudaMemcpyDeviceToHost, st));
+    CK(cudaMemcpyAsync(status, d_status, sizeof(int32_t) * nf, cudaMemcpyDeviceToHost, st));
+    CK(cudaStreamSynchronize(st));
+    return ORT_OK;
+}
+
 // ------------------------------------------------------------------------------------------
 // arbitrary rays / 2-D / paraxial / transfer / candidates: host wrappers stage through scratch
 // ------------------------------------------------------------------------------------------

@@ -17,6 +17,8 @@ enum Slot {
     SL_ZN_GPART, SL_ZN_RPART, SL_ZN_CSYM, SL_ZN_COEF, SL_ZN_RESID, SL_ZN_STATUS,              // Zernike fit
     SL_PSF_CTAB, SL_PSF_T, SL_PSF_RSUM, SL_PSF_E, SL_PSF_BVAL, SL_PSF_BIDX,                  // diffraction PSF: work
     SL_PSF_OUT, SL_PSF_STREHL, SL_PSF_PEAK, SL_PSF_STATUS,                                  // ... and the host form's results
+    SL_MTF_P, SL_MTF_PT, SL_MTF_BAD, SL_MTF_PSAG, SL_MTF_PTAN,                                // diffraction MTF: work
+    SL_MTF_OTF, SL_MTF_STATUS,                                                               // ... and the host form's results
     SL_COUNT
 };
 
@@ -36,6 +38,7 @@ struct ort_ctx {
     int fast_ok_layout;         // fast_ok as derived from R, t, n, K alone (polynomial terms force it to 0 while set)
     int bps[2][5];              // resident CTAs/SM of k_grid<STRICT|FAST, variant general|EXT|SIMPLE|SIMPLE x EXT|SIMPLE-conic> (grid_variant)
     int bps_focus[2][5];        // the same for k_focus (variants 0, 2, 4; 1 and 3 unused)
+    int mtf_occ[2][2];          // resident CTAs/SM of k_mtf_sag / k_mtf_tan [global, staged]; 0 until the first MTF call
     void* slot[SL_COUNT];
     size_t slot_bytes[SL_COUNT];
     // The scratch slots are shared by every entry point of the context.  Work that uses them is ordered across streams

@@ -1118,6 +1118,66 @@ def psf(surfaces, system, Hs, n_pix=None, pixel=None, k_rays=SPOT_RAYS, focus=No
     return out
 
 
+@dataclass
+class MTF:
+    """EXTENSION (no reference type): diffraction modulation transfer function of one field point -- the optical transfer
+    function of the PSF that psf() computes (scalar Fraunhofer model of the mirrored pupil, s = 1 / (lam f)), along two
+    azimuths (include/ort_b200.h, ort_wavefront_mtf_dev).  freqs in cycles/mm; otf[0] sagittal (frequency along x),
+    otf[1] tangential (along y), complex, otf(0) = 1; mtf = |otf|, ptf = angle(otf) in radians.  cutoff: the diffraction
+    cutoffs (sagittal, tangential) of the sampled pupil, past which otf is 0.  status 0 ok, 1 no kept ray, 3 a non-finite
+    OPD, 4 the pupil grid is not a lattice (otf NaN for status != 0)."""
+    H: float
+    freqs: np.ndarray
+    otf: np.ndarray
+    mtf: np.ndarray
+    ptf: np.ndarray
+    cutoff: tuple
+    status: int
+    n_kept: int
+    stats: np.ndarray = field(repr=False)
+
+
+def mtf(surfaces, system, Hs, freqs=None, k_rays=SPOT_RAYS, focus=None, lam=LAMBDA, vignette=False, backend=None,
+        arith=_lib.FAST):
+    """EXTENSION: diffraction MTF of every field point of Hs -> list of MTF.  The OPD sweep of wavefront() runs full grid
+    on the device and the OTF is computed there (ort_trace3d_mtf) as the autocorrelation of the mirrored pupil function
+    exp(2 pi i W) at the lattice lags the frequencies need, interpolated linearly between them.  Only the OTF values cross
+    PCIe.  freqs: cycles/mm, finite and >= 0, at most MTF_MAX_FREQS; default 32 evenly spaced from 0 to 1 / (lam F#) =
+    2 s y_EP."""
+    if not (isinstance(k_rays, (int, np.integer)) and k_rays >= 4):
+        raise ValueError("mtf: k_rays must be an integer >= 4")
+    if freqs is not None:
+        freqs = np.array(freqs, dtype=np.float64).ravel()
+        if not (1 <= len(freqs) <= _lib.MTF_MAX_FREQS):
+            raise ValueError(f"mtf: 1 to {_lib.MTF_MAX_FREQS} frequencies")
+        if not (np.all(np.isfinite(freqs)) and np.all(freqs >= 0)):
+            raise ValueError("mtf: frequencies must be finite and >= 0")
+    be = _be(backend)
+    p, xs, ys, flds, ext = _wavefront_setup(surfaces, system, Hs, k_rays, focus, vignette, backend, "mtf")
+    try:
+        scale = 1.0 / (lam * system.f)
+        if not (math.isfinite(scale) and scale > 0):
+            raise ValueError("mtf: 1 / (lam f) must be finite and > 0")
+        if freqs is None:
+            freqs = np.linspace(0.0, 2.0 * scale * p["y_EP"], 32)
+        # the lattice steps of the contract, by index: dx = xs[-1] / (nx - 1), dy = (ys[-1] - ys[0]) / (ny - 1)
+        cut_x = 2 * (len(xs) - 1) * (xs[-1] / (len(xs) - 1)) * scale
+        out = []
+        for j0 in range(0, len(flds), _lib.MAX_FIELDS):
+            sl = slice(j0, j0 + _lib.MAX_FIELDS)
+            r = be.trace3d_mtf(flds[sl], ys[sl], xs, p["stop"], p["a_stop"], freqs, scale, arith=arith, ext=ext,
+                               opd_scale=-1.0 / lam)
+            for j, H in enumerate(p["Hs"][sl]):
+                y = ys[j0 + j]
+                cut_y = (len(y) - 1) * abs((y[-1] - y[0]) / (len(y) - 1)) * scale
+                o = r["otf"][j].copy()
+                out.append(MTF(float(H), freqs.copy(), o, np.abs(o), np.angle(o), (float(cut_x), float(cut_y)),
+                               int(r["status"][j]), int(r["stats"][j]["n_kept"]), r["stats"][j:j + 1].copy()))
+    finally:
+        be.set_apertures(None)
+    return out
+
+
 # ------------------------------------------------------------------------------------------------
 # Seidel aberrations (SURVEY.md section 8 f2): the per-candidate objective of the reference's optimize()
 # ------------------------------------------------------------------------------------------------
