@@ -229,8 +229,8 @@ def _sets_for(ort, n_sets, ny, nx):
     return sets, t
 
 
-def _run(ctx, sets, t, ny, nx, n_u, n_v, stream=0):
-    out = _outs(sets["n_sets"], n_u, n_v)
+def _run(ctx, sets, t, ny, nx, n_u, n_v, stream=0, out=None):
+    out = _outs(sets["n_sets"], n_u, n_v) if out is None else out
     ctx.wavefront_psf_dev(sets, t["ys"].data_ptr(), 1, ny, t["xs"].data_ptr(), nx, n_u, n_v, 0.01, 0.012, 1.5,
                           *[o.data_ptr() for o in out], stream=stream)
     return out
@@ -256,18 +256,24 @@ def test_determinism_and_launch_count(ctx, ort):
 
 
 def test_enqueue_only(ctx, ort):
+    """ort_wavefront_psf_dev returns while the stream is still busy.  The output tensors are allocated before the timed
+    call: torch's first allocation on a new stream can need a cudaMalloc, and when its cache holds most of the device
+    (as after the full-size tests) the allocator may free cached blocks first, which waits for the device -- a wait in
+    the test, not in the library."""
     import torch
     sets, t = _sets_for(ort, 5, 2000, 1000)
-    _run(ctx, sets, t, 2000, 1000, 255, 255)
+    ref = _run(ctx, sets, t, 2000, 1000, 255, 255)
     torch.cuda.synchronize()
     st = torch.cuda.Stream()
     with torch.cuda.stream(st):
+        out = _outs(sets["n_sets"], 255, 255)
         torch.cuda._sleep(int(100e-3 * 2.0e9))           # ~100 ms at ~2 GHz
         t0 = time.perf_counter()
-        _run(ctx, sets, t, 2000, 1000, 255, 255, stream=st.cuda_stream)
+        _run(ctx, sets, t, 2000, 1000, 255, 255, stream=st.cuda_stream, out=out)
         dt = time.perf_counter() - t0
     st.synchronize()
     assert dt < 0.02, dt
+    assert all(torch.equal(a, b) for a, b in zip(out, ref))        # and the enqueued work ran to the same result
 
 
 def test_validation(ctx, ort):
